@@ -2,6 +2,7 @@
 """bench.py — feature-extractor front-end throughput (points/sec on 1024-point clouds) on N B200s.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload sph_dg|cu_dg|...] [--impl ours|reference] [--only]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
            bench.py --gpus N --steps K --warmup W
 
@@ -15,8 +16,13 @@ north-star target is stated on).  The other BASELINE configurations are measured
 `also`: configs[1] cu_dg, configs[4] the spherical resolution sweep r = 16 / 64, configs[2] the registration job
 (front end on both clouds of a pair -> fixed random MLP -> tcgen05 mutual-NN matcher -> RANSAC -> metrics).
 
-Timed regions last >= 200 ms whatever --steps says: the K-step loop is repeated `reps` times between one pair of CUDA
-events and `ms_per_step` is the mean over K * reps steps (`timed_steps`).
+Every timed region runs exactly K = --steps steps between one pair of CUDA events (after a few untimed warm-up steps) and
+`ms_per_step` is their mean; `timed_steps` = K.
+
+`--dump-outputs DIR` writes what the headline's last timed step computed, the engine's output buffers a caller reads (ppf
+[B,4,k,N], devox [B,C,N], edge [B,2C,N] in float32; the voxel indices ind [B,N] as float64), to DIR/<name>.npy.  Inputs
+are seeded, so two builds run with the same arguments can be compared output for output.  bench_outputs/ in the repository
+is git-ignored for this purpose.
 
 Keys beyond the base contract:
   roofline      dominant HBM kernel (vox_fill: the dense [C, r^3] grid + count grid written exactly once), algorithmic
@@ -35,7 +41,6 @@ it times the oracle port on the host.
 import argparse
 import importlib.util
 import json
-import math
 import os
 import subprocess
 import sys
@@ -65,7 +70,6 @@ for _r in (16, 64):
                                           "(BASELINE configs[4] sweep)" % _r)
 RING = 3            # independent input/output buffer sets cycled between timed steps (footprint > L2)
 LANES = 2           # steps in flight (tools/tune_lanes.py: cu_dg 140 / 149 / 149 us per step with 2 / 3 / 4 in flight, sph_dg 121 throughout)
-MIN_TIMED_MS = float(os.environ.get("RI_BENCH_MIN_MS", "250"))  # every timed region lasts at least this long (env: profiling runs under ncu only)
 E2E_DEPTH = 4       # slots of the host-facing pipeline (tools/exp_e2e.py: 2 / 3 / 4 / 6 slots -> 0.578 / 0.579 / 0.547 / 0.552 ms per step)
 
 
@@ -147,10 +151,6 @@ def traffic_from_profile(key):
         return None
 
 
-def reps_for(ms_estimate, steps):
-    return max(1, int(math.ceil(MIN_TIMED_MS / max(ms_estimate * steps, 1e-6))))
-
-
 # ===================================================================================================== ours
 class Harness:
     """Barrier + CUDA events + max over ranks around a callable that enqueues `steps` steps."""
@@ -164,7 +164,7 @@ class Harness:
             self.torch.distributed.barrier()
 
     def timed(self, body, steps, probe=3):
-        """body(n) enqueues n steps.  Returns (ms per step over steps * reps steps, steps * reps)."""
+        """body(n) enqueues n steps.  Runs `probe` untimed steps, then times `steps` steps: returns (ms per step, steps)."""
         torch = self.torch
         def once(n):
             self.barrier(); torch.cuda.synchronize()
@@ -175,13 +175,10 @@ class Harness:
             e1.record()
             torch.cuda.synchronize(); self.barrier()
             return self.shard.max_over_ranks(e0.elapsed_time(e1), self.dev), (t0, time.time())
-        est, _ = once(max(probe, 1))
-        reps = reps_for(est / max(probe, 1), steps)
-        if self.world > 1:                                   # every rank must loop the same number of times
-            reps = int(self.shard.max_over_ranks(reps, self.dev))
-        ms, w = once(steps * reps)
+        once(max(probe, 1))
+        ms, w = once(steps)
         self.windows.append(w)
-        return ms / (steps * reps), steps * reps
+        return ms / steps, steps
 
 
 def measure_workload(key, args, ri_b200, H, rank, world, local, headline):
@@ -242,6 +239,8 @@ def measure_workload(key, args, ri_b200, H, rank, world, local, headline):
             torch.cuda.current_stream().wait_stream(gather_stream)
     lane_steps(max(args.warmup, RING))
     ms, timed_steps = H.timed(lane_steps, args.steps)
+    if headline and args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, engines[(timed_steps - 1) % RING])
     pts_per_step = world * B * N
     value = pts_per_step / (ms * 1e-3)
     alg = engines[0].algorithmic_bytes()
@@ -274,10 +273,7 @@ def measure_workload(key, args, ri_b200, H, rank, world, local, headline):
         el = shard.max_over_ranks((time.perf_counter() - p0) * 1e3, dev)
         H.barrier()
         return el, (t0, time.time())
-    est, _ = e2e_once(5)
-    e2e_steps = max(args.steps, int(math.ceil(MIN_TIMED_MS / max(est / 5, 1e-6))))
-    if world > 1:
-        e2e_steps = int(shard.max_over_ranks(e2e_steps, dev))
+    e2e_steps = args.steps
     ms_e2e, w = e2e_once(e2e_steps); H.windows.append(w)
     ms_e2e /= e2e_steps
     out["e2e"] = {"value": pts_per_step / (ms_e2e * 1e-3), "unit": UNIT, "h2d_bytes_per_step": pipe.slot(0).h2d_bytes,
@@ -287,7 +283,7 @@ def measure_workload(key, args, ri_b200, H, rank, world, local, headline):
     if headline:
         for i in range(3):
             engines[i % RING].run_staged()
-        ms_sync, n_sync = H.timed(lambda n: [engines[i % RING].run_staged() for i in range(n)], min(args.steps, 50))
+        ms_sync, n_sync = H.timed(lambda n: [engines[i % RING].run_staged() for i in range(n)], args.steps)
         out["e2e"]["one_call_at_a_time"] = {"value": pts_per_step / (ms_sync * 1e-3), "ms_per_step": ms_sync,
                                             "api": "FrontEnd.run_staged() (full edge tensor [B,2C,N] shipped back)",
                                             "d2h_bytes_per_step": engines[0].d2h_bytes}
@@ -364,7 +360,16 @@ def measure_workload(key, args, ri_b200, H, rank, world, local, headline):
     return out
 
 
-def measure_registration(ri_b200, H, rank, world):
+def dump_outputs(out_dir, fe):
+    """The outputs of engine `fe`'s last step as DIR/<name>.npy (float32 as computed; int32 indices as float64, exactly)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in (("ppf", fe.ppf), ("devox", fe.devox), ("edge", fe.edge), ("ind", fe.ind)):
+        a = t.cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a if a.dtype == np.float32 else a.astype(np.float64))
+
+
+def measure_registration(ri_b200, H, rank, world, steps):
     """BASELINE configs[2]: 256 source/target pairs x 1024 pts over the GPUs of the box = 256 / world pairs per GPU:
     front end on both clouds of every pair (k-NN + PPF) -> descriptors = a FIXED random two-layer MLP on each point's
     sorted-neighbour point-pair features (stand-in for the dense layers, which are out of scope; rigid-motion invariant like
@@ -409,7 +414,7 @@ def measure_registration(ri_b200, H, rank, world):
         full = None
         for _ in range(3):
             full = step()
-        ms, n = H.timed(lambda n: [step() for _ in range(n)], 5, probe=2)
+        ms, n = H.timed(lambda n: [step() for _ in range(n)], steps, probe=2)
     except Exception as e:                                                                  # never take the headline down
         return {"error": repr(e)[:300]}
     full = full.cpu().numpy()
@@ -421,7 +426,7 @@ def measure_registration(ri_b200, H, rank, world):
             "rre_deg_median": float(np.median(full[:, 16])), "recall_rmse_lt_0.2": float((full[:, 18] < 0.2).mean())}
 
 
-def measure_matcher(ri_b200, H, rank, world):
+def measure_matcher(ri_b200, H, rank, world, steps):
     """The matcher alone (row a11): 32 pairs x 1024 x 1024 x 512 per GPU, descriptors resident in HBM."""
     torch = H.torch
     dev = H.dev
@@ -431,12 +436,12 @@ def measure_matcher(ri_b200, H, rank, world):
     mm = ri_b200.matcher.MutualMatcher(MP, MC, Mn, Mn, device=dev)
     for _ in range(3):
         mm(d1, d2)
-    ms, n = H.timed(lambda n: [mm(d1, d2) for _ in range(n)], 20)
+    ms, n = H.timed(lambda n: [mm(d1, d2) for _ in range(n)], steps)
     mi = ri_b200.matcher.MutualMatcher(MP, MC, Mn, Mn, device=dev, want_dist=False)     # indices only, as the reference returns
     for _ in range(3):
         mi(d1, d2)
     same_idx = bool(torch.equal(mi.idx1, mm.idx1) and torch.equal(mi.idx2, mm.idx2) and torch.equal(mi.count, mm.count))
-    ms_idx, _ = H.timed(lambda n: [mi(d1, d2) for _ in range(n)], 20)
+    ms_idx, _ = H.timed(lambda n: [mi(d1, d2) for _ in range(n)], steps)
     peaks = {}
     try:
         peaks = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))
@@ -473,8 +478,8 @@ def run_ours(args, rank, world, local):
             m = measure_workload(key, args, ri_b200, H, rank, world, local, headline=False)
             m.pop("_batch0"); m.pop("_engine_meta")
             also[key] = m
-        also["matcher"] = measure_matcher(ri_b200, H, rank, world)
-        also["registration_job"] = measure_registration(ri_b200, H, rank, world)
+        also["matcher"] = measure_matcher(ri_b200, H, rank, world, args.steps)
+        also["registration_job"] = measure_registration(ri_b200, H, rank, world, args.steps)
     if rank != 0:
         return
     sampler.stop()
@@ -493,7 +498,7 @@ def run_ours(args, rank, world, local):
                   "result_gather": ("all_gather_into_tensor of every step's voxel indices [B,N] i32 over NCCL, inside the timed region"
                                     if world > 1 else "single GPU: nothing to gather"),
                   "host_numa_binding": numa,
-                  "timed_region": "K-step loop repeated until >= %d ms (timed_steps steps between one pair of CUDA events)" % MIN_TIMED_MS},
+                  "timed_region": "timed_steps = --steps steps between one pair of CUDA events"},
         "roofline": head["roofline"],
         "e2e": head["e2e"],
         "gpu_launches": head["gpu_launches_per_step"] * head["timed_steps"],
@@ -629,8 +634,7 @@ def run_reference(args, rank, world, local):
             step(False)
         e1.record(); torch.cuda.synchronize(); barrier()
         return shard.max_over_ranks(e0.elapsed_time(e1), dev)
-    est = timed_events(2) / 2
-    n1 = int(shard.max_over_ranks(max(args.steps, int(math.ceil(MIN_TIMED_MS / max(est, 1e-6)))), dev))
+    n1 = args.steps
     ms = timed_events(n1) / n1
     for _ in range(3):
         step(True)
@@ -643,8 +647,7 @@ def run_reference(args, rank, world, local):
         el = shard.max_over_ranks((time.perf_counter() - t0) * 1e3, dev)
         barrier()
         return el
-    est2 = timed_wall(2) / 2
-    n2 = int(shard.max_over_ranks(max(min(args.steps, 50), int(math.ceil(MIN_TIMED_MS / max(est2, 1e-6)))), dev))
+    n2 = args.steps
     ms2 = timed_wall(n2) / n2
     if world > 1:
         torch.distributed.destroy_process_group()
@@ -674,7 +677,11 @@ def main():
     ap.add_argument("--only", action="store_true", help="measure only --workload (skip the `also` configurations)")
     ap.add_argument("--fuse-mean-in-flight", dest="fuse_mean_in_flight", action="store_true", default=True)
     ap.add_argument("--torch-mean-in-flight", dest="fuse_mean_in_flight", action="store_false")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the headline's last timed step to DIR/<name>.npy (bench_outputs/ is git-ignored)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
 
     world = int(os.environ.get("WORLD_SIZE", "1"))

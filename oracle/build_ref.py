@@ -106,29 +106,6 @@ def ref_grid_subsampling(points, features=None, labels=None, grid_size=0.1):
     return op[:M], (of[:M, :fdim] if fdim else None), (ol[:M, :ldim] if ldim else None)
 
 
-PYREF_DIR = os.path.join(OUT_DIR, "pyref")
-
-
-def stage_python(force=False):
-    """Copy the reference's PVCNN python package (the *.py files of PVCNN/, PVCNN/models, PVCNN/modules and
-    PVCNN/modules/functional — no sources of the CUDA backend, no build products) into oracle/_ref/pyref/PVCNN so that the
-    drop-in test (tests/test_dropin_reference_python.py) can import the reference's own, unmodified modules on the GPU
-    box, where /root/reference does not exist.  oracle/_ref/ is git-ignored: nothing of it enters this repository's history.
-    Returns the directory to put on sys.path, or None when neither the reference nor a staged copy exists."""
-    src_root = "/root/reference/PVCNN"
-    dst_root = os.path.join(PYREF_DIR, "PVCNN")
-    if not os.path.isdir(src_root):
-        return PYREF_DIR if os.path.isdir(dst_root) else None
-    if os.path.isdir(dst_root) and not force:
-        return PYREF_DIR
-    for sub in ("", "models", "modules", os.path.join("modules", "functional")):
-        os.makedirs(os.path.join(dst_root, sub), exist_ok=True)
-        for f in os.listdir(os.path.join(src_root, sub)):
-            if f.endswith(".py"):
-                shutil.copy2(os.path.join(src_root, sub, f), os.path.join(dst_root, sub, f))
-    return PYREF_DIR
-
-
 def load_ref():
     """Import the prebuilt reference backend (needs `import torch` first). Returns module or None."""
     p = so_path()
@@ -146,4 +123,3 @@ if __name__ == "__main__":
     p = build(force="--force" in sys.argv, verbose="-v" in sys.argv)
     print("reference backend:", p)
     print("reference grid subsampling:", build_gridsub(force="--force" in sys.argv))
-    print("reference python package staged at:", stage_python(force="--force" in sys.argv))

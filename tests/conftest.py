@@ -39,19 +39,10 @@ def oracle():
 
 
 @pytest.fixture(scope="session")
-def ref_backend():
-    """The reference's own CUDA backend recompiled for sm_100a (oracle/_ref/, built by oracle/build_ref.py where
-    /root/reference is mounted; git-ignored, shipped to the GPU box with the tree).  A GPU run without it FAILS — the parity
-    tests would otherwise pass on their golden-file and oracle halves alone and look the same; set RI_ALLOW_NO_REF=1 to turn
-    the failure into a (reported) skip."""
-    from oracle.build_ref import load_ref
-    mod, why = None, "oracle/_ref/_multi_shape_pvcnn_backend.so is missing"
-    try:
-        mod = load_ref()
-    except Exception as e:                       # an unloadable library is as bad as a missing one
-        why = "oracle/_ref did not load: %r" % (e,)
-    if mod is None:
-        if os.environ.get("RI_ALLOW_NO_REF") == "1":
-            pytest.skip(why)
-        pytest.fail(why + " (build it with `python oracle/build_ref.py` where /root/reference exists)")
-    return mod
+def reference(golden_dir):
+    """The reference kernels' bit-exact outputs on the parity tests' inputs (tests/golden/reference_outputs.npz, see
+    _util.ReferenceOutputs).  RI_RECORD_REFERENCE=<file.npz> records them from the reference backend (oracle/_ref)."""
+    from _util import ReferenceOutputs
+    rec = ReferenceOutputs(os.path.join(golden_dir, "reference_outputs.npz"), os.environ.get("RI_RECORD_REFERENCE"))
+    yield rec
+    rec.save()

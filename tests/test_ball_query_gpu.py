@@ -1,6 +1,7 @@
-"""GPU parity of ball query + grouping (SURVEY.md §8f row f1; csrc/ballquery.cu) against the reference's own kernels
-(oracle/_ref, live), the committed golden vectors they produced, and the C oracle.  Indices and gathered features are
-bit-exact; the gradient (float atomics on both sides) within 1e-5 of the largest entry."""
+"""GPU parity of ball query + grouping (SURVEY.md §8f row f1; csrc/ballquery.cu) against what the reference's own kernels
+return on the same inputs (tests/golden/reference_outputs.npz), the committed golden vectors they produced, and the C
+oracle.  Indices and gathered features are bit-exact; the gradient (float atomics on both sides) within 1e-5 of the largest
+entry."""
 import numpy as np
 import pytest
 import torch
@@ -34,21 +35,20 @@ def test_ball_query_golden(ri, golden_dir):
 
 @pytest.mark.parametrize("B,N,M,radius,u", [(32, 1024, 1024, 0.3, 128), (3, 5000, 700, 0.1, 32), (2, 100, 300, 0.5, 200),
                                            (2, 9000, 64, 0.05, 16), (1, 40, 40, 10.0, 64)])
-def test_ball_query_vs_reference_and_oracle(ri, ref_backend, oracle, B, N, M, radius, u):
+def test_ball_query_vs_reference_and_oracle(ri, reference, oracle, B, N, M, radius, u):
     from ri_b200 import synth
     pts = synth.make_clouds(B, N, seed=N + M)[:, :3].copy()
     ctr = (pts[:, :, :M] if M <= N else synth.make_clouds(B, M, seed=7)[:, :3]).copy()
     if M > 8:
         ctr[:, :, -3:] += 100.0                                     # centres with empty neighbourhoods
     idx = torch.ops.ri.ball_query(T(ctr), T(pts), radius, u)
-    if ref_backend is not None:
-        assert torch.equal(idx, ref_backend.ball_query(T(ctr), T(pts), radius, u))
+    case = "ball_query/%d-%d-%d-%g-%d" % (B, N, M, radius, u)
+    reference.equal(case, {"idx": idx}, lambda b: {"idx": b.ball_query(T(ctr), T(pts), radius, u)})
     if B * N * M <= 4e7:
         assert np.array_equal(idx.cpu().numpy(), oracle.ball_query(ctr, pts, radius, u))
     feats = np.random.default_rng(0).standard_normal((B, 5, N)).astype(np.float32)
     grp = torch.ops.ri.grouping(T(feats), idx)
-    if ref_backend is not None:
-        assert torch.equal(grp, ref_backend.grouping_forward(T(feats), idx))
+    reference.equal(case, {"grp": grp}, lambda b: {"grp": b.grouping_forward(T(feats), idx)})
     gy = torch.randn_like(grp)
     gx = torch.ops.ri.grouping_backward(gy, idx, N)
     want = torch.zeros((B, 5, N), device="cuda", dtype=torch.float64)
@@ -56,7 +56,7 @@ def test_ball_query_vs_reference_and_oracle(ri, ref_backend, oracle, B, N, M, ra
     assert scaled_err(gx.cpu().numpy(), want.cpu().numpy()) <= TOL
 
 
-def test_ball_query_module_and_autograd(ri, ref_backend):
+def test_ball_query_module_and_autograd(ri):
     """modules.BallQuery mirrors PVCNN/modules/ball_query.py: shapes, values, and gradients through F.grouping."""
     from ri_b200 import synth
     B, N, C = 2, 512, 7

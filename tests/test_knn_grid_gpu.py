@@ -1,6 +1,6 @@
 """GPU parity of the hash-grid k-NN (csrc/knn_grid.cu) — results must be BIT-IDENTICAL to the brute-force search:
 against ri_knn_f32 (itself pinned to the reference's KnnKernel and the golden vectors in test_parity_gpu.py), against
-the reference's own kernel where it finishes quickly, and against the C oracle on small cases.  Covers the edge cases
+what the reference's own kernel returns on one scan-sized cloud, and against the C oracle on small cases.  Covers the edge cases
 of knn/knn.cu:5-49: distance ties (duplicated points -> lower index first), m < k (sentinel slots), queries outside
 the reference bounding box, d^2 >= 10000 never inserted, degenerate (flat / single-point) clouds."""
 import numpy as np
@@ -48,16 +48,15 @@ def test_grid_equals_brute_force_on_clouds(ri, oracle, n, m, k):
         assert np.array_equal(i1.cpu().numpy(), oi) and np.array_equal(d1.cpu().numpy(), od)
 
 
-def test_grid_on_scan_sized_cloud_vs_reference_kernel(ri, ref_backend):
+def test_grid_on_scan_sized_cloud_vs_reference_kernel(ri, reference):
     """BASELINE configs[3]: ICL-NUIM-shaped scan, ~50k points, k = 20, self query."""
     from ri_b200 import synth
     x = np.stack([synth.make_scan(50000, seed=s)[:3] for s in range(2)])
     d0, i0, d1, i1 = both(x, x, 20)
     assert torch.equal(i0, i1) and torch.equal(d0, d1)
     assert bool((d1[:, 0] == 0).all()) and bool((d1[:, 1:] >= d1[:, :-1]).all())
-    if ref_backend is not None:                                        # the reference's own O(n m k) kernel on one scan
-        r1, _, j1, _ = ref_backend.knn_forward_cuda(T(x[:1]), T(x[:1]), 20)
-        assert torch.equal(j1, i1[:1]) and torch.equal(r1, d1[:1])
+    reference.equal("knn_grid_scan", {"idx": i1[:1], "dist": d1[:1]},  # the reference's own O(n m k) kernel on one scan
+                    lambda b: dict(zip(("dist", "_", "idx", "__"), b.knn_forward_cuda(T(x[:1]), T(x[:1]), 20))))
     # the size-routed public op takes the grid path at this size and returns the same thing
     d2, i2 = torch.ops.ri.knn_one(T(x), T(x), 20)
     assert torch.equal(i2, i1) and torch.equal(d2, d1)

@@ -6,7 +6,6 @@ set -u
 TAG=${1:-r2}
 OUT=gpurun_out/$TAG
 mkdir -p $OUT
-export RI_REQUIRE_REF=1
 nvidia-smi --query-gpu=name,clocks.sm,clocks.max.sm --format=csv > $OUT/gpu.txt 2>&1
 
 if [ "${SKIP_TESTS:-0}" != "1" ]; then
@@ -21,7 +20,6 @@ tail -c 1500 $OUT/bench.json
 
 if [ "${SKIP_NCU:-0}" != "1" ]; then
   # launch list of the bench command (short timed regions: a profiling run, its numbers are never bench values)
-  export RI_BENCH_MIN_MS=0
   timeout 300 python bench.py --steps 2 --warmup 3 > $OUT/bench_short.json 2> $OUT/bench_short.err; rc=$?; echo "short bench rc=$rc"
   if [ $rc -eq 0 ]; then
     timeout 900 ncu --metrics gpu__time_duration.sum --clock-control none -c 4000 --csv --log-file $OUT/launches.csv \
@@ -33,6 +31,5 @@ if [ "${SKIP_NCU:-0}" != "1" ]; then
       ncu -i $OUT/full_$W.ncu-rep --page raw --csv > $OUT/full_$W.csv 2>/dev/null
     done
   fi
-  unset RI_BENCH_MIN_MS
 fi
 ls -la $OUT
