@@ -282,6 +282,22 @@ int ri_registration_metrics_f32(const float* gt, const float* est, const float* 
 int ri_lrf_change_coords_f32(const float* coords, int cstride, const float* mean, int B, int N, int norm_mode,
                              float* out, float* bases, int* ok, void* stream);
 
+/* ---- ICP refinement (SURVEY.md 8f, next row f5) -----------------------------------------------------------------------
+ * Open3D's registration_icp (utils/open3d_func.py wraps it) for P independent pairs per call: T = init, then per iteration
+ * correspondences under T (nearest target point with d^2 < max_corr_dist^2, ties to the lowest target index), an update U
+ * (point-to-point: Horn's closed form, no scale; point-to-plane: Open3D's linearised 6x6 solve, identity when singular),
+ * T = U T, until |d fitness| < rel_fitness and |d inlier_rmse| < rel_rmse or max_iter updates.  max_iter == 0 is Open3D's
+ * evaluate_registration of init.
+ * src [P,n1,3], tgt [P,n2,3], tgt_normals [P,n2,3] (point_to_plane != 0 only; may be NULL otherwise), init [P,4,4] row-major
+ * (NULL = identity), fp32 point-major.  Outputs: T [P,4,4] fp32, fitness [P] and inlier_rmse [P] double, iters [P] int32
+ * (updates applied), corr [P,n1] int32 = target index or -1 under the returned T (may be NULL).  Bit-reproducible; no host
+ * synchronisation.  workspace >= ri_icp_workspace_bytes(P, n1, n2) bytes of device memory, 16-byte aligned. */
+size_t ri_icp_workspace_bytes(int P, int n1, int n2);
+int ri_icp_f32(const float* src, const float* tgt, const float* tgt_normals, const float* init, int P, int n1, int n2,
+               float max_corr_dist, int point_to_plane, int max_iter, float rel_fitness, float rel_rmse,
+               float* T, double* fitness, double* inlier_rmse, int* iters, int* corr,
+               void* workspace, size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -1,0 +1,467 @@
+// icp.cu — batched ICP refinement (point-to-point and point-to-plane) and registration evaluation, sm_100a
+// (SURVEY.md §8f row f5).
+//
+// Open3D's registration_icp / evaluate_registration (the reference reaches them through utils/open3d_func.py), for P
+// independent (source, target) pairs per call, with Open3D's loop per pair:
+//   T = init; res = evaluate(T)
+//   for i in range(max_iter):
+//       U = solve(res.correspondences); T = U T; prev, res = res, evaluate(T)
+//       if |prev.fitness - res.fitness| < rel_fitness and |prev.rmse - res.rmse| < rel_rmse: break
+//   -> T, res.fitness, res.inlier_rmse, iterations (= updates applied), res.correspondences
+//
+// Correspondence: q = T s in fp32 from the fp32 rounding of T; the nearest target point with d^2 < r^2 (strict, as the RANSAC
+// inlier test of pose.cu), d^2 = fma(dz,dz, fma(dy,dy, dx*dx)), d = q - t; equal distances go to the lowest target index
+// (the k-NN tie rule).  fitness = |C| / n1, inlier_rmse = sqrt(sum d^2 / |C|), both 0 when C is empty.
+// Point-to-point: Horn's quaternion on (q_i, t_i), no scale (the optimum of Open3D's Umeyama).  Point-to-plane: Open3D's
+// linearisation r_i = (q_i - t_i).n_i, J_i = [q_i x n_i, n_i], J^T J x = -J^T r in fp64; |det J^T J| < 1e-6 or a non-finite
+// x gives the identity update; U = Rz(x2) Ry(x1) Rx(x0) with translation x3..5 (TransformVector6dToMatrix4d).
+//
+// One deliberate difference from Open3D: Open3D transforms its copy of the source incrementally (s <- U s every
+// iteration); here every iteration transforms the ORIGINAL source by the accumulated T, which is kept in fp64 on the device.
+// The two agree up to rounding; this form does not accumulate fp32 error in the source over the iterations.
+//
+// Kernels (one call: 4 + (max_iter + 1) + 1 launches, no host synchronisation, no allocation)
+//   icp_setup      one CTA per pair: bounding box of the target -> uniform grid (grid_g cells per axis as knn_grid.cu,
+//                  <= 64, cell edge >= r / 2 so that a radius query touches at most 5 cells per axis); pair state
+//                  (T = init in fp64, done flag, ticket) initialised; cell histogram cleared.
+//   icp_bin<0/1>   histogram of the target's cells, then counting-sort scatter: float4 (x, y, z, index) in cell order,
+//                  normals in the same order.  (Order inside a cell is not fixed; nothing depends on it: the selection key
+//                  is (distance, index).)
+//   icp_scan       exclusive scan of the histogram.
+//   icp_iter       grid (source tiles, P), once per iteration.  A CTA of a converged pair exits at once.  Otherwise each
+//                  thread runs a radius-bounded 1-NN for its source points over the cells the query ball can touch,
+//                  accumulates count, sum d^2 and the solver's moments in fp64 (15 for point-to-point: sum q, sum t,
+//                  sum q t^T; 27 for point-to-plane: the upper triangle of J^T J and J^T r), the CTA reduces them in a
+//                  fixed order into partials[P][tiles][K].  The last CTA of the pair (threadfence + atomic ticket, reset
+//                  afterwards) sums the partials in tile order, computes fitness / rmse, applies the convergence test
+//                  against the previous iteration's values, and either marks the pair done or solves U and sets T = U T.
+//                  No float atomics anywhere: a call is bit-reproducible.
+//   icp_final      T (fp32), fitness, rmse (fp64), iterations (int32).
+#include "ri_common.cuh"
+#include "rigid.cuh"
+
+namespace {
+
+constexpr int kMaxG = 64;
+constexpr int kSetupThreads = 1024;
+constexpr int kThreads = 256;
+constexpr int kPerThread = 2;
+constexpr int kTile = kThreads * kPerThread;      // source points per CTA
+constexpr int kKMax = 29;                         // count, sum d^2, 27 point-to-plane moments
+constexpr int kKPoint = 17;                       // count, sum d^2, 15 point-to-point moments
+
+struct GridHdr {               // per pair, 16 ints at the head of its grid slab
+    float ox, oy, oz, h, inv_h;
+    int gx, gy, gz;
+    int pad[8];
+};
+
+struct PairState {             // per pair, 128 bytes
+    double T[12];              // 3x4 row-major, fp64
+    double fitness, rmse;      // of the last evaluation
+    int done, iters, ticket, pad;
+};
+
+__host__ __device__ inline int grid_g(int m)
+{
+    int g = 1;
+    while ((long long)(g + 1) * (g + 1) * (g + 1) * 2 <= (long long)(m > 0 ? m : 1) && g < kMaxG) ++g;   // ~cbrt(m/2)
+    return g;
+}
+
+struct IcpWs {                 // byte offsets into the workspace; the grid slab offsets are int32 indices inside one slab
+    size_t state, partials, grids, total;
+    int tiles, cells_max, hdr, start, cur, sorted, normals, stride;
+};
+__host__ __device__ inline IcpWs icp_ws_layout(int P, int n1, int n2)
+{
+    IcpWs w;
+    w.tiles = (n1 + kTile - 1) / kTile;
+    const int g = grid_g(n2);
+    w.cells_max = g * g * g;
+    int o = 0;
+    w.hdr = o; o += 16;
+    w.start = o; o += w.cells_max + 1;
+    w.cur = o; o += w.cells_max;
+    o = (o + 3) / 4 * 4;
+    w.sorted = o; o += 4 * n2;                                      // float4 (x, y, z, index)
+    w.normals = o; o += 4 * n2;                                     // float4 (nx, ny, nz, 0)
+    w.stride = o;
+    w.state = 0;
+    w.partials = (size_t)P * sizeof(PairState);
+    w.grids = (w.partials + (size_t)P * w.tiles * kKMax * sizeof(double) + 255) / 256 * 256;   // float4 slabs: 16-byte aligned
+    w.total = w.grids + (size_t)P * w.stride * sizeof(int);
+    return w;
+}
+
+__global__ void __launch_bounds__(kSetupThreads)
+icp_setup_kernel(const float* __restrict__ tgt, const float* __restrict__ init, int P, int n1, int n2, float r,
+                 unsigned char* __restrict__ ws)
+{
+    __shared__ float smin[3][kSetupThreads / 32], smax[3][kSetupThreads / 32];
+    const int p = blockIdx.x, tid = threadIdx.x;
+    const IcpWs L = icp_ws_layout(P, n1, n2);
+    int* W = reinterpret_cast<int*>(ws + L.grids) + (size_t)p * L.stride;
+    const float* X = tgt + (size_t)p * n2 * 3;
+    float lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
+    for (int j = tid; j < n2; j += kSetupThreads)
+#pragma unroll
+        for (int a = 0; a < 3; ++a) {
+            const float v = X[3 * (size_t)j + a];
+            lo[a] = fminf(lo[a], v); hi[a] = fmaxf(hi[a], v);
+        }
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            lo[a] = fminf(lo[a], __shfl_xor_sync(0xffffffffu, lo[a], o));
+            hi[a] = fmaxf(hi[a], __shfl_xor_sync(0xffffffffu, hi[a], o));
+        }
+        if ((tid & 31) == 0) { smin[a][tid >> 5] = lo[a]; smax[a][tid >> 5] = hi[a]; }
+    }
+    __syncthreads();
+    if (tid == 0) {
+        GridHdr H;
+        float e[3];
+        for (int a = 0; a < 3; ++a) {
+            float l = smin[a][0], h = smax[a][0];
+            for (int w = 1; w < kSetupThreads / 32; ++w) { l = fminf(l, smin[a][w]); h = fmaxf(h, smax[a][w]); }
+            if (!(l <= h)) { l = 0.f; h = 0.f; }               // NaN cloud
+            (a == 0 ? H.ox : a == 1 ? H.oy : H.oz) = l;
+            e[a] = h - l;
+        }
+        const int g = grid_g(n2);
+        const float emax = fmaxf(e[0], fmaxf(e[1], e[2]));
+        H.h = fmaxf(emax / (float)g, 0.5f * r);                 // >= r/2: a query ball spans at most 5 cells per axis
+        H.inv_h = 1.0f / H.h;
+        H.gx = min(g, (int)(e[0] * H.inv_h) + 1);
+        H.gy = min(g, (int)(e[1] * H.inv_h) + 1);
+        H.gz = min(g, (int)(e[2] * H.inv_h) + 1);
+        *reinterpret_cast<GridHdr*>(W + L.hdr) = H;
+        PairState* S = reinterpret_cast<PairState*>(ws + L.state) + p;
+        for (int k = 0; k < 12; ++k)
+            S->T[k] = init ? (double)init[(size_t)p * 16 + k] : (k % 5 == 0 ? 1.0 : 0.0);
+        S->fitness = 0.0; S->rmse = 0.0;
+        S->done = 0; S->iters = 0; S->ticket = 0;
+    }
+    for (int c = tid; c < L.cells_max; c += kSetupThreads) W[L.cur + c] = 0;
+}
+
+__device__ __forceinline__ int cell_of(const GridHdr& H, float x, float y, float z)
+{
+    const int cx = min(max((int)floorf((x - H.ox) * H.inv_h), 0), H.gx - 1);
+    const int cy = min(max((int)floorf((y - H.oy) * H.inv_h), 0), H.gy - 1);
+    const int cz = min(max((int)floorf((z - H.oz) * H.inv_h), 0), H.gz - 1);
+    return (cx * H.gy + cy) * H.gz + cz;
+}
+
+// PASS 0: histogram into cur; PASS 1: scatter through start + atomic cursor
+template <int PASS>
+__global__ void __launch_bounds__(256)
+icp_bin_kernel(const float* __restrict__ tgt, const float* __restrict__ nrm, int P, int n1, int n2,
+               unsigned char* __restrict__ ws)
+{
+    const int p = blockIdx.y, t = blockIdx.x * 256 + threadIdx.x;
+    if (t >= n2) return;
+    const IcpWs L = icp_ws_layout(P, n1, n2);
+    int* W = reinterpret_cast<int*>(ws + L.grids) + (size_t)p * L.stride;
+    const GridHdr H = *reinterpret_cast<const GridHdr*>(W + L.hdr);
+    const float* X = tgt + ((size_t)p * n2 + t) * 3;
+    const float x = X[0], y = X[1], z = X[2];
+    const int c = cell_of(H, x, y, z);
+    if (PASS == 0) {
+        atomicAdd(W + L.cur + c, 1);
+    } else {
+        const int pos = W[L.start + c] + atomicAdd(W + L.cur + c, 1);
+        reinterpret_cast<float4*>(W + L.sorted)[pos] = make_float4(x, y, z, __int_as_float(t));
+        if (nrm) {
+            const float* Nv = nrm + ((size_t)p * n2 + t) * 3;
+            reinterpret_cast<float4*>(W + L.normals)[pos] = make_float4(Nv[0], Nv[1], Nv[2], 0.f);
+        }
+    }
+}
+
+// exclusive scan of a pair's histogram; the cursors are reset to 0 for the scatter pass
+__global__ void __launch_bounds__(1024)
+icp_scan_kernel(int P, int n1, int n2, unsigned char* __restrict__ ws)
+{
+    __shared__ int swarp[32];
+    __shared__ int scarry, stotal;
+    const int p = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    const IcpWs L = icp_ws_layout(P, n1, n2);
+    int* W = reinterpret_cast<int*>(ws + L.grids) + (size_t)p * L.stride;
+    int* cur = W + L.cur;
+    int* start = W + L.start;
+    if (tid == 0) scarry = 0;
+    __syncthreads();
+    for (int c0 = 0; c0 < L.cells_max; c0 += 1024) {
+        const int c = c0 + tid;
+        const int v = c < L.cells_max ? cur[c] : 0;
+        int incl = v;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int t = __shfl_up_sync(0xffffffffu, incl, o);
+            if (lane >= o) incl += t;
+        }
+        if (lane == 31) swarp[wid] = incl;
+        __syncthreads();
+        if (wid == 0) {
+            const int w = swarp[lane];
+            int wi = w;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const int t = __shfl_up_sync(0xffffffffu, wi, o);
+                if (lane >= o) wi += t;
+            }
+            swarp[lane] = wi - w;
+            if (lane == 31) stotal = wi;
+        }
+        __syncthreads();
+        if (c < L.cells_max) { start[c] = scarry + swarp[wid] + incl - v; cur[c] = 0; }
+        __syncthreads();
+        if (tid == 0) scarry += stotal;
+        __syncthreads();
+    }
+    if (tid == 0) start[L.cells_max] = scarry;
+}
+
+// Cell range [lo, hi] of one axis that a ball of radius r around coordinate x can touch; false when it misses the grid.
+// In cell units (u = (x - o) / h) the exact range is [floor(u - r/h), floor(u + r/h)].  Every rounded quantity involved
+// (u, r/h, the cell coordinate a target point was binned with) is within a few ulps of a value of magnitude <= g + r/h
+// <= 66 whenever the ball reaches the grid, i.e. within 1e-4 cells; the 1e-3-cell widening on each side therefore cannot
+// drop a cell that holds a point within r.  Far outside the grid the widening may admit an extra cell: harmless, the
+// distance test decides.
+__device__ __forceinline__ bool axis_range(float x, float o, float inv_h, float rc, int g, int& lo, int& hi)
+{
+    const float u = (x - o) * inv_h;
+    const float a = floorf(u - rc - 1e-3f), b = floorf(u + rc + 1e-3f);
+    if (!(b >= 0.f) || !(a <= (float)(g - 1))) return false;
+    lo = a < 0.f ? 0 : (int)a;
+    hi = b > (float)(g - 1) ? g - 1 : (int)b;
+    return true;
+}
+
+template <bool PLANE>
+__global__ void __launch_bounds__(kThreads)
+icp_iter_kernel(const float* __restrict__ src, int P, int n1, int n2, float r, int it, int max_iter, float rel_fitness,
+                float rel_rmse, int* __restrict__ corr, unsigned char* __restrict__ ws)
+{
+    constexpr int K = PLANE ? kKMax : kKPoint;
+    __shared__ double red[(kThreads / 32) * K];
+    __shared__ double tot[K];
+    __shared__ float Tf[12];
+    __shared__ int s_flag;
+    const int p = blockIdx.y, tile = blockIdx.x, tid = threadIdx.x;
+    const IcpWs L = icp_ws_layout(P, n1, n2);
+    PairState* S = reinterpret_cast<PairState*>(ws + L.state) + p;
+    if (tid == 0) {
+        s_flag = S->done;
+        for (int k = 0; k < 12; ++k) Tf[k] = (float)S->T[k];
+    }
+    __syncthreads();
+    if (s_flag) return;
+
+    const int* W = reinterpret_cast<const int*>(ws + L.grids) + (size_t)p * L.stride;
+    const GridHdr H = *reinterpret_cast<const GridHdr*>(W + L.hdr);
+    const int* start = W + L.start;
+    const float4* Pt = reinterpret_cast<const float4*>(W + L.sorted);
+    const float4* Nt = reinterpret_cast<const float4*>(W + L.normals);
+    const float r2 = __fmul_rn(r, r);
+    const float rc = r * H.inv_h;
+
+    double acc[K];
+#pragma unroll
+    for (int k = 0; k < K; ++k) acc[k] = 0.0;
+
+#pragma unroll 1
+    for (int s = 0; s < kPerThread; ++s) {
+        const int i = tile * kTile + s * kThreads + tid;
+        if (i >= n1) break;
+        const float* Sv = src + ((size_t)p * n1 + i) * 3;
+        const float sx = Sv[0], sy = Sv[1], sz = Sv[2];
+        const float qx = __fadd_rn(__fmaf_rn(Tf[2], sz, __fmaf_rn(Tf[1], sy, __fmul_rn(Tf[0], sx))), Tf[3]);
+        const float qy = __fadd_rn(__fmaf_rn(Tf[6], sz, __fmaf_rn(Tf[5], sy, __fmul_rn(Tf[4], sx))), Tf[7]);
+        const float qz = __fadd_rn(__fmaf_rn(Tf[10], sz, __fmaf_rn(Tf[9], sy, __fmul_rn(Tf[8], sx))), Tf[11]);
+        float best = r2;
+        int bj = -1, bp = -1;
+        int x0, x1, y0, y1, z0, z1;
+        if (isfinite(qx) && isfinite(qy) && isfinite(qz) &&
+            axis_range(qx, H.ox, H.inv_h, rc, H.gx, x0, x1) && axis_range(qy, H.oy, H.inv_h, rc, H.gy, y0, y1) &&
+            axis_range(qz, H.oz, H.inv_h, rc, H.gz, z0, z1)) {
+            for (int x = x0; x <= x1; ++x)
+                for (int y = y0; y <= y1; ++y) {
+                    const int base = (x * H.gy + y) * H.gz;
+                    const int p0 = __ldg(start + base + z0), p1 = __ldg(start + base + z1 + 1);
+                    for (int q = p0; q < p1; ++q) {
+                        const float4 c = __ldg(Pt + q);
+                        const float dx = __fsub_rn(qx, c.x), dy = __fsub_rn(qy, c.y), dz = __fsub_rn(qz, c.z);
+                        const float d = __fmaf_rn(dz, dz, __fmaf_rn(dy, dy, __fmul_rn(dx, dx)));
+                        const int j = __float_as_int(c.w);
+                        if (d < best || (d == best && j < bj)) { best = d; bj = j; bp = q; }
+                    }
+                }
+        }
+        if (corr) corr[(size_t)p * n1 + i] = bj;
+        if (bj < 0) continue;
+        const float4 c = __ldg(Pt + bp);
+        const double dqx = qx, dqy = qy, dqz = qz, tx = c.x, ty = c.y, tz = c.z;
+        acc[0] += 1.0;
+        acc[1] += (double)best;
+        if (!PLANE) {
+            acc[2] += dqx; acc[3] += dqy; acc[4] += dqz;
+            acc[5] += tx; acc[6] += ty; acc[7] += tz;
+            acc[8] += dqx * tx; acc[9] += dqx * ty; acc[10] += dqx * tz;
+            acc[11] += dqy * tx; acc[12] += dqy * ty; acc[13] += dqy * tz;
+            acc[14] += dqz * tx; acc[15] += dqz * ty; acc[16] += dqz * tz;
+        } else {
+            const float4 nv = __ldg(Nt + bp);
+            const double nx = nv.x, ny = nv.y, nz = nv.z;
+            const double res = (dqx - tx) * nx + (dqy - ty) * ny + (dqz - tz) * nz;
+            const double J[6] = {dqy * nz - dqz * ny, dqz * nx - dqx * nz, dqx * ny - dqy * nx, nx, ny, nz};
+            int k = 2;
+#pragma unroll
+            for (int a = 0; a < 6; ++a)
+#pragma unroll
+                for (int b = a; b < 6; ++b) acc[k++] += J[a] * J[b];
+#pragma unroll
+            for (int a = 0; a < 6; ++a) acc[23 + a] += J[a] * res;
+        }
+    }
+
+    block_sum<K>(acc, red);
+    double* part = reinterpret_cast<double*>(ws + L.partials) + (size_t)p * L.tiles * kKMax;
+    if (tid == 0) {
+#pragma unroll
+        for (int k = 0; k < K; ++k) part[(size_t)tile * kKMax + k] = acc[k];
+        __threadfence();
+        s_flag = atomicAdd(&S->ticket, 1) == L.tiles - 1;
+    }
+    __syncthreads();
+    if (!s_flag) return;
+
+    // ---- last CTA of the pair: partials in tile order -> fitness, rmse, convergence, update
+    __threadfence();
+    if (tid < K) {
+        double v = 0.0;
+        for (int t = 0; t < L.tiles; ++t) v += __ldcg(part + (size_t)t * kKMax + tid);
+        tot[tid] = v;
+    }
+    __syncthreads();
+    if (tid != 0) return;
+    S->ticket = 0;
+    const double cnt = tot[0];
+    const double fitness = cnt / (double)n1;
+    const double rmse = cnt > 0.0 ? sqrt(tot[1] / cnt) : 0.0;
+    const bool converged = it > 0 && fabs(S->fitness - fitness) < (double)rel_fitness &&
+                           fabs(S->rmse - rmse) < (double)rel_rmse;
+    S->fitness = fitness;
+    S->rmse = rmse;
+    if (converged || it == max_iter) {
+        S->done = 1;
+        S->iters = it;
+        return;
+    }
+    double U[12] = {1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0};
+    if (!PLANE) {
+        if (cnt > 0.0) {
+            const double inv = 1.0 / cnt;
+            const double cq[3] = {tot[2] * inv, tot[3] * inv, tot[4] * inv};
+            const double ct[3] = {tot[5] * inv, tot[6] * inv, tot[7] * inv};
+            double Hm[9], R[9];
+#pragma unroll
+            for (int a = 0; a < 3; ++a)
+#pragma unroll
+                for (int b = 0; b < 3; ++b) Hm[3 * a + b] = tot[8 + 3 * a + b] - cnt * cq[a] * ct[b];
+            horn_rotation(Hm, R);
+#pragma unroll
+            for (int a = 0; a < 3; ++a) {
+                U[4 * a + 0] = R[3 * a + 0]; U[4 * a + 1] = R[3 * a + 1]; U[4 * a + 2] = R[3 * a + 2];
+                U[4 * a + 3] = ct[a] - (R[3 * a] * cq[0] + R[3 * a + 1] * cq[1] + R[3 * a + 2] * cq[2]);
+            }
+        }
+    } else {
+        double b[6], x[6];
+#pragma unroll
+        for (int a = 0; a < 6; ++a) b[a] = -tot[23 + a];
+        if (ldlt_solve6(tot + 2, b, x)) {
+            const double ca = cos(x[0]), sa = sin(x[0]), cb = cos(x[1]), sb = sin(x[1]), cg = cos(x[2]), sg = sin(x[2]);
+            // Rz(x2) Ry(x1) Rx(x0)
+            U[0] = cg * cb; U[1] = cg * sb * sa - sg * ca; U[2] = cg * sb * ca + sg * sa; U[3] = x[3];
+            U[4] = sg * cb; U[5] = sg * sb * sa + cg * ca; U[6] = sg * sb * ca - cg * sa; U[7] = x[4];
+            U[8] = -sb;     U[9] = cb * sa;                U[10] = cb * ca;               U[11] = x[5];
+        }
+    }
+    double Tn[12];
+#pragma unroll
+    for (int a = 0; a < 3; ++a)
+#pragma unroll
+        for (int c = 0; c < 4; ++c)
+            Tn[4 * a + c] = U[4 * a] * S->T[c] + U[4 * a + 1] * S->T[4 + c] + U[4 * a + 2] * S->T[8 + c] + (c == 3 ? U[4 * a + 3] : 0.0);
+#pragma unroll
+    for (int k = 0; k < 12; ++k) S->T[k] = Tn[k];
+}
+
+__global__ void icp_final_kernel(int P, int n1, int n2, const unsigned char* __restrict__ ws, float* __restrict__ T,
+                                 double* __restrict__ fitness, double* __restrict__ rmse, int* __restrict__ iters)
+{
+    const int p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= P) return;
+    const IcpWs L = icp_ws_layout(P, n1, n2);
+    const PairState* S = reinterpret_cast<const PairState*>(ws + L.state) + p;
+    float* O = T + (size_t)p * 16;
+    for (int k = 0; k < 12; ++k) O[k] = (float)S->T[k];
+    O[12] = 0.f; O[13] = 0.f; O[14] = 0.f; O[15] = 1.f;
+    fitness[p] = S->fitness;
+    rmse[p] = S->rmse;
+    iters[p] = S->iters;
+}
+
+}  // namespace
+
+extern "C" size_t ri_icp_workspace_bytes(int P, int n1, int n2)
+{
+    if (P <= 0 || n1 <= 0 || n2 <= 0) return 16;
+    return icp_ws_layout(P, n1, n2).total;
+}
+
+// src [P,n1,3], tgt [P,n2,3], tgt_normals [P,n2,3] (point-to-plane only), init [P,4,4] row-major (NULL = identity), all fp32
+// point-major.  -> T [P,4,4] fp32, fitness [P], inlier_rmse [P] fp64, iters [P] int32, corr [P,n1] (target index or -1 under
+// the returned T; NULL = not written).
+extern "C" int ri_icp_f32(const float* src, const float* tgt, const float* tgt_normals, const float* init, int P, int n1,
+                          int n2, float max_corr_dist, int point_to_plane, int max_iter, float rel_fitness, float rel_rmse,
+                          float* T, double* fitness, double* inlier_rmse, int* iters, int* corr, void* workspace,
+                          size_t workspace_bytes, void* stream)
+{
+    if (P < 0 || n1 <= 0 || n2 <= 0 || !(max_corr_dist > 0.f) || max_iter < 0) return RI_ERR_BAD_ARG;
+    if (point_to_plane && tgt_normals == nullptr) return RI_ERR_BAD_ARG;
+    if (P > 65535) return RI_ERR_UNSUPPORTED;
+    if (P == 0) return RI_OK;
+    const IcpWs L = icp_ws_layout(P, n1, n2);
+    if (L.tiles > 65535) return RI_ERR_UNSUPPORTED;
+    if (workspace == nullptr || ((uintptr_t)workspace & 15) != 0 || workspace_bytes < L.total) return RI_ERR_WORKSPACE;
+    cudaStream_t st = (cudaStream_t)stream;
+    unsigned char* ws = reinterpret_cast<unsigned char*>(workspace);
+    const float* nrm = point_to_plane ? tgt_normals : nullptr;
+    icp_setup_kernel<<<P, kSetupThreads, 0, st>>>(tgt, init, P, n1, n2, max_corr_dist, ws);
+    RI_LAUNCH_CHECK();
+    const dim3 gb((n2 + 255) / 256, P);
+    icp_bin_kernel<0><<<gb, 256, 0, st>>>(tgt, nrm, P, n1, n2, ws);
+    RI_LAUNCH_CHECK();
+    icp_scan_kernel<<<P, 1024, 0, st>>>(P, n1, n2, ws);
+    RI_LAUNCH_CHECK();
+    icp_bin_kernel<1><<<gb, 256, 0, st>>>(tgt, nrm, P, n1, n2, ws);
+    RI_LAUNCH_CHECK();
+    const dim3 gi(L.tiles, P);
+    for (int it = 0; it <= max_iter; ++it) {
+        if (point_to_plane)
+            icp_iter_kernel<true><<<gi, kThreads, 0, st>>>(src, P, n1, n2, max_corr_dist, it, max_iter, rel_fitness,
+                                                           rel_rmse, corr, ws);
+        else
+            icp_iter_kernel<false><<<gi, kThreads, 0, st>>>(src, P, n1, n2, max_corr_dist, it, max_iter, rel_fitness,
+                                                            rel_rmse, corr, ws);
+        RI_LAUNCH_CHECK();
+    }
+    icp_final_kernel<<<(P + 127) / 128, 128, 0, st>>>(P, n1, n2, ws, T, fitness, inlier_rmse, iters);
+    RI_LAUNCH_CHECK();
+    return RI_OK;
+}

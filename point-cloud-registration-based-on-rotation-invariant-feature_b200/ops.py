@@ -6,6 +6,8 @@ torch (so they live in the caching allocator, as the reference's torch::zeros ou
 hand-written sm_100a kernels on torch's CURRENT stream through ctypes.  There is no other implementation behind
 these names: no Triton, no eager fallback, no CPU path.
 """
+from typing import Optional
+
 import torch
 
 from . import _lib
@@ -773,3 +775,48 @@ def local_ppf_mlp_max(points_coords: torch.Tensor, points_normals: torch.Tensor,
 @local_ppf_mlp_max.register_fake
 def _(points_coords, points_normals, centers_coords, centers_normals, neighbors, w1, b1, w2, b2):
     return points_coords.new_empty((points_coords.shape[0], w2.shape[0], centers_coords.shape[2]))
+
+
+# ---------------------------------------------------------------------------------------------- ICP refinement (f5)
+@torch.library.custom_op("ri::icp", mutates_args=())
+def icp(src: torch.Tensor, tgt: torch.Tensor, tgt_normals: Optional[torch.Tensor], init: torch.Tensor, r: float,
+        point_to_plane: bool, max_iter: int, rel_fitness: float, rel_rmse: float, want_corr: bool) -> tuple[
+        torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    """src [P,n1,3], tgt [P,n2,3], tgt_normals [P,n2,3] or None, init [P,4,4] f32 -> (T [P,4,4] f32, fitness [P] f64,
+    inlier_rmse [P] f64, iterations [P] i32, corr [P,n1] i32 (target index or -1 under T; [P,0] unless want_corr)).
+    Open3D's registration_icp per pair, all pairs in one call (csrc/icp.cu); max_iter == 0 evaluates init."""
+    _req(src, "src", torch.float32); _req(tgt, "tgt", torch.float32); _req(init, "init", torch.float32)
+    ts = (src, tgt, init)
+    if tgt_normals is not None:
+        _req(tgt_normals, "tgt_normals", torch.float32)
+        ts = ts + (tgt_normals,)
+    dev = _same_device(*ts)
+    _shape(src, "src", None, None, 3)
+    P, n1, _ = src.shape
+    _shape(tgt, "tgt", P, None, 3)
+    n2 = tgt.shape[1]
+    _shape(init, "init", P, 4, 4)
+    if tgt_normals is not None:
+        _shape(tgt_normals, "tgt_normals", P, n2, 3)
+    elif point_to_plane:
+        raise RuntimeError("point-to-plane ICP needs tgt_normals")
+    with torch.cuda.device(dev):
+        T = torch.empty((P, 4, 4), dtype=torch.float32, device=dev)
+        fit = torch.empty((P,), dtype=torch.float64, device=dev)
+        rmse = torch.empty((P,), dtype=torch.float64, device=dev)
+        iters = torch.empty((P,), dtype=torch.int32, device=dev)
+        corr = torch.empty((P, n1 if want_corr else 0), dtype=torch.int32, device=dev)
+        nws = _L.ri_icp_workspace_bytes(P, n1, n2)
+        ws = torch.empty(nws, dtype=torch.uint8, device=dev)
+        _check(_L.ri_icp_f32(src.data_ptr(), tgt.data_ptr(), tgt_normals.data_ptr() if tgt_normals is not None else None,
+                             init.data_ptr(), P, n1, n2, float(r), int(point_to_plane), int(max_iter), float(rel_fitness),
+                             float(rel_rmse), T.data_ptr(), fit.data_ptr(), rmse.data_ptr(), iters.data_ptr(),
+                             corr.data_ptr() if want_corr else None, ws.data_ptr(), nws, _stream()), "ri_icp")
+    return T, fit, rmse, iters, corr
+
+
+@icp.register_fake
+def _(src, tgt, tgt_normals, init, r, point_to_plane, max_iter, rel_fitness, rel_rmse, want_corr):
+    P, n1 = src.shape[0], src.shape[1]
+    return (src.new_empty((P, 4, 4)), src.new_empty((P,), dtype=torch.float64), src.new_empty((P,), dtype=torch.float64),
+            src.new_empty((P,), dtype=torch.int32), src.new_empty((P, n1 if want_corr else 0), dtype=torch.int32))

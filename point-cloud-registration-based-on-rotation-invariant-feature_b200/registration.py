@@ -1,13 +1,16 @@
-"""Registration back end on the GPU: descriptors -> mutual matches -> rigid pose -> RRE / RTE / RMSE, whole batches of
-pairs per call (csrc/matcher.cu + csrc/pose.cu).
+"""Registration back end on the GPU: descriptors -> mutual matches -> rigid pose -> ICP refinement -> RRE / RTE / RMSE,
+whole batches of pairs per call (csrc/matcher.cu + csrc/pose.cu + csrc/icp.cu).
 
 Mirrors the reference's meter `MeterModelNet40_registration` (/root/reference/datasets/deepgmr_mn40.py:98-244): same
 constructor argument, same `update((feat1, feat2), (pt1, pt2, gt_trans))` / `compute()` contract, same thresholds
 (:107-109), same result keys (:141).  The reference copies the descriptors to the host and calls Open3D / TEASER++ once
 per pair (:121, :165-231); here `func='ransac'` runs the RANSAC configuration the reference hands to Open3D
 (utils/open3d_func.py:43-49: voxel_size 0.08, edge-length similarity 0.9, max_iter 1000) on the GPU for all pairs at once,
-and `func='kabsch'` the plain least squares over the mutual matches.  FGR, ICP and TEASER++ are third-party solvers the
-reference only calls into; they are not re-implemented (func='fgr' / 'icp' / 'teaserpp' raise).
+and `func='kabsch'` the plain least squares over the mutual matches.  `icp()` / `evaluate_registration()` are Open3D's
+registration_icp (point-to-point and point-to-plane) and evaluate_registration, batched over pairs; `register_pairs` and
+the meter refine their pose with it when given `icp={...}`.  FGR and TEASER++ are third-party solvers the reference only
+calls into; they are not re-implemented (func='fgr' / 'icp' / 'teaserpp' raise in `estimate_poses`: ICP refines a pose,
+it does not estimate one from matches).
 """
 import time
 
@@ -15,7 +18,8 @@ import torch
 
 from . import matcher
 
-__all__ = ['estimate_poses', 'registration_metrics', 'register_pairs', 'MeterModelNet40_registration']
+__all__ = ['estimate_poses', 'registration_metrics', 'icp', 'evaluate_registration', 'register_pairs',
+           'MeterModelNet40_registration']
 
 
 def estimate_poses(src, tgt, idx1, idx2, count, func='ransac', voxel_size=0.08, max_iter=1000, edge_similarity=0.9,
@@ -23,7 +27,8 @@ def estimate_poses(src, tgt, idx1, idx2, count, func='ransac', voxel_size=0.08, 
     """src [P,n1,3], tgt [P,n2,3] CUDA fp32; idx1/idx2/count: the mutual matches (matcher.mutual_nn).
     -> (T [P,4,4] fp32 mapping src onto tgt, inliers [P] int32)."""
     if func not in ('ransac', 'kabsch'):
-        raise ValueError("func must be 'ransac' or 'kabsch' (Open3D FGR / ICP and TEASER++ are third-party solvers)")
+        raise ValueError("func must be 'ransac' or 'kabsch' (Open3D FGR and TEASER++ are third-party solvers; ICP refines "
+                         "a pose: icp() or register_pairs(..., icp={...}))")
     hyps = int(max_iter) if func == 'ransac' else 0
     return torch.ops.ri.pose_from_matches(src.float().contiguous(), tgt.float().contiguous(), idx1.contiguous(),
                                           idx2.contiguous(), count.contiguous(), hyps, float(voxel_size),
@@ -36,17 +41,60 @@ def registration_metrics(gt_trans, est_trans, pts):
                                              pts.float().contiguous())
 
 
-def register_pairs(feat1, feat2, pt1, pt2, func='ransac', **kw):
-    """feat1/feat2 [P,C,n] (the extractor's layout), pt1/pt2 [P,n,3], all CUDA -> (T [P,4,4], inliers [P], matches dict)."""
+_ESTIMATIONS = ('point_to_point', 'point_to_plane')
+
+
+def icp(src, tgt, max_correspondence_distance, init=None, estimation='point_to_point', tgt_normals=None, max_iter=30,
+        relative_fitness=1e-6, relative_rmse=1e-6, return_correspondences=False):
+    """Open3D's registration_icp for P pairs at once.  src [P,n1,3], tgt [P,n2,3] CUDA fp32; init [P,4,4] (default identity);
+    tgt_normals [P,n2,3] for estimation='point_to_plane'.  Stops a pair when both its fitness and its inlier RMSE change by
+    less than the relative criteria (Open3D's ICPConvergenceCriteria), or after max_iter updates.
+    -> dict(transformation [P,4,4] fp32 src -> tgt, fitness [P] f64, inlier_rmse [P] f64, iterations [P] int32
+    [, correspondences [P,n1] int32: target index or -1, under the returned transformation])."""
+    if estimation not in _ESTIMATIONS:
+        raise ValueError("estimation must be one of %s, got %r" % (_ESTIMATIONS, estimation))
+    plane = estimation == 'point_to_plane'
+    if plane and tgt_normals is None:
+        raise ValueError("estimation='point_to_plane' needs tgt_normals")
+    src = src.float().contiguous()
+    if init is None:
+        init = torch.eye(4, dtype=torch.float32, device=src.device).expand(src.shape[0], 4, 4)
+    nrm = tgt_normals.float().contiguous() if plane else None
+    T, fit, rmse, iters, corr = torch.ops.ri.icp(src, tgt.float().contiguous(), nrm, init.float().contiguous(),
+                                                 float(max_correspondence_distance), plane, int(max_iter),
+                                                 float(relative_fitness), float(relative_rmse), bool(return_correspondences))
+    out = {'transformation': T, 'fitness': fit, 'inlier_rmse': rmse, 'iterations': iters}
+    if return_correspondences:
+        out['correspondences'] = corr
+    return out
+
+
+_icp = icp       # register_pairs() and the meter take an `icp` argument of their own
+
+
+def evaluate_registration(src, tgt, max_correspondence_distance, T):
+    """Open3D's evaluate_registration for P pairs: correspondences of src under T [P,4,4] within the distance, and
+    -> dict(fitness [P] f64, inlier_rmse [P] f64, correspondences [P,n1] int32 (target index or -1))."""
+    r = icp(src, tgt, max_correspondence_distance, init=T, max_iter=0, return_correspondences=True)
+    return {'fitness': r['fitness'], 'inlier_rmse': r['inlier_rmse'], 'correspondences': r['correspondences']}
+
+
+def register_pairs(feat1, feat2, pt1, pt2, func='ransac', icp=None, **kw):
+    """feat1/feat2 [P,C,n] (the extractor's layout), pt1/pt2 [P,n,3], all CUDA -> (T [P,4,4], inliers [P], matches dict).
+    icp: None, or a dict of `icp()` keyword arguments (max_correspondence_distance required) to refine the pose with."""
     m = matcher.mutual_nn(feat1, feat2, point_major=False, want_dist=False)      # the meter uses the matches only
     T, inl = estimate_poses(pt1, pt2, m['idx1'], m['idx2'], m['count'], func=func, **kw)
+    if icp is not None:
+        T = _icp(pt1, pt2, init=T, **icp)['transformation']
     return T, inl, m
 
 
 class MeterModelNet40_registration:
     """Same state, thresholds and result keys as the reference meter (deepgmr_mn40.py:98-141)."""
 
-    def __init__(self, func='ransac', device='cuda'):
+    def __init__(self, func='ransac', device='cuda', icp=None):
+        """icp: None, or a dict of `icp()` keyword arguments; the RANSAC / Kabsch pose is then refined with it (inside
+        reg_time)."""
         self.rre = 0
         self.rte = 0
         self.num = 0
@@ -59,6 +107,7 @@ class MeterModelNet40_registration:
         self.translate_thresh = 0.005
         self.func = func
         self.device = torch.device(device)
+        self.icp = icp
 
     def update(self, output, target):
         """output = (feat1, feat2) [b,C,n]; target = (pt1 [b,n,3], pt2 [b,n,3], gt_trans [b,4,4]) — numpy or torch."""
@@ -68,7 +117,7 @@ class MeterModelNet40_registration:
             pt1, pt2, gt = (torch.as_tensor(t, dtype=torch.float32).to(dev) for t in target)
             torch.cuda.synchronize(dev)
             t0 = time.time()
-            T, _, _ = register_pairs(feat1, feat2, pt1, pt2, func=self.func)
+            T, _, _ = register_pairs(feat1, feat2, pt1, pt2, func=self.func, icp=self.icp)
             torch.cuda.synchronize(dev)
             reg_time = time.time() - t0
             m = registration_metrics(gt, T, pt1).cpu()
