@@ -298,6 +298,29 @@ int ri_icp_f32(const float* src, const float* tgt, const float* tgt_normals, con
                float* T, double* fitness, double* inlier_rmse, int* iters, int* corr,
                void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- normal estimation for xyz-only clouds (SURVEY.md 8f, row f6) ----------------------------------------------------
+ * Open3D's estimate_normals with KDTreeSearchParamHybrid(radius, max_nn) (the reference calls it on the host,
+ * utils/open3d_func.py:77-83), B clouds per call.  xyz [B,3,N] fp32; radius > 0 (+inf = plain k-NN), 1 <= max_nn <= 32.
+ * For each point q:
+ *   neighbours  the max_nn smallest keys (d, index) among the points with d < min(r2, 10000), q itself included, where
+ *               d = fma(dz,dz, fma(dy,dy, dx*dx)), d* = q - p in fp32, and r2 = radius * radius in fp32.  That is exactly
+ *               the first max_nn entries of ri_knn_grid_f32(xyz, xyz, k = max_nn) whose distance is < min(r2, 10000).
+ *               The radius cut is strict, as in ri_icp_f32 and ri_ball_query_f32;
+ *   covariance  p - q in fp64, accumulated over that list in its (d, index) order; C = S2/n - mu mu^T (population);
+ *   normal      unit eigenvector of the smallest eigenvalue of C (fp64 cyclic Jacobi, lowest index on equal eigenvalues),
+ *               rounded to fp32; (0,0,1) when fewer than 3 neighbours or when trace(C) is not positive and finite;
+ *   orientation camera [B,3]: flipped when n.(camera_b - q) < 0 (orient_normals_towards_camera_location); prior [B,3,N]:
+ *               flipped when n.prior < 0 (Open3D's rule for a cloud that has normals); neither: the solver's sign
+ *               (deterministic, not part of the contract).  At most one of camera / prior; the (0,0,1) default is
+ *               oriented too.
+ * Outputs normals [B,3,N] fp32 and, unless NULL, counts [B,N] int32 = neighbours used (q included).  No host
+ * synchronisation; a cloud's result does not depend on the rest of the batch and is bit-reproducible.
+ * workspace >= ri_knn_grid_workspace_bytes(B, N, N) bytes, 16-byte aligned.  RI_ERR_BAD_ARG for radius <= 0 or NaN,
+ * max_nn <= 0 or both camera and prior; RI_ERR_UNSUPPORTED for max_nn > 32 or B > 65535. */
+int ri_estimate_normals_f32(const float* xyz, int B, int N, float radius, int max_nn, const float* camera,
+                            const float* prior, float* normals, int* counts, void* workspace, size_t workspace_bytes,
+                            void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -3,7 +3,7 @@
 
 #include <string.h>
 
-extern "C" int ri_abi_version(void) { return 3; }
+extern "C" int ri_abi_version(void) { return 4; }
 
 // ---- environment knobs (DESIGN.md §11): read once per process, here
 namespace {

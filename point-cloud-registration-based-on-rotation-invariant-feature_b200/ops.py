@@ -820,3 +820,45 @@ def _(src, tgt, tgt_normals, init, r, point_to_plane, max_iter, rel_fitness, rel
     P, n1 = src.shape[0], src.shape[1]
     return (src.new_empty((P, 4, 4)), src.new_empty((P,), dtype=torch.float64), src.new_empty((P,), dtype=torch.float64),
             src.new_empty((P,), dtype=torch.int32), src.new_empty((P, n1 if want_corr else 0), dtype=torch.int32))
+
+
+# ---------------------------------------------------------------------------------------------- normal estimation (f6)
+@torch.library.custom_op("ri::estimate_normals", mutates_args=())
+def estimate_normals(xyz: torch.Tensor, radius: float, max_nn: int, camera: Optional[torch.Tensor],
+                     prior: Optional[torch.Tensor]) -> tuple[torch.Tensor, torch.Tensor]:
+    """xyz [B,3,N] f32, camera [B,3] or None, prior [B,3,N] or None -> (normals [B,3,N] f32, counts [B,N] i32).
+    Open3D's estimate_normals with the hybrid (radius, max_nn) search, every cloud of the batch in one call
+    (csrc/normals.cu); at most one of camera / prior orients the result."""
+    _req(xyz, "xyz", torch.float32)
+    ts = (xyz,)
+    if camera is not None:
+        _req(camera, "camera", torch.float32)
+        ts = ts + (camera,)
+    if prior is not None:
+        _req(prior, "prior", torch.float32)
+        ts = ts + (prior,)
+    dev = _same_device(*ts)
+    _shape(xyz, "xyz", None, 3, None)
+    B, _, N = xyz.shape
+    if camera is not None:
+        _shape(camera, "camera", B, 3)
+    if prior is not None:
+        _shape(prior, "prior", B, 3, N)
+    if camera is not None and prior is not None:
+        raise RuntimeError("orient normals by a camera or by a prior, not both")
+    with torch.cuda.device(dev):
+        nrm = torch.empty((B, 3, N), dtype=torch.float32, device=dev)
+        cnt = torch.empty((B, N), dtype=torch.int32, device=dev)
+        nws = _L.ri_knn_grid_workspace_bytes(B, N, N)
+        ws = torch.empty(nws, dtype=torch.uint8, device=dev)
+        _check(_L.ri_estimate_normals_f32(xyz.data_ptr(), B, N, float(radius), int(max_nn),
+                                          camera.data_ptr() if camera is not None else None,
+                                          prior.data_ptr() if prior is not None else None, nrm.data_ptr(), cnt.data_ptr(),
+                                          ws.data_ptr(), nws, _stream()), "ri_estimate_normals")
+    return nrm, cnt
+
+
+@estimate_normals.register_fake
+def _(xyz, radius, max_nn, camera, prior):
+    B, _, N = xyz.shape
+    return xyz.new_empty((B, 3, N)), xyz.new_empty((B, N), dtype=torch.int32)
