@@ -261,8 +261,19 @@ int ri_grid_subsample_f32(const float* points, const float* features, const int*
  * edge-length similarity 0.9, sample residual and validation distance = voxel_size, max_iter hypotheses, point-to-point
  * least squares without scale), all pairs in one launch, then Horn's closed-form refit on the inliers.
  * src [P,n1,3], tgt [P,n2,3] point-major fp32; idx1, idx2 [P,ld], count [P] as ri_mutual_nn_tf32x3 returns them;
- * hyps == 0: least squares over all matches (Kabsch).  T [P,4,4] row-major fp32 (src -> tgt), inliers [P];
- * best: P * 8 bytes of scratch (may be NULL when hyps == 0). */
+ * hyps == 0: least squares over all matches (Kabsch).  T [P,4,4] row-major fp32 (src -> tgt), inliers [P].
+ * Every match counts: min(count[p], ld) matches, any number (they are staged in shared memory 4096 at a time); sampling,
+ * inlier counts, the refit and the Kabsch solve all run over all of them.
+ * Sampler: hypothesis h < hyps of pair p uses matches (i0, i1, i2) = sample3(seed, p, h, M), M = the pair's match count:
+ *   mix64 = the splitmix64 finaliser (x += 0x9E3779B97F4A7C15; x = (x ^ x>>30) * 0xBF58476D1CE4E5B9;
+ *           x = (x ^ x>>27) * 0x94D049BB133111EB; x ^ x>>31), all uint64 with wrap-around;
+ *   r0 = mix64(seed ^ (p << 32) ^ (uint32)h), r1 = mix64(r0), r2 = mix64(r1);
+ *   i0 = r0 % M; i1 = r1 % (M-1), +1 if >= i0; i2 = r2 % (M-2), +1 if >= min(i0,i1), +1 more if then >= max(i0,i1).
+ * The winner is the valid hypothesis with the most inliers, the lowest h on ties.
+ * best: P * 8 bytes of scratch (may be NULL when hyps == 0).  With hyps > 0 it holds, after the call, the winner of each
+ * pair as (inliers << 32) | (0xffffffff - h), or 0 when no hypothesis passed its checks.
+ * inliers[p] is always the count under the returned T[p]; when no pose was found (fewer than 3 matches, or no valid
+ * hypothesis) T[p] is the identity and inliers[p] is 0. */
 int ri_pose_from_matches_f32(const float* src, const float* tgt, const int* idx1, const int* idx2, const int* count,
                              int P, int n1, int n2, int ld, int hyps, float inlier_dist, float edge_similarity,
                              int refine_iters, unsigned long long seed, float* T, int* inliers,

@@ -30,7 +30,8 @@ namespace {
 
 constexpr int kHypThreads = 128;
 constexpr int kRefThreads = 256;
-constexpr int kMaxMatches = 4096;        // matched coordinates staged per pair: 6 floats each (96 KB at the cap)
+constexpr int kMaxMatches = 4096;        // matched coordinates staged per pair at a time: 6 floats each (96 KB); more
+                                         // matches are processed in chunks of this size
 
 __device__ __forceinline__ uint64_t mix64(uint64_t x)          // splitmix64 finaliser
 {
@@ -78,11 +79,43 @@ __device__ __forceinline__ bool tri_frame(float3 p0, float3 p1, float3 p2, float
     return true;
 }
 
-// hypothesis of one minimal sample: checks of open3d_func.py:46-48, rotation from the two triangle frames
-__device__ __forceinline__ bool hypothesis(const float3* __restrict__ A, const float3* __restrict__ Bm, int i0, int i1, int i2,
-                                           float edge_sim, float thresh, Rt& T)
+// the matched coordinates of pair p, read through the match lists: a(m) = src[idx1[m]], b(m) = tgt[idx2[m]]
+struct PairMatches {
+    const float* S; const float* Tg; const int* i1; const int* i2; int n1, n2;
+    __device__ __forceinline__ PairMatches(const float* src, const float* tgt, const int* idx1, const int* idx2, int p,
+                                           int n1_, int n2_, int ld)
+        : S(src + (size_t)p * n1_ * 3), Tg(tgt + (size_t)p * n2_ * 3), i1(idx1 + (size_t)p * ld), i2(idx2 + (size_t)p * ld),
+          n1(n1_), n2(n2_) {}
+    __device__ __forceinline__ void load(int m, float3& a, float3& b) const
+    {
+        int i = i1[m], j = i2[m];
+        i = i < 0 ? 0 : (i >= n1 ? n1 - 1 : i);
+        j = j < 0 ? 0 : (j >= n2 ? n2 - 1 : j);
+        a = make_float3(S[3 * i], S[3 * i + 1], S[3 * i + 2]);
+        b = make_float3(Tg[3 * j], Tg[3 * j + 1], Tg[3 * j + 2]);
+    }
+};
+
+// number of matches of pair p: count[p] clamped to [0, ld].  Every match is used; at most kMaxMatches are staged at once.
+__device__ __forceinline__ int match_count(const int* __restrict__ count, int p, int ld)
 {
-    const float3 a0 = A[i0], a1 = A[i1], a2 = A[i2], b0 = Bm[i0], b1 = Bm[i1], b2 = Bm[i2];
+    const int M = count[p];
+    return M < 0 ? 0 : (M > ld ? ld : M);
+}
+
+// stage matches [base, base + kMaxMatches) of [0, M) into A, Bm (the whole pair when M <= kMaxMatches); returns their number
+__device__ __forceinline__ int stage_matches(const PairMatches& pm, int base, int M, float3* A, float3* Bm)
+{
+    const int len = min(M - base, kMaxMatches);
+    for (int m = threadIdx.x; m < len; m += blockDim.x) pm.load(base + m, A[m], Bm[m]);
+    __syncthreads();
+    return len;
+}
+
+// hypothesis of one minimal sample: checks of open3d_func.py:46-48, rotation from the two triangle frames
+__device__ __forceinline__ bool hypothesis(float3 a0, float3 a1, float3 a2, float3 b0, float3 b1, float3 b2, float edge_sim,
+                                           float thresh, Rt& T)
+{
     // edge-length similarity: every edge of the source triangle within [sim, 1/sim] of the target's
     const float ea[3] = {sqrtf(f3dot(f3sub(a0, a1), f3sub(a0, a1))), sqrtf(f3dot(f3sub(a1, a2), f3sub(a1, a2))),
                          sqrtf(f3dot(f3sub(a2, a0), f3sub(a2, a0)))};
@@ -115,6 +148,18 @@ __device__ __forceinline__ bool hypothesis(const float3* __restrict__ A, const f
     return true;
 }
 
+// hypothesis h of pair p: its sample3 triple, read from shared memory when the whole pair is staged, else from global
+__device__ __forceinline__ bool sample_hypothesis(const PairMatches& pm, const float3* A, const float3* Bm, int M,
+                                                  unsigned long long seed, int p, int h, float edge_sim, float thresh, Rt& T)
+{
+    int i0, i1, i2;
+    sample3(seed, p, h, M, i0, i1, i2);
+    float3 a0, a1, a2, b0, b1, b2;
+    if (M <= kMaxMatches) { a0 = A[i0]; a1 = A[i1]; a2 = A[i2]; b0 = Bm[i0]; b1 = Bm[i1]; b2 = Bm[i2]; }
+    else { pm.load(i0, a0, b0); pm.load(i1, a1, b1); pm.load(i2, a2, b2); }
+    return hypothesis(a0, a1, a2, b0, b1, b2, edge_sim, thresh, T);
+}
+
 __device__ __forceinline__ bool inlier(const Rt& T, float3 a, float3 b, float t2h)
 {
     const float dx = T.r[0] * a.x + T.r[1] * a.y + T.r[2] * a.z + T.t[0] - b.x;
@@ -123,26 +168,17 @@ __device__ __forceinline__ bool inlier(const Rt& T, float3 a, float3 b, float t2
     return dx * dx + dy * dy + dz * dz < t2h;
 }
 
-// stage the matched coordinates of pair p: A[m] = src[idx1[m]], Bm[m] = tgt[idx2[m]]
-__device__ __forceinline__ int stage_matches(const float* __restrict__ src, const float* __restrict__ tgt,
-                                             const int* __restrict__ idx1, const int* __restrict__ idx2,
-                                             const int* __restrict__ count, int p, int n1, int n2, int ld,
-                                             float3* A, float3* Bm)
+// one block-strided pass over all M matches of the pair: f(a, b) for each.  `staged` is the base of the chunk held in
+// A / Bm; with M <= kMaxMatches that is the whole pair and nothing is restaged, otherwise the pass walks the chunks in
+// order and every thread of the block takes part in each restaging barrier.
+template <class F>
+__device__ __forceinline__ void for_each_match(const PairMatches& pm, int M, int& staged, float3* A, float3* Bm, F f)
 {
-    int M = count[p];
-    M = M < 0 ? 0 : (M > ld ? ld : M);
-    M = M > kMaxMatches ? kMaxMatches : M;
-    const float* S = src + (size_t)p * n1 * 3;
-    const float* Tg = tgt + (size_t)p * n2 * 3;
-    for (int m = threadIdx.x; m < M; m += blockDim.x) {
-        int i = idx1[(size_t)p * ld + m], j = idx2[(size_t)p * ld + m];
-        i = i < 0 ? 0 : (i >= n1 ? n1 - 1 : i);
-        j = j < 0 ? 0 : (j >= n2 ? n2 - 1 : j);
-        A[m] = make_float3(S[3 * i], S[3 * i + 1], S[3 * i + 2]);
-        Bm[m] = make_float3(Tg[3 * j], Tg[3 * j + 1], Tg[3 * j + 2]);
+    for (int base = 0; base < M; base += kMaxMatches) {
+        if (base != staged) { __syncthreads(); stage_matches(pm, base, M, A, Bm); staged = base; }
+        const int len = min(M - base, kMaxMatches);
+        for (int m = threadIdx.x; m < len; m += blockDim.x) f(A[m], Bm[m]);
     }
-    __syncthreads();
-    return M;
 }
 
 __global__ void __launch_bounds__(kHypThreads)
@@ -154,17 +190,24 @@ pose_ransac_kernel(const float* __restrict__ src, const float* __restrict__ tgt,
     const int p = blockIdx.y;
     float3* A = pose_smem;
     float3* Bm = pose_smem + min(ld, kMaxMatches);
-    const int M = stage_matches(src, tgt, idx1, idx2, count, p, n1, n2, ld, A, Bm);
+    const PairMatches pm(src, tgt, idx1, idx2, p, n1, n2, ld);
+    const int M = match_count(count, p, ld);
+    int len = stage_matches(pm, 0, M, A, Bm);
     const int h = blockIdx.x * kHypThreads + threadIdx.x;
-    if (M < 3 || h >= hyps) return;
-    int i0, i1, i2;
-    sample3(seed, p, h, M, i0, i1, i2);
+    if (M < 3) return;                                   // uniform over the block
     Rt T;
-    if (!hypothesis(A, Bm, i0, i1, i2, edge_sim, thresh, T)) return;
+    const bool valid = h < hyps && sample_hypothesis(pm, A, Bm, M, seed, p, h, edge_sim, thresh, T);
     const float t2h = thresh * thresh;
     int n = 0;
-    for (int m = 0; m < M; ++m) n += inlier(T, A[m], Bm[m], t2h) ? 1 : 0;
-    atomicMax(best + p, ((unsigned long long)(unsigned)n << 32) | (unsigned long long)(0xffffffffu - (unsigned)h));
+    for (int base = 0;;) {                               // every thread walks the chunks: the barriers are block-wide
+        if (valid)
+            for (int m = 0; m < len; ++m) n += inlier(T, A[m], Bm[m], t2h) ? 1 : 0;
+        base += kMaxMatches;
+        if (base >= M) break;
+        __syncthreads();
+        len = stage_matches(pm, base, M, A, Bm);
+    }
+    if (valid) atomicMax(best + p, ((unsigned long long)(unsigned)n << 32) | (unsigned long long)(0xffffffffu - (unsigned)h));
 }
 
 // use_all != 0: plain least squares over ALL matches (the Kabsch solve alone; no RANSAC seed needed)
@@ -177,12 +220,15 @@ pose_refine_kernel(const float* __restrict__ src, const float* __restrict__ tgt,
     extern __shared__ float3 pose_smem[];
     __shared__ double red[(kRefThreads / 32) * 9];
     __shared__ Rt Tcur;
-    __shared__ int ok;
+    __shared__ int ok, posed;
     __shared__ double cen[6];
     const int p = blockIdx.x;
     float3* A = pose_smem;
     float3* Bm = pose_smem + min(ld, kMaxMatches);
-    const int M = stage_matches(src, tgt, idx1, idx2, count, p, n1, n2, ld, A, Bm);
+    const PairMatches pm(src, tgt, idx1, idx2, p, n1, n2, ld);
+    const int M = match_count(count, p, ld);
+    stage_matches(pm, 0, M, A, Bm);
+    int staged = 0;
     const float t2h = thresh * thresh;
     if (threadIdx.x == 0) {
         ok = 0;
@@ -195,22 +241,22 @@ pose_refine_kernel(const float* __restrict__ src, const float* __restrict__ tgt,
                 const unsigned long long key = best[p];
                 if (key != 0ull) {
                     const int h = (int)(0xffffffffu - (unsigned)(key & 0xffffffffull));
-                    int i0, i1, i2;
-                    sample3(seed, p, h, M, i0, i1, i2);
                     Rt T;
-                    if (hypothesis(A, Bm, i0, i1, i2, edge_sim, thresh, T)) { Tcur = T; ok = 1; }
+                    if (sample_hypothesis(pm, A, Bm, M, seed, p, h, edge_sim, thresh, T)) { Tcur = T; ok = 1; }
                 }
             }
         }
+        posed = ok;                                      // a pose exists; ok may still drop during the refit
     }
     __syncthreads();
     for (int it = 0; it < iters && ok; ++it) {
         const Rt T = Tcur;
         double s[7] = {0, 0, 0, 0, 0, 0, 0};
-        for (int m = threadIdx.x; m < M; m += kRefThreads)
-            if (use_all || inlier(T, A[m], Bm[m], t2h)) {
-                s[0] += 1.0; s[1] += A[m].x; s[2] += A[m].y; s[3] += A[m].z; s[4] += Bm[m].x; s[5] += Bm[m].y; s[6] += Bm[m].z;
+        for_each_match(pm, M, staged, A, Bm, [&](float3 a, float3 b) {
+            if (use_all || inlier(T, a, b, t2h)) {
+                s[0] += 1.0; s[1] += a.x; s[2] += a.y; s[3] += a.z; s[4] += b.x; s[5] += b.y; s[6] += b.z;
             }
+        });
         block_sum<7>(s, red);
         if (threadIdx.x == 0) {
             if (s[0] < 3.0) ok = 0;
@@ -220,14 +266,15 @@ pose_refine_kernel(const float* __restrict__ src, const float* __restrict__ tgt,
         if (!ok) break;
         double h9[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
         const double cax = cen[0], cay = cen[1], caz = cen[2], cbx = cen[3], cby = cen[4], cbz = cen[5];
-        for (int m = threadIdx.x; m < M; m += kRefThreads)
-            if (use_all || inlier(T, A[m], Bm[m], t2h)) {
-                const double ax = A[m].x - cax, ay = A[m].y - cay, az = A[m].z - caz;
-                const double bx = Bm[m].x - cbx, by = Bm[m].y - cby, bz = Bm[m].z - cbz;
+        for_each_match(pm, M, staged, A, Bm, [&](float3 a, float3 b) {
+            if (use_all || inlier(T, a, b, t2h)) {
+                const double ax = a.x - cax, ay = a.y - cay, az = a.z - caz;
+                const double bx = b.x - cbx, by = b.y - cby, bz = b.z - cbz;
                 h9[0] += ax * bx; h9[1] += ax * by; h9[2] += ax * bz;
                 h9[3] += ay * bx; h9[4] += ay * by; h9[5] += ay * bz;
                 h9[6] += az * bx; h9[7] += az * by; h9[8] += az * bz;
             }
+        });
         block_sum<9>(h9, red);
         if (threadIdx.x == 0) {
             double R[9];
@@ -240,10 +287,11 @@ pose_refine_kernel(const float* __restrict__ src, const float* __restrict__ tgt,
         }
         __syncthreads();
     }
-    // final inlier count under the returned pose
+    // final inlier count under the returned pose (also when a refit round fell below 3 inliers and kept the pose
+    // that round was evaluated under); no pose at all -> identity, 0 inliers
     const Rt T = Tcur;
     double c1[1] = {0};
-    for (int m = threadIdx.x; m < M; m += kRefThreads) c1[0] += inlier(T, A[m], Bm[m], t2h) ? 1.0 : 0.0;
+    for_each_match(pm, M, staged, A, Bm, [&](float3 a, float3 b) { c1[0] += inlier(T, a, b, t2h) ? 1.0 : 0.0; });
     block_sum<1>(c1, red);
     if (threadIdx.x == 0) {
         float* O = T_out + (size_t)p * 16;
@@ -251,7 +299,7 @@ pose_refine_kernel(const float* __restrict__ src, const float* __restrict__ tgt,
         O[4] = T.r[3]; O[5] = T.r[4]; O[6] = T.r[5]; O[7] = T.t[1];
         O[8] = T.r[6]; O[9] = T.r[7]; O[10] = T.r[8]; O[11] = T.t[2];
         O[12] = 0.f; O[13] = 0.f; O[14] = 0.f; O[15] = 1.f;
-        inliers_out[p] = ok ? (int)c1[0] : 0;
+        inliers_out[p] = posed ? (int)c1[0] : 0;
     }
 }
 

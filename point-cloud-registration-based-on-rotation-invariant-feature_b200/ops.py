@@ -651,7 +651,16 @@ def pose_from_matches(src: torch.Tensor, tgt: torch.Tensor, idx1: torch.Tensor, 
     _req(src, "src", torch.float32); _req(tgt, "tgt", torch.float32)
     _req(idx1, "idx1", torch.int32); _req(idx2, "idx2", torch.int32); _req(count, "count", torch.int32)
     dev = _same_device(src, tgt, idx1, idx2, count)
+    _shape(src, "src", None, None, 3)
     P, n1, _ = src.shape
+    _shape(tgt, "tgt", P, None, 3)
+    _shape(idx1, "idx1", P, None)
+    _shape(idx2, "idx2", P, idx1.shape[1])
+    _shape(count, "count", P)
+    if int(refine_iters) < 1:
+        raise RuntimeError("refine_iters must be >= 1")
+    if not float(inlier_dist) > 0.0:
+        raise RuntimeError("inlier_dist must be > 0")
     n2 = tgt.shape[1]
     ld = idx1.shape[1]
     with torch.cuda.device(dev):
