@@ -332,6 +332,39 @@ int ri_estimate_normals_f32(const float* xyz, int B, int N, float radius, int ma
                             const float* prior, float* normals, int* counts, void* workspace, size_t workspace_bytes,
                             void* stream);
 
+/* ---- Fast Global Registration (SURVEY.md 8f, row f7) -----------------------------------------------------------------
+ * Open3D's registration_fgr_based_on_feature_matching (Zhou, Park, Koltun, ECCV 2016; the reference's alternative to RANSAC,
+ * utils/open3d_func.py:50-62) over the mutual matches, P pairs in one launch.  src, tgt, idx1, idx2, count as in
+ * ri_pose_from_matches_f32: pair p has M = min(count[p], ld) matches, match m pairs a_m = src[idx1[m]] with b_m = tgt[idx2[m]].
+ *   tuple test  (tuple_test != 0; AdvancedMatching)  trial t = 0, 1, ... < 100 M draws r0 = mix64(seed ^ (p << 32) ^ (uint32)t),
+ *               r1 = mix64(r0), r2 = mix64(r1) (mix64 as in ri_pose_from_matches_f32) and i_k = r_k % M, independently.
+ *               Edge lengths |a_i0 - a_i1|, |a_i1 - a_i2|, |a_i2 - a_i0| (and the same over the b's) are computed in fp64 from
+ *               the fp32 coordinates as sqrt((dx*dx + dy*dy) + dz*dz), each operation rounded (no contraction).  The trial is
+ *               accepted when every edge has l_a * s < l_b && l_b < l_a / s, s = (double)tuple_scale.  The list is
+ *               (i0, i1, i2) of each of the first max_tuples accepted trials, in trial order; fewer when the trials run out.
+ *               tuple_test == 0: the list is the M matches in order.
+ *   normalise   mu_s, mu_t = means of all n1 source / n2 target points (fp64); scale = the largest |x - mu| over both clouds;
+ *               g = scale, par = 1 (use_absolute_scale == 0) or g = 1, par = scale; points are used as (x - mu) * (1 / g).
+ *   GNC         (fp64) T' = I moves the normalised target onto the normalised source; per iteration it < iterations:
+ *               par /= division_factor when decrease_mu && it % 4 == 0 && par > max_corr_dist; per correspondence q = T' q^,
+ *               r = p^ - q, w = (par / (r.r + par))^2, rows r_x: J = (0, -q_z, q_y, -1, 0, 0), r_y: (q_z, 0, -q_x, 0, -1, 0),
+ *               r_z: (-q_y, q_x, 0, 0, 0, -1); x = -(J^T W J)^-1 J^T W r (Delta = I when a pivot of the LDL^T factorisation is
+ *               not positive or x is not finite); T' = [Rz(x2) Ry(x1) Rx(x0) | x3 x4 x5] T'.
+ *   output      T[p] = inverse of [R' | mu_s - R' mu_t + g t'] (maps src onto tgt), rounded to fp32, row-major [4,4];
+ *               inliers[p] = #{m < M : |R a_m + t - b_m|^2 < inlier_dist^2} under that fp32 T, with the arithmetic of
+ *               ri_pose_from_matches_f32.  No pose (M < 3 or a list shorter than 10): T[p] = I and inliers[p] = 0.
+ * corr [P, 3 * max_tuples] receives the list's match positions, -1 past its end; required when tuple_test != 0 (the list is
+ * read back from it), may be NULL otherwise (and is not written).  ncorr [P] = the list's length (3 x accepted trials, or M).
+ * No host synchronisation; a pair's result is bit-reproducible and does not depend on the rest of the batch.
+ * RI_ERR_BAD_ARG for max_corr_dist <= 0, iterations < 0, division_factor <= 1, tuple_scale outside (0, 1], max_tuples < 1,
+ * inlier_dist <= 0, or corr == NULL with tuple_test != 0; RI_ERR_UNSUPPORTED for 100 * ld >= 2^32 (the trial index is
+ * 32-bit) or max_tuples > INT_MAX / 3. */
+int ri_fgr_f32(const float* src, const float* tgt, const int* idx1, const int* idx2, const int* count,
+               int P, int n1, int n2, int ld, float max_corr_dist, int iterations, float division_factor,
+               int use_absolute_scale, int decrease_mu, int tuple_test, float tuple_scale, int max_tuples,
+               unsigned long long seed, float inlier_dist, float* T, int* inliers, int* corr, int* ncorr,
+               void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -383,7 +383,7 @@ icp_iter_kernel(const float* __restrict__ src, int P, int n1, int n2, float r, i
         double b[6], x[6];
 #pragma unroll
         for (int a = 0; a < 6; ++a) b[a] = -tot[23 + a];
-        if (ldlt_solve6(tot + 2, b, x)) {
+        if (ldlt_solve6(tot + 2, b, x, 1e-6)) {
             const double ca = cos(x[0]), sa = sin(x[0]), cb = cos(x[1]), sb = sin(x[1]), cg = cos(x[2]), sg = sin(x[2]);
             // Rz(x2) Ry(x1) Rx(x0)
             U[0] = cg * cb; U[1] = cg * sb * sa - sg * ca; U[2] = cg * sb * ca + sg * sa; U[3] = x[3];

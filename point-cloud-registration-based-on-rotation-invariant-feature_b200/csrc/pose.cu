@@ -25,6 +25,7 @@
 //   pose_metrics_kernel  one CTA per pair: RRE (degrees), RTE, RMSE exactly as the reference's meter computes them.
 #include "ri_common.cuh"
 #include "rigid.cuh"
+#include "matches.cuh"
 
 namespace {
 
@@ -32,14 +33,6 @@ constexpr int kHypThreads = 128;
 constexpr int kRefThreads = 256;
 constexpr int kMaxMatches = 4096;        // matched coordinates staged per pair at a time: 6 floats each (96 KB); more
                                          // matches are processed in chunks of this size
-
-__device__ __forceinline__ uint64_t mix64(uint64_t x)          // splitmix64 finaliser
-{
-    x += 0x9E3779B97F4A7C15ull;
-    x = (x ^ (x >> 30)) * 0xBF58476D1CE4E5B9ull;
-    x = (x ^ (x >> 27)) * 0x94D049BB133111EBull;
-    return x ^ (x >> 31);
-}
 
 // three distinct indices in [0, M), M >= 3, from (seed, pair, hypothesis)
 __device__ __forceinline__ void sample3(uint64_t seed, int pair, int hyp, int M, int& i0, int& i1, int& i2)
@@ -53,8 +46,6 @@ __device__ __forceinline__ void sample3(uint64_t seed, int pair, int hyp, int M,
     if (i2 >= lo) ++i2;
     if (i2 >= hi) ++i2;
 }
-
-struct Rt { float r[9]; float t[3]; };
 
 __device__ __forceinline__ float3 f3sub(float3 a, float3 b) { return make_float3(a.x - b.x, a.y - b.y, a.z - b.z); }
 __device__ __forceinline__ float f3dot(float3 a, float3 b) { return a.x * b.x + a.y * b.y + a.z * b.z; }
@@ -77,30 +68,6 @@ __device__ __forceinline__ bool tri_frame(float3 p0, float3 p1, float3 p2, float
     e2 = f3scale(w, 1.0f / nw);
     e3 = f3cross(e1, e2);
     return true;
-}
-
-// the matched coordinates of pair p, read through the match lists: a(m) = src[idx1[m]], b(m) = tgt[idx2[m]]
-struct PairMatches {
-    const float* S; const float* Tg; const int* i1; const int* i2; int n1, n2;
-    __device__ __forceinline__ PairMatches(const float* src, const float* tgt, const int* idx1, const int* idx2, int p,
-                                           int n1_, int n2_, int ld)
-        : S(src + (size_t)p * n1_ * 3), Tg(tgt + (size_t)p * n2_ * 3), i1(idx1 + (size_t)p * ld), i2(idx2 + (size_t)p * ld),
-          n1(n1_), n2(n2_) {}
-    __device__ __forceinline__ void load(int m, float3& a, float3& b) const
-    {
-        int i = i1[m], j = i2[m];
-        i = i < 0 ? 0 : (i >= n1 ? n1 - 1 : i);
-        j = j < 0 ? 0 : (j >= n2 ? n2 - 1 : j);
-        a = make_float3(S[3 * i], S[3 * i + 1], S[3 * i + 2]);
-        b = make_float3(Tg[3 * j], Tg[3 * j + 1], Tg[3 * j + 2]);
-    }
-};
-
-// number of matches of pair p: count[p] clamped to [0, ld].  Every match is used; at most kMaxMatches are staged at once.
-__device__ __forceinline__ int match_count(const int* __restrict__ count, int p, int ld)
-{
-    const int M = count[p];
-    return M < 0 ? 0 : (M > ld ? ld : M);
 }
 
 // stage matches [base, base + kMaxMatches) of [0, M) into A, Bm (the whole pair when M <= kMaxMatches); returns their number
@@ -158,14 +125,6 @@ __device__ __forceinline__ bool sample_hypothesis(const PairMatches& pm, const f
     if (M <= kMaxMatches) { a0 = A[i0]; a1 = A[i1]; a2 = A[i2]; b0 = Bm[i0]; b1 = Bm[i1]; b2 = Bm[i2]; }
     else { pm.load(i0, a0, b0); pm.load(i1, a1, b1); pm.load(i2, a2, b2); }
     return hypothesis(a0, a1, a2, b0, b1, b2, edge_sim, thresh, T);
-}
-
-__device__ __forceinline__ bool inlier(const Rt& T, float3 a, float3 b, float t2h)
-{
-    const float dx = T.r[0] * a.x + T.r[1] * a.y + T.r[2] * a.z + T.t[0] - b.x;
-    const float dy = T.r[3] * a.x + T.r[4] * a.y + T.r[5] * a.z + T.t[1] - b.y;
-    const float dz = T.r[6] * a.x + T.r[7] * a.y + T.r[8] * a.z + T.t[2] - b.z;
-    return dx * dx + dy * dy + dz * dz < t2h;
 }
 
 // one block-strided pass over all M matches of the pair: f(a, b) for each.  `staged` is the base of the chunk held in

@@ -1,4 +1,4 @@
-// rigid.cuh — fp64 rigid-transform solvers and the block reduction shared by csrc/pose.cu and csrc/icp.cu.
+// rigid.cuh — fp64 rigid-transform solvers and the block reduction shared by csrc/pose.cu, csrc/icp.cu and csrc/fgr.cu.
 #pragma once
 #include <cuda_runtime.h>
 
@@ -86,9 +86,12 @@ __device__ void block_sum(double (&v)[NV], double* red)
 
 // Solves A x = b for the symmetric 6x6 A given by its 21 upper-triangle entries in row order (A00 A01 .. A05 A11 .. A55),
 // by an LDL^T factorisation without pivoting (A = J^T J is positive semi-definite).  det = prod(D) = det(A).  Returns false
-// when |det| < 1e-6 or the factorisation or the solution is not finite — Open3D's SolveLinearSystemPSD rejects the same
-// systems, and its caller (SolveJacobianSystemAndObtainExtrinsicMatrix) then returns the identity.
-__device__ bool ldlt_solve6(const double up[21], const double b[6], double x[6])
+// when the factorisation or the solution is not finite, and
+//   min_det > 0:  when |det| < min_det.  ICP passes 1e-6: Open3D's SolveLinearSystemPSD rejects the same systems, and its
+//                 caller (SolveJacobianSystemAndObtainExtrinsicMatrix) then returns the identity;
+//   min_det <= 0: when a pivot D[j] is not positive, i.e. A is not numerically positive definite (FGR: where an LLT
+//                 factorisation would break down).
+__device__ bool ldlt_solve6(const double up[21], const double b[6], double x[6], double min_det)
 {
     double L[6][6], D[6];
     double A[6][6];
@@ -98,6 +101,7 @@ __device__ bool ldlt_solve6(const double up[21], const double b[6], double x[6])
 #pragma unroll
         for (int j = i; j < 6; ++j) { A[i][j] = up[k]; A[j][i] = up[k]; ++k; }
     double det = 1.0;
+    bool pd = true;
 #pragma unroll
     for (int j = 0; j < 6; ++j) {
         double d = A[j][j];
@@ -105,6 +109,7 @@ __device__ bool ldlt_solve6(const double up[21], const double b[6], double x[6])
         for (int m = 0; m < j; ++m) d -= L[j][m] * L[j][m] * D[m];
         D[j] = d;
         det *= d;
+        pd = pd && d > 0.0;
 #pragma unroll
         for (int i = j + 1; i < 6; ++i) {
             double s = A[i][j];
@@ -113,7 +118,7 @@ __device__ bool ldlt_solve6(const double up[21], const double b[6], double x[6])
             L[i][j] = s / d;
         }
     }
-    if (!(fabs(det) >= 1e-6) || !isfinite(det)) return false;
+    if ((min_det > 0.0 ? !(fabs(det) >= min_det) : !pd) || !isfinite(det)) return false;
     double y[6];
 #pragma unroll
     for (int i = 0; i < 6; ++i) {                      // L y = b

@@ -871,3 +871,56 @@ def estimate_normals(xyz: torch.Tensor, radius: float, max_nn: int, camera: Opti
 def _(xyz, radius, max_nn, camera, prior):
     B, _, N = xyz.shape
     return xyz.new_empty((B, 3, N)), xyz.new_empty((B, N), dtype=torch.int32)
+
+
+# ---------------------------------------------------------------------------------------------- Fast Global Registration (f7)
+@torch.library.custom_op("ri::fgr", mutates_args=())
+def fgr(src: torch.Tensor, tgt: torch.Tensor, idx1: torch.Tensor, idx2: torch.Tensor, count: torch.Tensor,
+        max_corr_dist: float, iterations: int, division_factor: float, use_absolute_scale: bool, decrease_mu: bool,
+        tuple_test: bool, tuple_scale: float, max_tuples: int, seed: int, inlier_dist: float) -> tuple[
+        torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    """src [P,n1,3], tgt [P,n2,3] f32; idx1/idx2 [P,ld], count [P] i32 (mutual matches) -> (T [P,4,4] f32 src->tgt,
+    inliers [P] i32, corr [P,3*max_tuples] i32 (the tuple list's match positions, -1 padded; [P,0] without the tuple test),
+    ncorr [P] i32).  Open3D's FGR per pair, all pairs in one launch (csrc/fgr.cu)."""
+    _req(src, "src", torch.float32); _req(tgt, "tgt", torch.float32)
+    _req(idx1, "idx1", torch.int32); _req(idx2, "idx2", torch.int32); _req(count, "count", torch.int32)
+    dev = _same_device(src, tgt, idx1, idx2, count)
+    _shape(src, "src", None, None, 3)
+    P, n1, _ = src.shape
+    _shape(tgt, "tgt", P, None, 3)
+    _shape(idx1, "idx1", P, None)
+    _shape(idx2, "idx2", P, idx1.shape[1])
+    _shape(count, "count", P)
+    if not float(max_corr_dist) > 0.0:
+        raise RuntimeError("maximum_correspondence_distance must be > 0")
+    if int(iterations) < 0:
+        raise RuntimeError("iteration_number must be >= 0")
+    if not float(division_factor) > 1.0:
+        raise RuntimeError("division_factor must be > 1")
+    if not 0.0 < float(tuple_scale) <= 1.0:
+        raise RuntimeError("tuple_scale must be in (0, 1]")
+    if not 1 <= int(max_tuples) <= 0x7FFFFFFF // 3:
+        raise RuntimeError("maximum_tuple_count must be in [1, %d]" % (0x7FFFFFFF // 3))
+    if not float(inlier_dist) > 0.0:
+        raise RuntimeError("inlier_dist must be > 0")
+    n2 = tgt.shape[1]
+    ld = idx1.shape[1]
+    with torch.cuda.device(dev):
+        T = torch.empty((P, 4, 4), dtype=torch.float32, device=dev)
+        inl = torch.empty((P,), dtype=torch.int32, device=dev)
+        corr = torch.empty((P, 3 * int(max_tuples) if tuple_test else 0), dtype=torch.int32, device=dev)
+        ncorr = torch.empty((P,), dtype=torch.int32, device=dev)
+        _check(_L.ri_fgr_f32(src.data_ptr(), tgt.data_ptr(), idx1.data_ptr(), idx2.data_ptr(), count.data_ptr(),
+                             P, n1, n2, ld, float(max_corr_dist), int(iterations), float(division_factor),
+                             int(use_absolute_scale), int(decrease_mu), int(tuple_test), float(tuple_scale), int(max_tuples),
+                             int(seed) & 0xFFFFFFFFFFFFFFFF, float(inlier_dist), T.data_ptr(), inl.data_ptr(),
+                             corr.data_ptr() if tuple_test else None, ncorr.data_ptr(), _stream()), "ri_fgr")
+    return T, inl, corr, ncorr
+
+
+@fgr.register_fake
+def _(src, tgt, idx1, idx2, count, max_corr_dist, iterations, division_factor, use_absolute_scale, decrease_mu, tuple_test,
+      tuple_scale, max_tuples, seed, inlier_dist):
+    P = src.shape[0]
+    return (src.new_empty((P, 4, 4)), count.new_empty((P,)), count.new_empty((P, 3 * max_tuples if tuple_test else 0)),
+            count.new_empty((P,)))

@@ -1,16 +1,16 @@
 """Registration back end on the GPU: descriptors -> mutual matches -> rigid pose -> ICP refinement -> RRE / RTE / RMSE,
-whole batches of pairs per call (csrc/matcher.cu + csrc/pose.cu + csrc/icp.cu).
+whole batches of pairs per call (csrc/matcher.cu + csrc/pose.cu + csrc/fgr.cu + csrc/icp.cu).
 
 Mirrors the reference's meter `MeterModelNet40_registration` (/root/reference/datasets/deepgmr_mn40.py:98-244): same
 constructor argument, same `update((feat1, feat2), (pt1, pt2, gt_trans))` / `compute()` contract, same thresholds
 (:107-109), same result keys (:141).  The reference copies the descriptors to the host and calls Open3D / TEASER++ once
 per pair (:121, :165-231); here `func='ransac'` runs the RANSAC configuration the reference hands to Open3D
 (utils/open3d_func.py:43-49: voxel_size 0.08, edge-length similarity 0.9, max_iter 1000) on the GPU for all pairs at once,
-and `func='kabsch'` the plain least squares over the mutual matches.  `icp()` / `evaluate_registration()` are Open3D's
-registration_icp (point-to-point and point-to-plane) and evaluate_registration, batched over pairs; `register_pairs` and
-the meter refine their pose with it when given `icp={...}`.  FGR and TEASER++ are third-party solvers the reference only
-calls into; they are not re-implemented (func='fgr' / 'icp' / 'teaserpp' raise in `estimate_poses`: ICP refines a pose,
-it does not estimate one from matches).
+`func='fgr'` Open3D's Fast Global Registration over the same matches (`fgr()`), and `func='kabsch'` the plain least squares
+over the mutual matches.  `icp()` / `evaluate_registration()` are Open3D's registration_icp (point-to-point and
+point-to-plane) and evaluate_registration, batched over pairs; `register_pairs` and the meter refine their pose with it
+when given `icp={...}`.  TEASER++ is a third-party solver the reference only calls into; it is not re-implemented
+(func='icp' / 'teaserpp' raise in `estimate_poses`: ICP refines a pose, it does not estimate one from matches).
 """
 import time
 
@@ -18,21 +18,59 @@ import torch
 
 from . import matcher
 
-__all__ = ['estimate_poses', 'registration_metrics', 'icp', 'evaluate_registration', 'register_pairs',
+__all__ = ['estimate_poses', 'fgr', 'registration_metrics', 'icp', 'evaluate_registration', 'register_pairs',
            'MeterModelNet40_registration']
 
 
 def estimate_poses(src, tgt, idx1, idx2, count, func='ransac', voxel_size=0.08, max_iter=1000, edge_similarity=0.9,
                    refine_iters=3, seed=0):
     """src [P,n1,3], tgt [P,n2,3] CUDA fp32; idx1/idx2/count: the mutual matches (matcher.mutual_nn).
-    -> (T [P,4,4] fp32 mapping src onto tgt, inliers [P] int32)."""
-    if func not in ('ransac', 'kabsch'):
-        raise ValueError("func must be 'ransac' or 'kabsch' (Open3D FGR and TEASER++ are third-party solvers; ICP refines "
-                         "a pose: icp() or register_pairs(..., icp={...}))")
+    -> (T [P,4,4] fp32 mapping src onto tgt, inliers [P] int32).
+    func='fgr' is fgr() with maximum_correspondence_distance = 0.5 * voxel_size (the value of Open3D's FGR tutorial) and
+    inlier_dist = voxel_size, Open3D's other defaults, and `seed`; max_iter, edge_similarity and refine_iters are unused."""
+    if func not in ('ransac', 'kabsch', 'fgr'):
+        raise ValueError("func must be 'ransac', 'fgr' or 'kabsch' (TEASER++ is a third-party solver; ICP refines a pose: "
+                         "icp() or register_pairs(..., icp={...}))")
+    if func == 'fgr':
+        r = fgr(src, tgt, idx1, idx2, count, maximum_correspondence_distance=0.5 * float(voxel_size), seed=seed,
+                inlier_dist=float(voxel_size))
+        return r['transformation'], r['inliers']
     hyps = int(max_iter) if func == 'ransac' else 0
     return torch.ops.ri.pose_from_matches(src.float().contiguous(), tgt.float().contiguous(), idx1.contiguous(),
                                           idx2.contiguous(), count.contiguous(), hyps, float(voxel_size),
                                           float(edge_similarity), int(refine_iters), int(seed))
+
+
+def _int64(seed):
+    """A 64-bit seed as the signed integer a torch op argument holds (the library reads the same 64 bits unsigned)."""
+    s = int(seed) & 0xFFFFFFFFFFFFFFFF
+    return s - (1 << 64) if s >= 1 << 63 else s
+
+
+def fgr(src, tgt, idx1, idx2, count, maximum_correspondence_distance=0.025, iteration_number=64, division_factor=1.4,
+        use_absolute_scale=False, decrease_mu=True, tuple_test=True, tuple_scale=0.95, maximum_tuple_count=1000, seed=0,
+        inlier_dist=None, return_correspondences=False):
+    """Open3D's registration_fgr_based_on_feature_matching (FastGlobalRegistrationOption's names and defaults) for P pairs
+    at once, over given matches: src [P,n1,3], tgt [P,n2,3] CUDA fp32; idx1/idx2 [P,ld], count [P] (matcher.mutual_nn).
+    The tuple test samples with `seed`; inliers are counted within inlier_dist (default: maximum_correspondence_distance)
+    under the returned pose, as in estimate_poses.  include/ri_b200.h (ri_fgr_f32) states the arithmetic.
+    -> dict(transformation [P,4,4] fp32 src -> tgt, inliers [P] int32, num_correspondences [P] int32
+    [, correspondences [P,L] int32: the list's match positions, -1 padded; L = 3 * maximum_tuple_count with the tuple
+    test, else ld])."""
+    if inlier_dist is None:
+        inlier_dist = maximum_correspondence_distance
+    T, inl, corr, ncorr = torch.ops.ri.fgr(src.float().contiguous(), tgt.float().contiguous(), idx1.contiguous(),
+                                           idx2.contiguous(), count.contiguous(), float(maximum_correspondence_distance),
+                                           int(iteration_number), float(division_factor), bool(use_absolute_scale),
+                                           bool(decrease_mu), bool(tuple_test), float(tuple_scale),
+                                           int(maximum_tuple_count), _int64(seed), float(inlier_dist))
+    out = {'transformation': T, 'inliers': inl, 'num_correspondences': ncorr}
+    if return_correspondences:
+        if not tuple_test:                             # the list is the first ncorr matches
+            pos = torch.arange(idx1.shape[1], dtype=torch.int32, device=ncorr.device).expand(idx1.shape[0], -1)
+            corr = torch.where(pos < ncorr[:, None], pos, -1)
+        out['correspondences'] = corr
+    return out
 
 
 def registration_metrics(gt_trans, est_trans, pts):
@@ -93,8 +131,8 @@ class MeterModelNet40_registration:
     """Same state, thresholds and result keys as the reference meter (deepgmr_mn40.py:98-141)."""
 
     def __init__(self, func='ransac', device='cuda', icp=None):
-        """icp: None, or a dict of `icp()` keyword arguments; the RANSAC / Kabsch pose is then refined with it (inside
-        reg_time)."""
+        """func: 'ransac', 'fgr' or 'kabsch' (estimate_poses).  icp: None, or a dict of `icp()` keyword arguments; the
+        estimated pose is then refined with it (inside reg_time)."""
         self.rre = 0
         self.rte = 0
         self.num = 0
