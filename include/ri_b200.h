@@ -365,6 +365,34 @@ int ri_fgr_f32(const float* src, const float* tgt, const int* idx1, const int* i
                unsigned long long seed, float inlier_dist, float* T, int* inliers, int* corr, int* ncorr,
                void* stream);
 
+/* ---- FPFH descriptors (SURVEY.md 8f, row f8) -------------------------------------------------------------------------
+ * Open3D's compute_fpfh_feature with KDTreeSearchParamHybrid(radius, max_nn) (Rusu, Blodow, Beetz, ICRA 2009;
+ * pipelines/registration/Feature.cpp), B clouds per call.  xyz [B,3,N], normals [B,3,N] fp32 (used as given, not
+ * renormalised); radius > 0 (+inf = plain k-NN), 1 <= max_nn <= 128.  For each point q:
+ *   neighbours  the list of ri_estimate_normals_f32: the max_nn smallest keys (d, index) with d < min(r2, 10000), q included,
+ *               d = fma(dz,dz, fma(dy,dy, dx*dx)), d* = q - p in fp32 — the first max_nn entries of the k-NN (ri_knn_f32,
+ *               k = max_nn) whose distance passes the cut.  n = its length.  Nothing within the cap is dropped.
+ *   pair        feature (f0, f1, f2) of (p1, n1) with (p2, n2), fp64 from the fp32 inputs, each operation rounded:
+ *               dp = p2 - p1, L = |dp| (L == 0: (0,0,0)); a1 = n1.dp / L, a2 = n2.dp / L; if acos|a1| > acos|a2| swap n1
+ *               and n2, negate dp, f2 = -a2, else f2 = a1; v = dp x n1' (|v| == 0: (0,0,0)), v /= |v|, w = n1' x v;
+ *               f1 = v.n2', f0 = atan2(w.n2', n1'.n2').  Dot products are (x*x' + y*y') + z*z'.
+ *   SPFH        n <= 1: zeros.  Otherwise the pair features of (q, n_q) with list positions k = 1 .. n-1 (position 0 is
+ *               skipped whatever it holds) binned as b0 = floor(11 (f0 + pi) / (2 pi)), b1 = floor(11 (f1 + 1) * 0.5),
+ *               b2 = floor(11 (f2 + 1) * 0.5), each clamped to [0, 10]; counts c_j over 3 x 11 bins;
+ *               spfh_j = c_j * (100 / (n - 1)) in fp64 (Open3D adds 100 / (n - 1) c_j times: a few fp64 ulp apart).
+ *   FPFH        n <= 1: zeros.  Otherwise for k = 1 .. n-1 in list order: w_k = |p_k - q|^2 in fp64 from the fp32
+ *               coordinates (skipped when 0); val = spfh_j(p_k) / w_k is added to feat_j and to sum[j / 11]; then
+ *               fpfh_j = feat_j * (sum != 0 ? 100 / sum : 0) + spfh_j(q), rounded to fp32.  An exact duplicate of q with a
+ *               lower index sorts before q, so q meets itself at a later position: pair feature (0,0,0), weight skipped.
+ * Outputs fpfh [B,33,N] fp32; unless NULL, spfh [B,33,N] fp32 (c = round(spfh * (n - 1) / 100) recovers the counts) and
+ * counts [B,N] int32 = n.  No host synchronisation, no float atomics: a cloud's result does not depend on the rest of the
+ * batch and is bit-reproducible.  workspace >= ri_fpfh_workspace_bytes(B, N, max_nn) bytes (the grid, the lists and the
+ * packed bin counts), 16-byte aligned.  RI_ERR_BAD_ARG for radius <= 0 or NaN or max_nn <= 0; RI_ERR_UNSUPPORTED for
+ * max_nn > 128 or B > 65535. */
+size_t ri_fpfh_workspace_bytes(int B, int N, int max_nn);
+int ri_compute_fpfh_f32(const float* xyz, const float* normals, int B, int N, float radius, int max_nn, float* fpfh,
+                        float* spfh, int* counts, void* workspace, size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -59,7 +59,9 @@ SIGNATURES = {
     "ri_estimate_normals_f32": (_I, [_P, _I, _I, ctypes.c_float, _I, _P, _P, _P, _P, _P, _Z, _P]),
     "ri_fgr_f32": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, ctypes.c_float, _I, ctypes.c_float, _I, _I, _I,
                         ctypes.c_float, _I, ctypes.c_ulonglong, ctypes.c_float, _P, _P, _P, _P, _P]),
-    "ri_mutual_nn_workspace_bytes": (_Z, [_I, _I, _I, _I]),
+    "ri_fpfh_workspace_bytes": (_Z, [_I, _I, _I]),
+    "ri_compute_fpfh_f32": (_I, [_P, _P, _I, _I, ctypes.c_float, _I, _P, _P, _P, _P, _Z, _P]),
+    "ri_mutual_nn_workspace_bytes":(_Z, [_I, _I, _I, _I]),
     "ri_mutual_nn_tf32x3": (_I, [_P, _P, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P, _Z, _P]),
 }
 

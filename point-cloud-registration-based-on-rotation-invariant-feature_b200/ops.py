@@ -924,3 +924,41 @@ def _(src, tgt, idx1, idx2, count, max_corr_dist, iterations, division_factor, u
     P = src.shape[0]
     return (src.new_empty((P, 4, 4)), count.new_empty((P,)), count.new_empty((P, 3 * max_tuples if tuple_test else 0)),
             count.new_empty((P,)))
+
+
+# ---------------------------------------------------------------------------------------------- FPFH descriptors (f8)
+@torch.library.custom_op("ri::compute_fpfh", mutates_args=())
+def compute_fpfh(xyz: torch.Tensor, normals: torch.Tensor, radius: float, max_nn: int, with_spfh: bool,
+                 with_counts: bool) -> tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """xyz [B,3,N], normals [B,3,N] f32 -> (fpfh [B,33,N] f32, spfh [B,33,N] f32 ([0] unless with_spfh),
+    counts [B,N] i32 ([0] unless with_counts)).  Open3D's compute_fpfh_feature with the hybrid (radius, max_nn) search,
+    every cloud of the batch in one call (csrc/fpfh.cu)."""
+    _req(xyz, "xyz", torch.float32); _req(normals, "normals", torch.float32)
+    dev = _same_device(xyz, normals)
+    _shape(xyz, "xyz", None, 3, None)
+    B, _, N = xyz.shape
+    _shape(normals, "normals", B, 3, N)
+    if not float(radius) > 0.0:
+        raise RuntimeError("radius must be > 0")
+    if not 1 <= int(max_nn) <= 128:
+        raise RuntimeError("max_nn must be in [1, 128]")
+    if B > 65535:
+        raise RuntimeError("at most 65535 clouds per call")
+    with torch.cuda.device(dev):
+        fpfh = torch.empty((B, 33, N), dtype=torch.float32, device=dev)
+        spfh = torch.empty((B, 33, N) if with_spfh else (0,), dtype=torch.float32, device=dev)
+        cnt = torch.empty((B, N) if with_counts else (0,), dtype=torch.int32, device=dev)
+        nws = _L.ri_fpfh_workspace_bytes(B, N, int(max_nn))
+        ws = torch.empty(nws, dtype=torch.uint8, device=dev)
+        _check(_L.ri_compute_fpfh_f32(xyz.data_ptr(), normals.data_ptr(), B, N, float(radius), int(max_nn),
+                                      fpfh.data_ptr(), spfh.data_ptr() if with_spfh else None,
+                                      cnt.data_ptr() if with_counts else None, ws.data_ptr(), nws, _stream()),
+               "ri_compute_fpfh")
+    return fpfh, spfh, cnt
+
+
+@compute_fpfh.register_fake
+def _(xyz, normals, radius, max_nn, with_spfh, with_counts):
+    B, _, N = xyz.shape
+    return (xyz.new_empty((B, 33, N)), xyz.new_empty((B, 33, N) if with_spfh else (0,)),
+            xyz.new_empty((B, N) if with_counts else (0,), dtype=torch.int32))
