@@ -309,6 +309,36 @@ int ri_icp_f32(const float* src, const float* tgt, const float* tgt_normals, con
                float* T, double* fitness, double* inlier_rmse, int* iters, int* corr,
                void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- Generalized ICP (SURVEY.md 8f, row f9) ---------------------------------------------------------------------------
+ * Open3D's registration_generalized_icp (Segal, Haehnel, Thrun, RSS 2009; plane-to-plane) for P independent pairs per call.
+ * The loop, the correspondences, fitness, inlier_rmse, iters, corr and the fp64 accumulated T are exactly ri_icp_f32's
+ * (T = init, evaluate; per iteration solve U, T = U T, re-evaluate; stop when |d fitness| < rel_fitness and
+ * |d inlier_rmse| < rel_rmse or after max_iter updates; max_iter == 0 evaluates init).  Only the update differs:
+ *   covariance  C(n) = I - (1 - epsilon) n^ n^T per point, n^ = n / |n| in fp64; a zero-length or non-finite normal gives
+ *               C = I.  (Open3D's normals path, R_{e1->n} diag(eps,1,1) R_{e1->n}^T, and its no-normals path, the 20-NN
+ *               covariance's SVD with singular values (1,1,eps), both build this matrix from the smallest-eigenvalue
+ *               direction.)  The sign of a normal does not matter.
+ *   term        for a correspondence (source s, target t): q = T s as in ri_icp_f32; a = R n^_s with R the rotation of the
+ *               same fp32 T, evaluated in fp64; b = n^_t; M = C_t + R C_s R^T = 2I - (1 - epsilon)(a a^T + b b^T) (for
+ *               0 < epsilon <= 1 its eigenvalues lie in [2 epsilon, 2]); d = q - t; J0 = [-[q]x, I3].
+ *   update      H = sum J0^T M^-1 J0 and g = sum J0^T M^-1 d in fp64 with fixed-order reductions, M^-1 in closed form
+ *               (adjugate over determinant); H x = -g by LDL^T, |det H| < 1e-6 or a non-finite x gives U = I (the
+ *               point-to-plane rule); U = [Rz(x2) Ry(x1) Rx(x0) | x3 x4 x5].
+ * Deltas from Open3D: (1) Open3D forms W = (M^-1)^(1/2) and sums (W J0)^T (W J0) and (W J0)^T (W d); with its default L2
+ * kernel that equals H and g in exact arithmetic, so the two differ by rounding only.  (2) Open3D's GetRotationFromE1ToX
+ * returns the identity when n.e1 < -0.99, so for normals within about 8 degrees of -x it uses the covariance of e1 instead of
+ * that of n; here the exact formula is used for every normal (read from Open3D's GeneralizedICP.cpp, not verified against
+ * a build of it).  (3) Robust kernels and caller-supplied covariance matrices are not supported.
+ * src [P,n1,3], tgt [P,n2,3], src_normals [P,n1,3], tgt_normals [P,n2,3] (both required), init [P,4,4] row-major
+ * (NULL = identity), fp32 point-major.  Outputs as ri_icp_f32.  Bit-reproducible (no float atomics); a pair's result does not
+ * depend on the rest of the batch; max_iter + 6 launches, no host synchronisation, no allocation.
+ * workspace >= ri_icp_workspace_bytes(P, n1, n2).  RI_ERR_BAD_ARG for n1 or n2 <= 0, max_corr_dist <= 0 or NaN,
+ * epsilon <= 0 or not finite, max_iter < 0, or a NULL normals pointer. */
+int ri_generalized_icp_f32(const float* src, const float* tgt, const float* src_normals, const float* tgt_normals,
+                           const float* init, int P, int n1, int n2, float max_corr_dist, float epsilon, int max_iter,
+                           float rel_fitness, float rel_rmse, float* T, double* fitness, double* inlier_rmse, int* iters,
+                           int* corr, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- normal estimation for xyz-only clouds (SURVEY.md 8f, row f6) ----------------------------------------------------
  * Open3D's estimate_normals with KDTreeSearchParamHybrid(radius, max_nn) (the reference calls it on the host,
  * utils/open3d_func.py:77-83), B clouds per call.  xyz [B,3,N] fp32; radius > 0 (+inf = plain k-NN), 1 <= max_nn <= 32.

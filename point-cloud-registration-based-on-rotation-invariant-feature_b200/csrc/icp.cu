@@ -1,5 +1,5 @@
-// icp.cu — batched ICP refinement (point-to-point and point-to-plane) and registration evaluation, sm_100a
-// (SURVEY.md §8f row f5).
+// icp.cu — batched ICP refinement (point-to-point, point-to-plane and generalized / plane-to-plane) and registration
+// evaluation, sm_100a (SURVEY.md §8f rows f5 and f9).
 //
 // Open3D's registration_icp / evaluate_registration (the reference reaches them through utils/open3d_func.py), for P
 // independent (source, target) pairs per call, with Open3D's loop per pair:
@@ -15,6 +15,10 @@
 // Point-to-point: Horn's quaternion on (q_i, t_i), no scale (the optimum of Open3D's Umeyama).  Point-to-plane: Open3D's
 // linearisation r_i = (q_i - t_i).n_i, J_i = [q_i x n_i, n_i], J^T J x = -J^T r in fp64; |det J^T J| < 1e-6 or a non-finite
 // x gives the identity update; U = Rz(x2) Ry(x1) Rx(x0) with translation x3..5 (TransformVector6dToMatrix4d).
+// Generalized ICP (row f9, Open3D's registration_generalized_icp): covariances C(n) = I - (1 - eps) n^ n^T from unit normals
+// (C = I for a zero-length or non-finite normal); per correspondence a = R n^_s (R the rotation of the fp32 T that moved the
+// point, in fp64), b = n^_t, M = C_t + R C_s R^T = 2I - (1 - eps)(a a^T + b b^T), d = q - t, J0 = [-[q]x, I3];
+// H = sum J0^T M^-1 J0, g = sum J0^T M^-1 d in fp64, then the point-to-plane solve and composition above on (H, g).
 //
 // One deliberate difference from Open3D: Open3D transforms its copy of the source incrementally (s <- U s every
 // iteration); here every iteration transforms the ORIGINAL source by the accumulated T, which is kept in fp64 on the device.
@@ -31,7 +35,7 @@
 //   icp_iter       grid (source tiles, P), once per iteration.  A CTA of a converged pair exits at once.  Otherwise each
 //                  thread runs a radius-bounded 1-NN for its source points over the cells the query ball can touch,
 //                  accumulates count, sum d^2 and the solver's moments in fp64 (15 for point-to-point: sum q, sum t,
-//                  sum q t^T; 27 for point-to-plane: the upper triangle of J^T J and J^T r), the CTA reduces them in a
+//                  sum q t^T; 27 for point-to-plane and generalized ICP: the upper triangle of H and g), the CTA reduces them in a
 //                  fixed order into partials[P][tiles][K].  The last CTA of the pair (threadfence + atomic ticket, reset
 //                  afterwards) sums the partials in tile order, computes fitness / rmse, applies the convergence test
 //                  against the previous iteration's values, and either marks the pair done or solves U and sets T = U T.
@@ -47,8 +51,10 @@ constexpr int kSetupThreads = 1024;
 constexpr int kThreads = 256;
 constexpr int kPerThread = 2;
 constexpr int kTile = kThreads * kPerThread;      // source points per CTA
-constexpr int kKMax = 29;                         // count, sum d^2, 27 point-to-plane moments
+constexpr int kKMax = 29;                         // count, sum d^2, 27 point-to-plane / generalized moments
 constexpr int kKPoint = 17;                       // count, sum d^2, 15 point-to-point moments
+
+enum Estimator : int { kPointToPoint = 0, kPointToPlane = 1, kGeneralized = 2 };
 
 struct GridHdr {               // per pair, 16 ints at the head of its grid slab
     float ox, oy, oz, h, inv_h;
@@ -241,11 +247,91 @@ __device__ __forceinline__ bool axis_range(float x, float o, float inv_h, float 
     return true;
 }
 
-template <bool PLANE>
+// n / |n| in fp64; the zero vector (which makes C(n) = I) for a zero-length or non-finite n.  -n gives exactly -(n / |n|).
+__device__ __forceinline__ void unit_or_zero(float x, float y, float z, double u[3])
+{
+    const double dx = x, dy = y, dz = z;
+    const double l2 = dx * dx + dy * dy + dz * dz;
+    if (!(l2 > 0.0 && isfinite(l2))) {                 // explicit zeros: a NaN or infinite component times 0 is NaN
+        u[0] = 0.0; u[1] = 0.0; u[2] = 0.0;
+        return;
+    }
+    const double s = 1.0 / sqrt(l2);
+    u[0] = dx * s; u[1] = dy * s; u[2] = dz * s;
+}
+
+// The linearised 6x6 step shared by point-to-plane and generalized ICP, on the reduced 29-slot moments m (m[2..22]: the upper
+// triangle of H in row order, m[23..28]: g): H x = -g with the 1e-6 determinant rule of ldlt_solve6, then
+// U = [Rz(x2) Ry(x1) Rx(x0) | x3..5]; U is left unchanged (the identity) when the solve fails.  b and x are the caller's
+// scratch: local arrays of an inlined callee are allocated ahead of the caller's, which reorders the accumulators' registers.
+__device__ __forceinline__ void linearised_update(const double* m, double b[6], double x[6], double U[12])
+{
+#pragma unroll
+    for (int a = 0; a < 6; ++a) b[a] = -m[23 + a];
+    if (ldlt_solve6(m + 2, b, x, 1e-6)) {
+        const double ca = cos(x[0]), sa = sin(x[0]), cb = cos(x[1]), sb = sin(x[1]), cg = cos(x[2]), sg = sin(x[2]);
+        // Rz(x2) Ry(x1) Rx(x0)
+        U[0] = cg * cb; U[1] = cg * sb * sa - sg * ca; U[2] = cg * sb * ca + sg * sa; U[3] = x[3];
+        U[4] = sg * cb; U[5] = sg * sb * sa + cg * ca; U[6] = sg * sb * ca - cg * sa; U[7] = x[4];
+        U[8] = -sb;     U[9] = cb * sa;                U[10] = cb * ca;               U[11] = x[5];
+    }
+}
+
+// One generalized-ICP correspondence into acc[2..28]: q = T s (fp32), t its target point, ns the source normal (caller's
+// frame), nt the target normal, Tf the fp32 T that moved s, c = 1 - eps.  M^-1 is the adjugate of the symmetric M over its
+// determinant (eigenvalues of M in [2 min(eps, 1), 2 max(eps, 1)]: never singular).  With u_k = e_k x q (J0's k-th
+// column) the moments are H_kl = u_k.M^-1 u_l, H_k(3+l) = (M^-1 u_k)_l, H_(3+k)(3+l) = M^-1_kl, g_k = (M^-1 u_k).d,
+// g_(3+k) = (M^-1 d)_k.
+__device__ __forceinline__ void gicp_moments(const float* Tf, double qx, double qy, double qz, double tx, double ty,
+                                             double tz, const float* ns, float4 nt, double c, double* acc)
+{
+    double n[3], a[3], b[3];
+    unit_or_zero(ns[0], ns[1], ns[2], n);
+    unit_or_zero(nt.x, nt.y, nt.z, b);
+#pragma unroll
+    for (int k = 0; k < 3; ++k)
+        a[k] = (double)Tf[4 * k] * n[0] + (double)Tf[4 * k + 1] * n[1] + (double)Tf[4 * k + 2] * n[2];
+    const double m00 = 2.0 - c * (a[0] * a[0] + b[0] * b[0]), m11 = 2.0 - c * (a[1] * a[1] + b[1] * b[1]);
+    const double m22 = 2.0 - c * (a[2] * a[2] + b[2] * b[2]);
+    const double m01 = -c * (a[0] * a[1] + b[0] * b[1]), m02 = -c * (a[0] * a[2] + b[0] * b[2]);
+    const double m12 = -c * (a[1] * a[2] + b[1] * b[2]);
+    double i00 = m11 * m22 - m12 * m12, i01 = m02 * m12 - m01 * m22, i02 = m01 * m12 - m02 * m11;
+    double i11 = m00 * m22 - m02 * m02, i12 = m01 * m02 - m00 * m12, i22 = m00 * m11 - m01 * m01;
+    const double inv = 1.0 / (m00 * i00 + m01 * i01 + m02 * i02);
+    i00 *= inv; i01 *= inv; i02 *= inv; i11 *= inv; i12 *= inv; i22 *= inv;
+    const double dx = qx - tx, dy = qy - ty, dz = qz - tz;
+    // w_k = M^-1 u_k with u_0 = (0, -qz, qy), u_1 = (qz, 0, -qx), u_2 = (-qy, qx, 0)
+    const double w0[3] = {i02 * qy - i01 * qz, i12 * qy - i11 * qz, i22 * qy - i12 * qz};
+    const double w1[3] = {i00 * qz - i02 * qx, i01 * qz - i12 * qx, i02 * qz - i22 * qx};
+    const double w2[3] = {i01 * qx - i00 * qy, i11 * qx - i01 * qy, i12 * qx - i02 * qy};
+    acc[2] += w0[2] * qy - w0[1] * qz;                  // H_00 = u_0.w_0
+    acc[3] += w1[2] * qy - w1[1] * qz;                  // H_01 = u_0.w_1
+    acc[4] += w2[2] * qy - w2[1] * qz;                  // H_02 = u_0.w_2
+    acc[5] += w0[0]; acc[6] += w0[1]; acc[7] += w0[2];
+    acc[8] += w1[0] * qz - w1[2] * qx;                  // H_11 = u_1.w_1
+    acc[9] += w2[0] * qz - w2[2] * qx;                  // H_12 = u_1.w_2
+    acc[10] += w1[0]; acc[11] += w1[1]; acc[12] += w1[2];
+    acc[13] += w2[1] * qx - w2[0] * qy;                 // H_22 = u_2.w_2
+    acc[14] += w2[0]; acc[15] += w2[1]; acc[16] += w2[2];
+    acc[17] += i00; acc[18] += i01; acc[19] += i02;
+    acc[20] += i11; acc[21] += i12;
+    acc[22] += i22;
+    acc[23] += w0[0] * dx + w0[1] * dy + w0[2] * dz;
+    acc[24] += w1[0] * dx + w1[1] * dy + w1[2] * dz;
+    acc[25] += w2[0] * dx + w2[1] * dy + w2[2] * dz;
+    acc[26] += i00 * dx + i01 * dy + i02 * dz;
+    acc[27] += i01 * dx + i11 * dy + i12 * dz;
+    acc[28] += i02 * dx + i12 * dy + i22 * dz;
+}
+
+// EST = kPointToPoint / kPointToPlane / kGeneralized.  src_nrm [P,n1,3] and eps are read by kGeneralized only.
+template <int EST>
 __global__ void __launch_bounds__(kThreads)
 icp_iter_kernel(const float* __restrict__ src, int P, int n1, int n2, float r, int it, int max_iter, float rel_fitness,
-                float rel_rmse, int* __restrict__ corr, unsigned char* __restrict__ ws)
+                float rel_rmse, int* __restrict__ corr, unsigned char* __restrict__ ws, const float* __restrict__ src_nrm,
+                float eps)
 {
+    constexpr bool PLANE = EST != kPointToPoint;       // the 27-moment layout and the linearised solve
     constexpr int K = PLANE ? kKMax : kKPoint;
     __shared__ double red[(kThreads / 32) * K];
     __shared__ double tot[K];
@@ -313,7 +399,7 @@ icp_iter_kernel(const float* __restrict__ src, int P, int n1, int n2, float r, i
             acc[8] += dqx * tx; acc[9] += dqx * ty; acc[10] += dqx * tz;
             acc[11] += dqy * tx; acc[12] += dqy * ty; acc[13] += dqy * tz;
             acc[14] += dqz * tx; acc[15] += dqz * ty; acc[16] += dqz * tz;
-        } else {
+        } else if (EST == kPointToPlane) {
             const float4 nv = __ldg(Nt + bp);
             const double nx = nv.x, ny = nv.y, nz = nv.z;
             const double res = (dqx - tx) * nx + (dqy - ty) * ny + (dqz - tz) * nz;
@@ -325,6 +411,9 @@ icp_iter_kernel(const float* __restrict__ src, int P, int n1, int n2, float r, i
                 for (int b = a; b < 6; ++b) acc[k++] += J[a] * J[b];
 #pragma unroll
             for (int a = 0; a < 6; ++a) acc[23 + a] += J[a] * res;
+        } else {
+            gicp_moments(Tf, dqx, dqy, dqz, tx, ty, tz, src_nrm + ((size_t)p * n1 + i) * 3, __ldg(Nt + bp),
+                         1.0 - (double)eps, acc);
         }
     }
 
@@ -381,15 +470,7 @@ icp_iter_kernel(const float* __restrict__ src, int P, int n1, int n2, float r, i
         }
     } else {
         double b[6], x[6];
-#pragma unroll
-        for (int a = 0; a < 6; ++a) b[a] = -tot[23 + a];
-        if (ldlt_solve6(tot + 2, b, x, 1e-6)) {
-            const double ca = cos(x[0]), sa = sin(x[0]), cb = cos(x[1]), sb = sin(x[1]), cg = cos(x[2]), sg = sin(x[2]);
-            // Rz(x2) Ry(x1) Rx(x0)
-            U[0] = cg * cb; U[1] = cg * sb * sa - sg * ca; U[2] = cg * sb * ca + sg * sa; U[3] = x[3];
-            U[4] = sg * cb; U[5] = sg * sb * sa + cg * ca; U[6] = sg * sb * ca - cg * sa; U[7] = x[4];
-            U[8] = -sb;     U[9] = cb * sa;                U[10] = cb * ca;               U[11] = x[5];
-        }
+        linearised_update(tot, b, x, U);
     }
     double Tn[12];
 #pragma unroll
@@ -416,6 +497,47 @@ __global__ void icp_final_kernel(int P, int n1, int n2, const unsigned char* __r
     iters[p] = S->iters;
 }
 
+// The launch sequence of one call, after the arguments have been checked (P > 0): setup, binning, max_iter + 1 iteration
+// launches, final.  nrm: target normals binned with the grid (NULL for point-to-point).
+int icp_launch(int est, const float* src, const float* tgt, const float* nrm, const float* src_nrm, const float* init,
+               int P, int n1, int n2, float max_corr_dist, float eps, int max_iter, float rel_fitness, float rel_rmse,
+               float* T, double* fitness, double* inlier_rmse, int* iters, int* corr, void* workspace,
+               size_t workspace_bytes, void* stream)
+{
+    if (P > 65535) return RI_ERR_UNSUPPORTED;
+    if (P == 0) return RI_OK;
+    const IcpWs L = icp_ws_layout(P, n1, n2);
+    if (L.tiles > 65535) return RI_ERR_UNSUPPORTED;
+    if (workspace == nullptr || ((uintptr_t)workspace & 15) != 0 || workspace_bytes < L.total) return RI_ERR_WORKSPACE;
+    cudaStream_t st = (cudaStream_t)stream;
+    unsigned char* ws = reinterpret_cast<unsigned char*>(workspace);
+    icp_setup_kernel<<<P, kSetupThreads, 0, st>>>(tgt, init, P, n1, n2, max_corr_dist, ws);
+    RI_LAUNCH_CHECK();
+    const dim3 gb((n2 + 255) / 256, P);
+    icp_bin_kernel<0><<<gb, 256, 0, st>>>(tgt, nrm, P, n1, n2, ws);
+    RI_LAUNCH_CHECK();
+    icp_scan_kernel<<<P, 1024, 0, st>>>(P, n1, n2, ws);
+    RI_LAUNCH_CHECK();
+    icp_bin_kernel<1><<<gb, 256, 0, st>>>(tgt, nrm, P, n1, n2, ws);
+    RI_LAUNCH_CHECK();
+    const dim3 gi(L.tiles, P);
+    for (int it = 0; it <= max_iter; ++it) {
+        if (est == kGeneralized)
+            icp_iter_kernel<kGeneralized><<<gi, kThreads, 0, st>>>(src, P, n1, n2, max_corr_dist, it, max_iter,
+                                                                   rel_fitness, rel_rmse, corr, ws, src_nrm, eps);
+        else if (est == kPointToPlane)
+            icp_iter_kernel<kPointToPlane><<<gi, kThreads, 0, st>>>(src, P, n1, n2, max_corr_dist, it, max_iter,
+                                                                    rel_fitness, rel_rmse, corr, ws, nullptr, 0.f);
+        else
+            icp_iter_kernel<kPointToPoint><<<gi, kThreads, 0, st>>>(src, P, n1, n2, max_corr_dist, it, max_iter,
+                                                                    rel_fitness, rel_rmse, corr, ws, nullptr, 0.f);
+        RI_LAUNCH_CHECK();
+    }
+    icp_final_kernel<<<(P + 127) / 128, 128, 0, st>>>(P, n1, n2, ws, T, fitness, inlier_rmse, iters);
+    RI_LAUNCH_CHECK();
+    return RI_OK;
+}
+
 }  // namespace
 
 extern "C" size_t ri_icp_workspace_bytes(int P, int n1, int n2)
@@ -434,34 +556,21 @@ extern "C" int ri_icp_f32(const float* src, const float* tgt, const float* tgt_n
 {
     if (P < 0 || n1 <= 0 || n2 <= 0 || !(max_corr_dist > 0.f) || max_iter < 0) return RI_ERR_BAD_ARG;
     if (point_to_plane && tgt_normals == nullptr) return RI_ERR_BAD_ARG;
-    if (P > 65535) return RI_ERR_UNSUPPORTED;
-    if (P == 0) return RI_OK;
-    const IcpWs L = icp_ws_layout(P, n1, n2);
-    if (L.tiles > 65535) return RI_ERR_UNSUPPORTED;
-    if (workspace == nullptr || ((uintptr_t)workspace & 15) != 0 || workspace_bytes < L.total) return RI_ERR_WORKSPACE;
-    cudaStream_t st = (cudaStream_t)stream;
-    unsigned char* ws = reinterpret_cast<unsigned char*>(workspace);
-    const float* nrm = point_to_plane ? tgt_normals : nullptr;
-    icp_setup_kernel<<<P, kSetupThreads, 0, st>>>(tgt, init, P, n1, n2, max_corr_dist, ws);
-    RI_LAUNCH_CHECK();
-    const dim3 gb((n2 + 255) / 256, P);
-    icp_bin_kernel<0><<<gb, 256, 0, st>>>(tgt, nrm, P, n1, n2, ws);
-    RI_LAUNCH_CHECK();
-    icp_scan_kernel<<<P, 1024, 0, st>>>(P, n1, n2, ws);
-    RI_LAUNCH_CHECK();
-    icp_bin_kernel<1><<<gb, 256, 0, st>>>(tgt, nrm, P, n1, n2, ws);
-    RI_LAUNCH_CHECK();
-    const dim3 gi(L.tiles, P);
-    for (int it = 0; it <= max_iter; ++it) {
-        if (point_to_plane)
-            icp_iter_kernel<true><<<gi, kThreads, 0, st>>>(src, P, n1, n2, max_corr_dist, it, max_iter, rel_fitness,
-                                                           rel_rmse, corr, ws);
-        else
-            icp_iter_kernel<false><<<gi, kThreads, 0, st>>>(src, P, n1, n2, max_corr_dist, it, max_iter, rel_fitness,
-                                                            rel_rmse, corr, ws);
-        RI_LAUNCH_CHECK();
-    }
-    icp_final_kernel<<<(P + 127) / 128, 128, 0, st>>>(P, n1, n2, ws, T, fitness, inlier_rmse, iters);
-    RI_LAUNCH_CHECK();
-    return RI_OK;
+    return icp_launch(point_to_plane ? kPointToPlane : kPointToPoint, src, tgt, point_to_plane ? tgt_normals : nullptr,
+                      nullptr, init, P, n1, n2, max_corr_dist, 0.f, max_iter, rel_fitness, rel_rmse, T, fitness,
+                      inlier_rmse, iters, corr, workspace, workspace_bytes, stream);
+}
+
+// ri_icp_f32 with the generalized (plane-to-plane) estimator: src_normals [P,n1,3] and tgt_normals [P,n2,3] fp32 point-major
+// (both required; used through n / |n|), eps the covariances' smallest eigenvalue (finite, > 0).
+extern "C" int ri_generalized_icp_f32(const float* src, const float* tgt, const float* src_normals,
+                                      const float* tgt_normals, const float* init, int P, int n1, int n2,
+                                      float max_corr_dist, float epsilon, int max_iter, float rel_fitness,
+                                      float rel_rmse, float* T, double* fitness, double* inlier_rmse, int* iters,
+                                      int* corr, void* workspace, size_t workspace_bytes, void* stream)
+{
+    if (P < 0 || n1 <= 0 || n2 <= 0 || !(max_corr_dist > 0.f) || max_iter < 0) return RI_ERR_BAD_ARG;
+    if (!(epsilon > 0.f) || !isfinite(epsilon) || src_normals == nullptr || tgt_normals == nullptr) return RI_ERR_BAD_ARG;
+    return icp_launch(kGeneralized, src, tgt, tgt_normals, src_normals, init, P, n1, n2, max_corr_dist, epsilon, max_iter,
+                      rel_fitness, rel_rmse, T, fitness, inlier_rmse, iters, corr, workspace, workspace_bytes, stream);
 }

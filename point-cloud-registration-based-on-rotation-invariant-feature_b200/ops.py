@@ -6,6 +6,7 @@ torch (so they live in the caching allocator, as the reference's torch::zeros ou
 hand-written sm_100a kernels on torch's CURRENT stream through ctypes.  There is no other implementation behind
 these names: no Triton, no eager fallback, no CPU path.
 """
+import math
 from typing import Optional
 
 import torch
@@ -826,6 +827,67 @@ def icp(src: torch.Tensor, tgt: torch.Tensor, tgt_normals: Optional[torch.Tensor
 
 @icp.register_fake
 def _(src, tgt, tgt_normals, init, r, point_to_plane, max_iter, rel_fitness, rel_rmse, want_corr):
+    P, n1 = src.shape[0], src.shape[1]
+    return (src.new_empty((P, 4, 4)), src.new_empty((P,), dtype=torch.float64), src.new_empty((P,), dtype=torch.float64),
+            src.new_empty((P,), dtype=torch.int32), src.new_empty((P, n1 if want_corr else 0), dtype=torch.int32))
+
+
+# ---------------------------------------------------------------------------------------------- Generalized ICP (f9)
+def check_generalized_icp(src, tgt, src_normals, tgt_normals, init, r, epsilon, max_iter):
+    """Raise RuntimeError unless the arguments of generalized_icp are valid; a normals argument may be None here (the
+    Python wrapper estimates it after this check, so a bad call launches nothing)."""
+    ts = [(src, "src"), (tgt, "tgt"), (init, "init")]
+    ts += [(t, nm) for t, nm in ((src_normals, "src_normals"), (tgt_normals, "tgt_normals")) if t is not None]
+    for t, nm in ts:
+        _req(t, nm, torch.float32)
+    _same_device(*(t for t, _ in ts))
+    _shape(src, "src", None, None, 3)
+    P, n1, _ = src.shape
+    _shape(tgt, "tgt", P, None, 3)
+    _shape(init, "init", P, 4, 4)
+    if src_normals is not None:
+        _shape(src_normals, "src_normals", P, n1, 3)
+    if tgt_normals is not None:
+        _shape(tgt_normals, "tgt_normals", P, tgt.shape[1], 3)
+    if n1 < 1 or tgt.shape[1] < 1:
+        raise RuntimeError("src and tgt need at least one point per pair")
+    if not float(r) > 0.0:
+        raise RuntimeError("max_correspondence_distance must be > 0")
+    if not (math.isfinite(float(epsilon)) and float(epsilon) > 0.0):
+        raise RuntimeError("epsilon must be finite and > 0")
+    if int(max_iter) < 0:
+        raise RuntimeError("max_iter must be >= 0")
+
+
+@torch.library.custom_op("ri::generalized_icp", mutates_args=())
+def generalized_icp(src: torch.Tensor, tgt: torch.Tensor, src_normals: torch.Tensor, tgt_normals: torch.Tensor,
+                    init: torch.Tensor, r: float, epsilon: float, max_iter: int, rel_fitness: float, rel_rmse: float,
+                    want_corr: bool) -> tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    """src [P,n1,3], tgt [P,n2,3], src_normals [P,n1,3], tgt_normals [P,n2,3], init [P,4,4] f32 -> (T [P,4,4] f32,
+    fitness [P] f64, inlier_rmse [P] f64, iterations [P] i32, corr [P,n1] i32 ([P,0] unless want_corr)).
+    Open3D's registration_generalized_icp per pair, all pairs in one call (csrc/icp.cu); max_iter == 0 evaluates init."""
+    check_generalized_icp(src, tgt, src_normals, tgt_normals, init, r, epsilon, max_iter)
+    P, n1, _ = src.shape
+    n2 = tgt.shape[1]
+    dev = src.device
+    with torch.cuda.device(dev):
+        T = torch.empty((P, 4, 4), dtype=torch.float32, device=dev)
+        fit = torch.empty((P,), dtype=torch.float64, device=dev)
+        rmse = torch.empty((P,), dtype=torch.float64, device=dev)
+        iters = torch.empty((P,), dtype=torch.int32, device=dev)
+        corr = torch.empty((P, n1 if want_corr else 0), dtype=torch.int32, device=dev)
+        nws = _L.ri_icp_workspace_bytes(P, n1, n2)
+        ws = torch.empty(nws, dtype=torch.uint8, device=dev)
+        _check(_L.ri_generalized_icp_f32(src.data_ptr(), tgt.data_ptr(), src_normals.data_ptr(), tgt_normals.data_ptr(),
+                                         init.data_ptr(), P, n1, n2, float(r), float(epsilon), int(max_iter),
+                                         float(rel_fitness), float(rel_rmse), T.data_ptr(), fit.data_ptr(),
+                                         rmse.data_ptr(), iters.data_ptr(), corr.data_ptr() if want_corr else None,
+                                         ws.data_ptr(), nws, _stream()), "ri_generalized_icp")
+    return T, fit, rmse, iters, corr
+
+
+@generalized_icp.register_fake
+def _(src, tgt, src_normals, tgt_normals, init, r, epsilon, max_iter, rel_fitness, rel_rmse, want_corr):
     P, n1 = src.shape[0], src.shape[1]
     return (src.new_empty((P, 4, 4)), src.new_empty((P,), dtype=torch.float64), src.new_empty((P,), dtype=torch.float64),
             src.new_empty((P,), dtype=torch.int32), src.new_empty((P, n1 if want_corr else 0), dtype=torch.int32))

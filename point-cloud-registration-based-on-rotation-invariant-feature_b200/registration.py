@@ -9,17 +9,18 @@ per pair (:121, :165-231); here `func='ransac'` runs the RANSAC configuration th
 `func='fgr'` Open3D's Fast Global Registration over the same matches (`fgr()`), and `func='kabsch'` the plain least squares
 over the mutual matches.  `icp()` / `evaluate_registration()` are Open3D's registration_icp (point-to-point and
 point-to-plane) and evaluate_registration, batched over pairs; `register_pairs` and the meter refine their pose with it
-when given `icp={...}`.  TEASER++ is a third-party solver the reference only calls into; it is not re-implemented
+when given `icp={...}`.  `generalized_icp()` is Open3D's registration_generalized_icp (plane-to-plane, covariances from
+normals), a separate refinement after any of them: `generalized_icp(pt1, pt2, r, init=T)`.  TEASER++ is a third-party solver the reference only calls into; it is not re-implemented
 (func='icp' / 'teaserpp' raise in `estimate_poses`: ICP refines a pose, it does not estimate one from matches).
 """
 import time
 
 import torch
 
-from . import matcher
+from . import matcher, ops
 
-__all__ = ['estimate_poses', 'fgr', 'registration_metrics', 'icp', 'evaluate_registration', 'register_pairs',
-           'MeterModelNet40_registration']
+__all__ = ['estimate_poses', 'fgr', 'registration_metrics', 'icp', 'generalized_icp', 'evaluate_registration',
+           'register_pairs', 'MeterModelNet40_registration']
 
 
 def estimate_poses(src, tgt, idx1, idx2, count, func='ransac', voxel_size=0.08, max_iter=1000, edge_similarity=0.9,
@@ -108,6 +109,45 @@ def icp(src, tgt, max_correspondence_distance, init=None, estimation='point_to_p
 
 
 _icp = icp       # register_pairs() and the meter take an `icp` argument of their own
+
+
+def generalized_icp(src, tgt, max_correspondence_distance, init=None, epsilon=1e-3, src_normals=None, tgt_normals=None,
+                    max_iter=30, relative_fitness=1e-6, relative_rmse=1e-6, return_correspondences=False):
+    """Open3D's registration_generalized_icp (plane-to-plane) for P pairs at once.  src [P,n1,3], tgt [P,n2,3] CUDA fp32;
+    init [P,4,4] (default identity).  The loop, the stopping rule, fitness, inlier_rmse and the correspondences are icp()'s;
+    the update minimises sum d^T (C_t + R C_s R^T)^-1 d over correspondences, d = T s - t, with the covariances
+    C(n) = I - (1 - epsilon) n n^T built from unit normals (a zero or non-finite normal gives C = I).
+    src_normals [P,n1,3] / tgt_normals [P,n2,3]: each cloud's normals in its own frame; a missing one is estimated with
+    functional.estimate_normals(cloud, radius=inf, max_nn=20), i.e. from the 20 nearest neighbours (distance^2 < 10000;
+    (0,0,1) with fewer than 3).  A normal's sign does not matter.
+    Deltas from Open3D: M^-1 is used directly rather than its square root (equal up to rounding); every normal uses the
+    exact covariance, where Open3D substitutes that of e1 for normals within about 8 degrees of -x (read from its source,
+    not verified against a build); no robust kernels and no caller-supplied covariance matrices.
+    include/ri_b200.h (ri_generalized_icp_f32) states the arithmetic.
+    -> dict(transformation [P,4,4] fp32 src -> tgt, fitness [P] f64, inlier_rmse [P] f64, iterations [P] int32
+    [, correspondences [P,n1] int32: target index or -1, under the returned transformation])."""
+    from .functional import estimate_normals
+    src = src.float().contiguous()
+    tgt = tgt.float().contiguous()
+    if init is None:
+        init = torch.eye(4, dtype=torch.float32, device=src.device).expand(src.shape[0], 4, 4)
+    init = init.float().contiguous()
+    src_normals = None if src_normals is None else src_normals.float().contiguous()
+    tgt_normals = None if tgt_normals is None else tgt_normals.float().contiguous()
+    ops.check_generalized_icp(src, tgt, src_normals, tgt_normals, init, max_correspondence_distance, epsilon, max_iter)
+    estimate = lambda x: estimate_normals(x.transpose(1, 2), radius=float('inf'), max_nn=20).transpose(1, 2).contiguous()
+    if src_normals is None:
+        src_normals = estimate(src)
+    if tgt_normals is None:
+        tgt_normals = estimate(tgt)
+    T, fit, rmse, iters, corr = torch.ops.ri.generalized_icp(src, tgt, src_normals, tgt_normals, init,
+                                                             float(max_correspondence_distance), float(epsilon),
+                                                             int(max_iter), float(relative_fitness), float(relative_rmse),
+                                                             bool(return_correspondences))
+    out = {'transformation': T, 'fitness': fit, 'inlier_rmse': rmse, 'iterations': iters}
+    if return_correspondences:
+        out['correspondences'] = corr
+    return out
 
 
 def evaluate_registration(src, tgt, max_correspondence_distance, T):
