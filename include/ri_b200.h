@@ -395,7 +395,48 @@ int ri_fgr_f32(const float* src, const float* tgt, const int* idx1, const int* i
                unsigned long long seed, float inlier_dist, float* T, int* inliers, int* corr, int* ncorr,
                void* stream);
 
-/* ---- FPFH descriptors (SURVEY.md 8f, row f8) -------------------------------------------------------------------------
+/* ---- TEASER++ with a known scale (SURVEY.md 8f, row f10) -------------------------------------------------------------
+ * TEASER++ (Yang, Shi, Carlone, T-RO 2020; the reference's registration solver, deepgmr_mn40.py:175-230) over the mutual
+ * matches, P pairs per call.  src, tgt, idx1, idx2, count as in ri_pose_from_matches_f32: pair p has M = min(count[p], ld)
+ * matches a_m = src[idx1[m]], b_m = tgt[idx2[m]]; every match is a vertex.  tests/teaser_oracle.py replays every step.
+ *   graph     edge (i, j), i != j, iff |l_a - l_b| <= beta, beta = 2 * noise_bound * sqrt(cbar2) (fp64, in that order);
+ *             l = |u - v| in fp64 from the fp32 coordinates as sqrt((dx*dx + dy*dy) + dz*dz), each operation rounded (no
+ *             contraction), |l_a - l_b| likewise: the graph is bit-exact.
+ *   order     pi sorts the vertices by degree descending, then index ascending; "first" below means first in pi.
+ *   clique    (a) for each of the first min(M, 64) vertices v of pi: C = {v}, cand = N(v); repeatedly add the first vertex of
+ *             cand and intersect cand with its neighbourhood; best = the largest C, the earliest v on ties.  (b) Repeatedly
+ *             remove every alive vertex whose alive-degree is below |best|.  (c) BBMC branch and bound over the alive
+ *             vertices: expand(C, P) colours P greedily (each class takes, in pi order, every remaining vertex not adjacent
+ *             to the class so far), then visits the vertices in reverse colouring order, returning when |C| + colour <=
+ *             |best|; v with P & N(v) empty ends a clique C + {v}, which replaces best when strictly larger; otherwise
+ *             expand(C + {v}, P & N(v)); then P -= {v}.  Each expand call costs one node; when a call would exceed
+ *             max_clique_nodes the search stops, exact[p] = 0, and the best clique so far is kept (exact[p] = 1 otherwise).
+ *   rotation  chain TIMs over the clique c(0) < ... < c(K-1): v_k = a_c(k+1) - a_c(k), w_k = b_c(k+1) - b_c(k), k + 1 taken
+ *             mod K (fp64).  GNC-TLS with weights 1, c2 = beta^2, prev = 0: per iteration < max_iterations: R = Horn's
+ *             rotation of S = sum wt_k v_k w_k^T (as ri_pose_from_matches_f32's refit), r2_k = |w_k - R v_k|^2; on the first
+ *             iteration mu = 1 / (2 max r2 / c2 - 1), stop if mu <= 0; cost = sum wt_k r2_k (the weights before this update);
+ *             wt = 0 if r2 >= (mu+1)/mu c2, 1 if r2 <= mu/(mu+1) c2, else sqrt(c2 mu (mu+1) / r2) - mu; mu *= gnc_factor;
+ *             stop if |cost - prev| < cost_threshold; prev = cost.  R = I when max_iterations == 0.
+ *   translation  per axis, x_k = b_c(k) - R a_c(k) (fp64), r = noise_bound * sqrt(cbar2): the events x_k - r (enter) and
+ *             x_k + r (leave), ordered by value, then enter before leave, then k; after each event the consensus set S
+ *             (when not empty) gives t = sum_S x / |S| and cost = sum_S (x - t)^2 + (K - |S|) r^2, sums in index order;
+ *             the minimum cost wins, the earliest event on ties.
+ *   output    T[p] = [R | t] rounded to fp32, row-major [4,4], maps src onto tgt; inliers[p] = #{m < M : |R a_m + t - b_m|^2
+ *             < inlier_dist^2} under that fp32 T, with the arithmetic of ri_pose_from_matches_f32.  M < 3 or a clique of
+ *             fewer than 3 vertices: T[p] = I and inliers[p] = 0.
+ * clique [P,ld] (may be NULL) receives the clique as ascending match positions, -1 past its end; clique_size [P] and
+ * exact [P] are required.  No host synchronisation, no float atomics: a pair's result is bit-reproducible and does not
+ * depend on the rest of the batch.  workspace >= ri_teaser_workspace_bytes(P, ld) bytes (0 when P <= 0 or ld is outside
+ * [1, 32768]), 256-byte aligned.  RI_ERR_BAD_ARG for a non-positive or non-finite noise_bound, cbar2 or inlier_dist,
+ * gnc_factor <= 1, max_iterations < 0, max_clique_nodes < 1, or clique_size / exact NULL; RI_ERR_UNSUPPORTED for
+ * ld > 32768 or P > 65535; RI_ERR_WORKSPACE for a missing or short workspace. */
+size_t ri_teaser_workspace_bytes(int P, int ld);
+int ri_teaser_f32(const float* src, const float* tgt, const int* idx1, const int* idx2, const int* count, int P, int n1,
+                  int n2, int ld, float noise_bound, float cbar2, float gnc_factor, int max_iterations, float cost_threshold,
+                  long long max_clique_nodes, float inlier_dist, float* T, int* inliers, int* clique, int* clique_size,
+                  int* exact, void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---- FPFH descriptors (SURVEY.md 8f, row f8)-------------------------------------------------------------------------
  * Open3D's compute_fpfh_feature with KDTreeSearchParamHybrid(radius, max_nn) (Rusu, Blodow, Beetz, ICRA 2009;
  * pipelines/registration/Feature.cpp), B clouds per call.  xyz [B,3,N], normals [B,3,N] fp32 (used as given, not
  * renormalised); radius > 0 (+inf = plain k-NN), 1 <= max_nn <= 128.  For each point q:

@@ -61,6 +61,9 @@ SIGNATURES = {
     "ri_estimate_normals_f32": (_I, [_P, _I, _I, ctypes.c_float, _I, _P, _P, _P, _P, _P, _Z, _P]),
     "ri_fgr_f32": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, ctypes.c_float, _I, ctypes.c_float, _I, _I, _I,
                         ctypes.c_float, _I, ctypes.c_ulonglong, ctypes.c_float, _P, _P, _P, _P, _P]),
+    "ri_teaser_workspace_bytes": (_Z, [_I, _I]),
+    "ri_teaser_f32": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, ctypes.c_float, ctypes.c_float, ctypes.c_float, _I,
+                           ctypes.c_float, ctypes.c_longlong, ctypes.c_float, _P, _P, _P, _P, _P, _P, _Z, _P]),
     "ri_fpfh_workspace_bytes": (_Z, [_I, _I, _I]),
     "ri_compute_fpfh_f32": (_I, [_P, _P, _I, _I, ctypes.c_float, _I, _P, _P, _P, _P, _Z, _P]),
     "ri_mutual_nn_workspace_bytes":(_Z, [_I, _I, _I, _I]),

@@ -41,15 +41,6 @@ struct FgrParams {
     int iterations, use_absolute_scale, decrease_mu, tuple_test, max_tuples;
 };
 
-// |u - v| in fp64 from fp32 coordinates, in the fixed order sqrt((dx*dx + dy*dy) + dz*dz), without contraction
-__device__ __forceinline__ double edge_len(float3 u, float3 v)
-{
-    const double dx = __dsub_rn((double)u.x, (double)v.x);
-    const double dy = __dsub_rn((double)u.y, (double)v.y);
-    const double dz = __dsub_rn((double)u.z, (double)v.z);
-    return __dsqrt_rn(__dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), __dmul_rn(dz, dz)));
-}
-
 __device__ __forceinline__ bool edge_ok(double la, double lb, double s)
 {
     return __dmul_rn(la, s) < lb && lb < __ddiv_rn(la, s);
@@ -68,20 +59,6 @@ __device__ __forceinline__ bool tuple_trial(const PairMatches& pm, unsigned long
     pm.load(i0, a0, b0); pm.load(i1, a1, b1); pm.load(i2, a2, b2);
     return edge_ok(edge_len(a0, a1), edge_len(b0, b1), s) && edge_ok(edge_len(a1, a2), edge_len(b1, b2), s) &&
            edge_ok(edge_len(a2, a0), edge_len(b2, b0), s);
-}
-
-// block-wide maximum of one double per thread; result valid in thread 0
-__device__ __forceinline__ double block_max(double v, double* red)
-{
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v = fmax(v, __shfl_down_sync(0xffffffffu, v, o));
-    __syncthreads();
-    if (lane == 0) red[warp] = v;
-    __syncthreads();
-    if (threadIdx.x == 0)
-        for (int w = 1; w < nw; ++w) v = fmax(v, red[w]);
-    return v;
 }
 
 __global__ void __launch_bounds__(kThreads, 2)

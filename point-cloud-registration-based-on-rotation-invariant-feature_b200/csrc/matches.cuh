@@ -1,6 +1,7 @@
-// matches.cuh — how the pose solvers read the mutual matches, shared by csrc/pose.cu (RANSAC, Kabsch) and csrc/fgr.cu (FGR):
-// the splitmix64 finaliser their samplers hash with, the gather of a pair's matched coordinates, the clamped match count
-// and the inlier test, so that every mode reads the same matches and its inlier count means the same thing.
+// matches.cuh — how the pose solvers read the mutual matches, shared by csrc/pose.cu (RANSAC, Kabsch), csrc/fgr.cu (FGR) and
+// csrc/teaser.cu (TEASER++):
+// the splitmix64 finaliser their samplers hash with, the gather of a pair's matched coordinates, the clamped match count,
+// the fp64 edge length and the inlier test, so that every mode reads the same matches and its inlier count means the same thing.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -39,6 +40,15 @@ __device__ __forceinline__ int match_count(const int* __restrict__ count, int p,
 {
     const int M = count[p];
     return M < 0 ? 0 : (M > ld ? ld : M);
+}
+
+// |u - v| in fp64 from fp32 coordinates, in the fixed order sqrt((dx*dx + dy*dy) + dz*dz), without contraction
+__device__ __forceinline__ double edge_len(float3 u, float3 v)
+{
+    const double dx = __dsub_rn((double)u.x, (double)v.x);
+    const double dy = __dsub_rn((double)u.y, (double)v.y);
+    const double dz = __dsub_rn((double)u.z, (double)v.z);
+    return __dsqrt_rn(__dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), __dmul_rn(dz, dz)));
 }
 
 __device__ __forceinline__ bool inlier(const Rt& T, float3 a, float3 b, float t2h)

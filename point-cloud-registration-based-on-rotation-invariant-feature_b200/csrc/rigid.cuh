@@ -1,4 +1,5 @@
-// rigid.cuh — fp64 rigid-transform solvers and the block reduction shared by csrc/pose.cu, csrc/icp.cu and csrc/fgr.cu.
+// rigid.cuh — fp64 rigid-transform solvers and the block reduction shared by csrc/pose.cu, csrc/icp.cu, csrc/fgr.cu
+// and csrc/teaser.cu.
 #pragma once
 #include <cuda_runtime.h>
 
@@ -82,6 +83,20 @@ __device__ void block_sum(double (&v)[NV], double* red)
         for (int w = 1; w < nw; ++w)
 #pragma unroll
             for (int k = 0; k < NV; ++k) v[k] += red[w * NV + k];
+}
+
+// block-wide maximum of one double per thread; result valid in thread 0
+__device__ __forceinline__ double block_max(double v, double* red)
+{
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v = fmax(v, __shfl_down_sync(0xffffffffu, v, o));
+    __syncthreads();
+    if (lane == 0) red[warp] = v;
+    __syncthreads();
+    if (threadIdx.x == 0)
+        for (int w = 1; w < nw; ++w) v = fmax(v, red[w]);
+    return v;
 }
 
 // Solves A x = b for the symmetric 6x6 A given by its 21 upper-triangle entries in row order (A00 A01 .. A05 A11 .. A55),

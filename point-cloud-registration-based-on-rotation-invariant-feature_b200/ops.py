@@ -1024,3 +1024,64 @@ def _(xyz, normals, radius, max_nn, with_spfh, with_counts):
     B, _, N = xyz.shape
     return (xyz.new_empty((B, 33, N)), xyz.new_empty((B, 33, N) if with_spfh else (0,)),
             xyz.new_empty((B, N) if with_counts else (0,), dtype=torch.int32))
+
+
+# ---------------------------------------------------------------------------------------------- TEASER++ (f10)
+TEASER_MAX_LD = 1 << 15
+
+
+@torch.library.custom_op("ri::teaser", mutates_args=())
+def teaser(src: torch.Tensor, tgt: torch.Tensor, idx1: torch.Tensor, idx2: torch.Tensor, count: torch.Tensor,
+           noise_bound: float, cbar2: float, gnc_factor: float, max_iterations: int, cost_threshold: float,
+           max_clique_nodes: int, inlier_dist: float) -> tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor,
+                                                              torch.Tensor]:
+    """src [P,n1,3], tgt [P,n2,3] f32; idx1/idx2 [P,ld], count [P] i32 (mutual matches) -> (T [P,4,4] f32 src->tgt,
+    inliers [P] i32, clique [P,ld] i32 (ascending match positions, -1 padded), clique_size [P] i32, exact [P] i32).
+    TEASER++ with a known scale per pair, all pairs in one call (csrc/teaser.cu)."""
+    _req(src, "src", torch.float32); _req(tgt, "tgt", torch.float32)
+    _req(idx1, "idx1", torch.int32); _req(idx2, "idx2", torch.int32); _req(count, "count", torch.int32)
+    dev = _same_device(src, tgt, idx1, idx2, count)
+    _shape(src, "src", None, None, 3)
+    P, n1, _ = src.shape
+    _shape(tgt, "tgt", P, None, 3)
+    _shape(idx1, "idx1", P, None)
+    _shape(idx2, "idx2", P, idx1.shape[1])
+    _shape(count, "count", P)
+    for name, v in (("noise_bound", noise_bound), ("cbar2", cbar2), ("inlier_dist", inlier_dist)):
+        if not (math.isfinite(float(v)) and float(v) > 0.0):
+            raise RuntimeError("%s must be finite and > 0" % name)
+    if not float(gnc_factor) > 1.0:
+        raise RuntimeError("rotation_gnc_factor must be > 1")
+    if int(max_iterations) < 0:
+        raise RuntimeError("rotation_max_iterations must be >= 0")
+    if not 1 <= int(max_clique_nodes) < 1 << 63:
+        raise RuntimeError("max_clique_nodes must be >= 1")
+    n2 = tgt.shape[1]
+    ld = idx1.shape[1]
+    if ld > TEASER_MAX_LD or P > 65535:
+        raise RuntimeError("ri_teaser: unsupported size (ld <= %d and P <= 65535)" % TEASER_MAX_LD)
+    with torch.cuda.device(dev):
+        T = torch.empty((P, 4, 4), dtype=torch.float32, device=dev)
+        inl = torch.empty((P,), dtype=torch.int32, device=dev)
+        clique = torch.empty((P, ld), dtype=torch.int32, device=dev)
+        size = torch.empty((P,), dtype=torch.int32, device=dev)
+        exact = torch.empty((P,), dtype=torch.int32, device=dev)
+        if P == 0 or ld == 0 or n1 == 0 or n2 == 0:
+            T.copy_(torch.eye(4, device=dev).expand(P, 4, 4)); inl.zero_(); size.zero_(); exact.fill_(1)
+            return T, inl, clique, size, exact
+        nws = _L.ri_teaser_workspace_bytes(P, ld)
+        ws = torch.empty(nws, dtype=torch.uint8, device=dev)
+        _check(_L.ri_teaser_f32(src.data_ptr(), tgt.data_ptr(), idx1.data_ptr(), idx2.data_ptr(), count.data_ptr(),
+                                P, n1, n2, ld, float(noise_bound), float(cbar2), float(gnc_factor), int(max_iterations),
+                                float(cost_threshold), int(max_clique_nodes), float(inlier_dist), T.data_ptr(),
+                                inl.data_ptr(), clique.data_ptr(), size.data_ptr(), exact.data_ptr(), ws.data_ptr(), nws,
+                                _stream()), "ri_teaser")
+    return T, inl, clique, size, exact
+
+
+@teaser.register_fake
+def _(src, tgt, idx1, idx2, count, noise_bound, cbar2, gnc_factor, max_iterations, cost_threshold, max_clique_nodes,
+      inlier_dist):
+    P, ld = idx1.shape
+    return (src.new_empty((P, 4, 4)), count.new_empty((P,)), count.new_empty((P, ld)), count.new_empty((P,)),
+            count.new_empty((P,)))

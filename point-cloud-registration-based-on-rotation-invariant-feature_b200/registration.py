@@ -1,17 +1,18 @@
 """Registration back end on the GPU: descriptors -> mutual matches -> rigid pose -> ICP refinement -> RRE / RTE / RMSE,
-whole batches of pairs per call (csrc/matcher.cu + csrc/pose.cu + csrc/fgr.cu + csrc/icp.cu).
+whole batches of pairs per call (csrc/matcher.cu + csrc/pose.cu + csrc/fgr.cu + csrc/teaser.cu + csrc/icp.cu).
 
 Mirrors the reference's meter `MeterModelNet40_registration` (/root/reference/datasets/deepgmr_mn40.py:98-244): same
 constructor argument, same `update((feat1, feat2), (pt1, pt2, gt_trans))` / `compute()` contract, same thresholds
 (:107-109), same result keys (:141).  The reference copies the descriptors to the host and calls Open3D / TEASER++ once
 per pair (:121, :165-231); here `func='ransac'` runs the RANSAC configuration the reference hands to Open3D
 (utils/open3d_func.py:43-49: voxel_size 0.08, edge-length similarity 0.9, max_iter 1000) on the GPU for all pairs at once,
-`func='fgr'` Open3D's Fast Global Registration over the same matches (`fgr()`), and `func='kabsch'` the plain least squares
-over the mutual matches.  `icp()` / `evaluate_registration()` are Open3D's registration_icp (point-to-point and
-point-to-plane) and evaluate_registration, batched over pairs; `register_pairs` and the meter refine their pose with it
-when given `icp={...}`.  `generalized_icp()` is Open3D's registration_generalized_icp (plane-to-plane, covariances from
-normals), a separate refinement after any of them: `generalized_icp(pt1, pt2, r, init=T)`.  TEASER++ is a third-party solver the reference only calls into; it is not re-implemented
-(func='icp' / 'teaserpp' raise in `estimate_poses`: ICP refines a pose, it does not estimate one from matches).
+`func='fgr'` Open3D's Fast Global Registration over the same matches (`fgr()`), `func='teaserpp'` TEASER++ with a known
+scale (`teaser()`: maximum clique of the pairwise-consistency graph, GNC-TLS rotation, adaptive-voting translation), and
+`func='kabsch'` the plain least squares over the mutual matches.  `icp()` / `evaluate_registration()` are Open3D's
+registration_icp (point-to-point and point-to-plane) and evaluate_registration, batched over pairs; `register_pairs` and
+the meter refine their pose with it when given `icp={...}`.  `generalized_icp()` is Open3D's registration_generalized_icp
+(plane-to-plane, covariances from normals), a separate refinement after any of them: `generalized_icp(pt1, pt2, r, init=T)`.
+func='icp' raises in `estimate_poses`: ICP refines a pose, it does not estimate one from matches.
 """
 import time
 
@@ -19,22 +20,30 @@ import torch
 
 from . import matcher, ops
 
-__all__ = ['estimate_poses', 'fgr', 'registration_metrics', 'icp', 'generalized_icp', 'evaluate_registration',
+__all__ = ['estimate_poses', 'fgr', 'teaser', 'registration_metrics', 'icp', 'generalized_icp', 'evaluate_registration',
            'register_pairs', 'MeterModelNet40_registration']
 
 
 def estimate_poses(src, tgt, idx1, idx2, count, func='ransac', voxel_size=0.08, max_iter=1000, edge_similarity=0.9,
-                   refine_iters=3, seed=0):
+                   refine_iters=3, seed=0, noise_bound=None):
     """src [P,n1,3], tgt [P,n2,3] CUDA fp32; idx1/idx2/count: the mutual matches (matcher.mutual_nn).
     -> (T [P,4,4] fp32 mapping src onto tgt, inliers [P] int32).
     func='fgr' is fgr() with maximum_correspondence_distance = 0.5 * voxel_size (the value of Open3D's FGR tutorial) and
-    inlier_dist = voxel_size, Open3D's other defaults, and `seed`; max_iter, edge_similarity and refine_iters are unused."""
-    if func not in ('ransac', 'kabsch', 'fgr'):
-        raise ValueError("func must be 'ransac', 'fgr' or 'kabsch' (TEASER++ is a third-party solver; ICP refines a pose: "
+    inlier_dist = voxel_size, Open3D's other defaults, and `seed`; max_iter, edge_similarity and refine_iters are unused.
+    func='teaserpp' is teaser() with `noise_bound` (required: it is in the clouds' units and has no unit-free default),
+    inlier_dist = voxel_size and TEASER++'s other defaults; max_iter, edge_similarity, refine_iters and seed are unused.
+    The other modes ignore noise_bound."""
+    if func not in ('ransac', 'kabsch', 'fgr', 'teaserpp'):
+        raise ValueError("func must be 'ransac', 'fgr', 'teaserpp' or 'kabsch' (ICP refines a pose: "
                          "icp() or register_pairs(..., icp={...}))")
     if func == 'fgr':
         r = fgr(src, tgt, idx1, idx2, count, maximum_correspondence_distance=0.5 * float(voxel_size), seed=seed,
                 inlier_dist=float(voxel_size))
+        return r['transformation'], r['inliers']
+    if func == 'teaserpp':
+        if noise_bound is None:
+            raise ValueError("func='teaserpp' needs noise_bound (the bound on a match's noise, in the clouds' units)")
+        r = teaser(src, tgt, idx1, idx2, count, noise_bound, inlier_dist=float(voxel_size))
         return r['transformation'], r['inliers']
     hyps = int(max_iter) if func == 'ransac' else 0
     return torch.ops.ri.pose_from_matches(src.float().contiguous(), tgt.float().contiguous(), idx1.contiguous(),
@@ -71,6 +80,36 @@ def fgr(src, tgt, idx1, idx2, count, maximum_correspondence_distance=0.025, iter
             pos = torch.arange(idx1.shape[1], dtype=torch.int32, device=ncorr.device).expand(idx1.shape[0], -1)
             corr = torch.where(pos < ncorr[:, None], pos, -1)
         out['correspondences'] = corr
+    return out
+
+
+# expand calls of the exact maximum-clique search per pair; no pair of tools/bench_teaser.py's workloads reaches it
+# (profiles/r6_teaser.md)
+MAX_CLIQUE_NODES = 100000
+
+
+def teaser(src, tgt, idx1, idx2, count, noise_bound, cbar2=1.0, rotation_gnc_factor=1.4, rotation_max_iterations=100,
+           rotation_cost_threshold=1e-12, max_clique_nodes=MAX_CLIQUE_NODES, inlier_dist=None, return_clique=False):
+    """TEASER++ (RobustRegistrationSolver with a known scale: estimate_scaling=False) for P pairs at once, over given
+    matches: src [P,n1,3], tgt [P,n2,3] CUDA fp32; idx1/idx2 [P,ld], count [P] (matcher.mutual_nn).  Options carry
+    TEASER++'s names; noise_bound is in the clouds' units.  Pipeline: the pairwise-consistency graph (edge when two
+    matches' lengths differ by at most 2 noise_bound sqrt(cbar2)), its maximum clique (deterministic branch and bound with
+    a budget of max_clique_nodes expand calls; clique_exact says whether it finished), GNC-TLS rotation over the clique's
+    chain TIMs, adaptive-voting translation.  Inliers are counted within inlier_dist (default: noise_bound) under the
+    returned pose, as in estimate_poses.  include/ri_b200.h (ri_teaser_f32) states the arithmetic and DESIGN.md §8 the
+    deltas from TEASER++.
+    -> dict(transformation [P,4,4] fp32 src -> tgt, inliers [P] int32, clique_size [P] int32, clique_exact [P] bool
+    [, clique [P,ld] int32: ascending match positions, -1 padded])."""
+    if inlier_dist is None:
+        inlier_dist = noise_bound
+    T, inl, clique, size, exact = torch.ops.ri.teaser(src.float().contiguous(), tgt.float().contiguous(),
+                                                      idx1.contiguous(), idx2.contiguous(), count.contiguous(),
+                                                      float(noise_bound), float(cbar2), float(rotation_gnc_factor),
+                                                      int(rotation_max_iterations), float(rotation_cost_threshold),
+                                                      int(max_clique_nodes), float(inlier_dist))
+    out = {'transformation': T, 'inliers': inl, 'clique_size': size, 'clique_exact': exact.bool()}
+    if return_clique:
+        out['clique'] = clique
     return out
 
 
@@ -170,9 +209,11 @@ def register_pairs(feat1, feat2, pt1, pt2, func='ransac', icp=None, **kw):
 class MeterModelNet40_registration:
     """Same state, thresholds and result keys as the reference meter (deepgmr_mn40.py:98-141)."""
 
-    def __init__(self, func='ransac', device='cuda', icp=None):
-        """func: 'ransac', 'fgr' or 'kabsch' (estimate_poses).  icp: None, or a dict of `icp()` keyword arguments; the
-        estimated pose is then refined with it (inside reg_time)."""
+    def __init__(self, func='ransac', device='cuda', icp=None, noise_bound=None):
+        """func: 'ransac', 'fgr', 'teaserpp' or 'kabsch' (estimate_poses).  icp: None, or a dict of `icp()` keyword
+        arguments; the estimated pose is then refined with it (inside reg_time).  noise_bound: required by 'teaserpp'."""
+        if func == 'teaserpp' and noise_bound is None:
+            raise ValueError("func='teaserpp' needs noise_bound (the bound on a match's noise, in the clouds' units)")
         self.rre = 0
         self.rte = 0
         self.num = 0
@@ -186,6 +227,7 @@ class MeterModelNet40_registration:
         self.func = func
         self.device = torch.device(device)
         self.icp = icp
+        self.kw = {} if noise_bound is None else {'noise_bound': noise_bound}
 
     def update(self, output, target):
         """output = (feat1, feat2) [b,C,n]; target = (pt1 [b,n,3], pt2 [b,n,3], gt_trans [b,4,4]) — numpy or torch."""
@@ -195,7 +237,7 @@ class MeterModelNet40_registration:
             pt1, pt2, gt = (torch.as_tensor(t, dtype=torch.float32).to(dev) for t in target)
             torch.cuda.synchronize(dev)
             t0 = time.time()
-            T, _, _ = register_pairs(feat1, feat2, pt1, pt2, func=self.func, icp=self.icp)
+            T, _, _ = register_pairs(feat1, feat2, pt1, pt2, func=self.func, icp=self.icp, **self.kw)
             torch.cuda.synchronize(dev)
             reg_time = time.time() - t0
             m = registration_metrics(gt, T, pt1).cpu()
