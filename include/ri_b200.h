@@ -180,7 +180,10 @@ int ri_trilinear_devox_f32(const float* coords, const float* feat, int B, int C,
                            float* outs, int* inds, float* wgts, void* stream);
 
 /* spherical_trilinear_devoxelize_forward (interpolate/spherical_trilinear_devox.cpp:19-56), index quirks kept.
- * coords = normalised Cartesian coords, g_inds [B,N] = spherical cell of each point. Requires r >= 4. */
+ * coords = normalised Cartesian coords, g_inds [B,N] = spherical cell of each point.
+ * Requires r >= 4, else RI_ERR_UNSUPPORTED before any launch: the reference's corner rows are radians truncated to ints
+ * (alpha row <= 6, beta row <= 3, gamma row always 0), so the highest corner index is r^2 + 7r + 4, which stays below r^3
+ * only from r = 4 on. */
 int ri_sph_trilinear_devox_f32(const float* coords, const float* feat, const int* g_inds, int B, int C, int N, int r,
                                float* outs, int* inds, float* wgts, void* stream);
 

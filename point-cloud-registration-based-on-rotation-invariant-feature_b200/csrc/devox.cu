@@ -661,6 +661,10 @@ extern "C" int ri_trilinear_devox_f32(const float* coords, const float* feat, in
 extern "C" int ri_sph_trilinear_devox_f32(const float* coords, const float* feat, const int* g_inds,
                                           int B, int C, int N, int r, float* outs, int* inds, float* wgts, void* stream)
 {
+    // The reference's corner rows are radians truncated to ints (a_lo <= 6, b_lo <= 3) and the gamma row is always 0, so
+    // the highest corner index is r^2 + 7r + 4: inside the r^3 grid only for r >= 4.  Smaller grids would read (forward)
+    // and atomically add (backward) past the end of every channel plane.
+    if (r > 0 && r < 4) return RI_ERR_UNSUPPORTED;
     if (g_inds == nullptr) return RI_ERR_BAD_ARG;
     return devox_impl<true>(coords, feat, g_inds, B, C, N, r, outs, inds, wgts, (cudaStream_t)stream);
 }

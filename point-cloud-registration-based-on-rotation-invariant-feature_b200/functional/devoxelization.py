@@ -27,7 +27,7 @@ class TrilinearDevoxelization(Function):
 
 
 class SphericalTrilinearDevoxelization(Function):
-    """(features [B,C,r,r,r], normalised coords [B,3,N], g_inds [B,N], r, is_training=True) -> [B,C,N]"""
+    """(features [B,C,r,r,r], normalised coords [B,3,N], g_inds [B,N], r >= 4, is_training=True) -> [B,C,N]"""
 
     @staticmethod
     def forward(ctx, features, coords, g_inds, resolution, is_training=True):

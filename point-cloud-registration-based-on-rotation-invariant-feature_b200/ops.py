@@ -381,6 +381,8 @@ def sph_trilinear_devox(coords: torch.Tensor, features: torch.Tensor, g_inds: to
     _shape(g_inds, "g_inds", B, N)
     if r <= 0 or features.numel() != B * C * r ** 3:
         raise RuntimeError("features must hold B*C*r^3 elements")
+    if r < 4:
+        raise RuntimeError("spherical devoxelization needs r >= 4: its corner indices reach r^2 + 7r + 4")
     with torch.cuda.device(dev):
         outs = torch.empty((B, C, N), dtype=torch.float32, device=dev)
         inds = torch.empty((B, 8, N), dtype=torch.int32, device=dev)

@@ -81,6 +81,17 @@ def test_abi_version_and_workspace_query(built_lib):
     assert 4 * 1024 * 4 + 64 * 1024 * 4 <= small < big <= 32 * (6 * 1024 * 4 + 64 * 1024 * 4 + 1024)
 
 
+def test_spherical_devox_refuses_r_below_4_before_any_launch(built_lib):
+    """The spherical devoxelizer's corner indices reach r^2 + 7r + 4, past the r^3 grid for r = 2 and 3: the entry point
+    returns RI_ERR_UNSUPPORTED (-3) before touching a pointer or the device (null pointers, no GPU needed here)."""
+    fn = built_lib.ri_sph_trilinear_devox_f32
+    fn.restype = ctypes.c_int
+    fn.argtypes = [ctypes.c_void_p] * 3 + [ctypes.c_int] * 4 + [ctypes.c_void_p] * 4
+    for r in (2, 3):
+        assert fn(None, None, None, 2, 5, 100, r, None, None, None, None) == -3, r
+    assert fn(None, None, None, 2, 5, 100, 4, None, None, None, None) == -1     # r = 4 passes the guard (null g_inds: bad arg)
+
+
 def test_backend_has_reference_function_names():
     """The hot-path subset of src/bindings.cpp:13-56."""
     import ri_b200
