@@ -331,7 +331,7 @@ int ri_icp_f32(const float* src, const float* tgt, const float* tgt_normals, con
  * kernel that equals H and g in exact arithmetic, so the two differ by rounding only.  (2) Open3D's GetRotationFromE1ToX
  * returns the identity when n.e1 < -0.99, so for normals within about 8 degrees of -x it uses the covariance of e1 instead of
  * that of n; here the exact formula is used for every normal (read from Open3D's GeneralizedICP.cpp, not verified against
- * a build of it).  (3) Robust kernels and caller-supplied covariance matrices are not supported.
+ * a build of it).  (3) Caller-supplied covariance matrices are not supported (robust kernels: ri_robust_icp_f32).
  * src [P,n1,3], tgt [P,n2,3], src_normals [P,n1,3], tgt_normals [P,n2,3] (both required), init [P,4,4] row-major
  * (NULL = identity), fp32 point-major.  Outputs as ri_icp_f32.  Bit-reproducible (no float atomics); a pair's result does not
  * depend on the rest of the batch; max_iter + 6 launches, no host synchronisation, no allocation.
@@ -341,6 +341,41 @@ int ri_generalized_icp_f32(const float* src, const float* tgt, const float* src_
                            const float* init, int P, int n1, int n2, float max_corr_dist, float epsilon, int max_iter,
                            float rel_fitness, float rel_rmse, float* T, double* fitness, double* inlier_rmse, int* iters,
                            int* corr, void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---- Robust kernels for point-to-plane and generalized ICP (SURVEY.md 8f, row f11) -------------------------------------
+ * Open3D's TransformationEstimationPointToPlane(loss) and TransformationEstimationForGeneralizedICP(epsilon, loss).  The
+ * loop, the correspondences, the stopping rule, fitness, inlier_rmse, iters, corr and the fp64 accumulated T are exactly
+ * ri_icp_f32's; only the update's sums are weighted, in fp64, by w(r) = Open3D's RobustKernel::Weight (formulas recalled
+ * from Open3D's RobustKernel.cpp, not verified against its source or a build), e = |r|:
+ *   RI_LOSS_L2      1                                  RI_LOSS_CAUCHY  1 / (1 + (r/k)^2)
+ *   RI_LOSS_L1      1 / e  (0 at e = 0, delta 1)       RI_LOSS_GM      k / (k + r^2)^2   (k in squared units, w(0) = 1/k)
+ *   RI_LOSS_HUBER   k / max(e, k)                      RI_LOSS_TUKEY   (1 - (e/k)^2)^2 for e <= k, else 0
+ *   point-to-plane (generalized == 0): r = (q - t).n_t, J = [q x n_t, n_t] with n_t as given (not normalised);
+ *               H = sum w(r) J^T J, g = sum w(r) J^T r (w J_a first, then the same fma as ri_icp_f32: with w = 1 exactly the
+ *               sums, and so every output, are bit-identical to ri_icp_f32's point-to-plane).
+ *   generalized (!= 0): M as in ri_generalized_icp_f32, W = (M^-1)^(1/2) (principal root, closed form from the eigenvectors
+ *               a +- b of M), r = W d, row k weighted by w(r_k): H = sum J0^T A J0, g = sum J0^T A d with
+ *               A = W diag(w(r_0), w(r_1), w(r_2)) W (with L2, A = M^-1 up to rounding).  The rows are the world axes, so
+ *               a robust result is not invariant to rotating both clouds together (as in Open3D).
+ *   Then the point-to-plane solve: |det H| < 1e-6 or a non-finite x gives U = I.
+ * Deltas from Open3D: (1) L1 gives w = 0 at r = 0 exactly, where Open3D's +inf makes the step non-finite (identity update).
+ * (2) As in ri_icp_f32, the original source is transformed by the accumulated T.  (3) The 1e-6 determinant rule sees the
+ * weighted H, so a kernel changes which systems count as singular (e.g. GM with a large k).
+ * src, tgt, tgt_normals (required), src_normals (required and read when generalized != 0 only), init: as
+ * ri_generalized_icp_f32.  Outputs as ri_icp_f32.  Bit-reproducible; a pair's result does not depend on the rest of the
+ * batch.  workspace >= ri_icp_workspace_bytes(P, n1, n2).  RI_ERR_BAD_ARG for the argument errors of ri_icp_f32, a NULL
+ * normals pointer, epsilon <= 0 or not finite (generalized), an unknown loss, or k <= 0 or not finite for Huber, Cauchy, GM
+ * and Tukey. */
+#define RI_LOSS_L2 0
+#define RI_LOSS_L1 1
+#define RI_LOSS_HUBER 2
+#define RI_LOSS_CAUCHY 3
+#define RI_LOSS_GM 4
+#define RI_LOSS_TUKEY 5
+int ri_robust_icp_f32(const float* src, const float* tgt, const float* src_normals, const float* tgt_normals,
+                      const float* init, int P, int n1, int n2, float max_corr_dist, int generalized, float epsilon,
+                      int loss, float k, int max_iter, float rel_fitness, float rel_rmse, float* T, double* fitness,
+                      double* inlier_rmse, int* iters, int* corr, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- normal estimation for xyz-only clouds (SURVEY.md 8f, row f6) ----------------------------------------------------
  * Open3D's estimate_normals with KDTreeSearchParamHybrid(radius, max_nn) (the reference calls it on the host,

@@ -58,6 +58,8 @@ SIGNATURES = {
                         _P, _P, _P, _P, _P, _P, _Z, _P]),
     "ri_generalized_icp_f32": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, ctypes.c_float, ctypes.c_float, _I, ctypes.c_float,
                                     ctypes.c_float, _P, _P, _P, _P, _P, _P, _Z, _P]),
+    "ri_robust_icp_f32": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, ctypes.c_float, _I, ctypes.c_float, _I, ctypes.c_float,
+                               _I, ctypes.c_float, ctypes.c_float, _P, _P, _P, _P, _P, _P, _Z, _P]),
     "ri_estimate_normals_f32": (_I, [_P, _I, _I, ctypes.c_float, _I, _P, _P, _P, _P, _P, _Z, _P]),
     "ri_fgr_f32": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, ctypes.c_float, _I, ctypes.c_float, _I, _I, _I,
                         ctypes.c_float, _I, ctypes.c_ulonglong, ctypes.c_float, _P, _P, _P, _P, _P]),

@@ -1,5 +1,5 @@
 // icp.cu — batched ICP refinement (point-to-point, point-to-plane and generalized / plane-to-plane) and registration
-// evaluation, sm_100a (SURVEY.md §8f rows f5 and f9).
+// evaluation, sm_100a (SURVEY.md §8f rows f5, f9 and f11).
 //
 // Open3D's registration_icp / evaluate_registration (the reference reaches them through utils/open3d_func.py), for P
 // independent (source, target) pairs per call, with Open3D's loop per pair:
@@ -19,6 +19,10 @@
 // (C = I for a zero-length or non-finite normal); per correspondence a = R n^_s (R the rotation of the fp32 T that moved the
 // point, in fp64), b = n^_t, M = C_t + R C_s R^T = 2I - (1 - eps)(a a^T + b b^T), d = q - t, J0 = [-[q]x, I3];
 // H = sum J0^T M^-1 J0, g = sum J0^T M^-1 d in fp64, then the point-to-plane solve and composition above on (H, g).
+// Robust kernels (row f11, Open3D's RobustKernel of TransformationEstimationPointToPlane / ForGeneralizedICP): the same loop
+// with every residual row weighted by w(r) (robust_weight).  Point-to-plane: w of the scalar residual multiplies J^T J and
+// J r.  Generalized: W = (M^-1)^(1/2) in closed form, r = W d, row k weighted by w(r_k); H and g are the sums above with M^-1
+// replaced by A = W diag(w) W.
 //
 // One deliberate difference from Open3D: Open3D transforms its copy of the source incrementally (s <- U s every
 // iteration); here every iteration transforms the ORIGINAL source by the accumulated T, which is kept in fp64 on the device.
@@ -32,7 +36,9 @@
 //                  normals in the same order.  (Order inside a cell is not fixed; nothing depends on it: the selection key
 //                  is (distance, index).)
 //   icp_scan       exclusive scan of the histogram.
-//   icp_iter       grid (source tiles, P), once per iteration.  A CTA of a converged pair exits at once.  Otherwise each
+//   icp_iter       grid (source tiles, P), once per iteration (one instantiation per estimator, plus a robust one each for
+//                  point-to-plane and generalized ICP that takes the loss and its parameter as launch arguments).  A CTA of
+//                  a converged pair exits at once.  Otherwise each
 //                  thread runs a radius-bounded 1-NN for its source points over the cells the query ball can touch,
 //                  accumulates count, sum d^2 and the solver's moments in fp64 (15 for point-to-point: sum q, sum t,
 //                  sum q t^T; 27 for point-to-plane and generalized ICP: the upper triangle of H and g), the CTA reduces them in a
@@ -43,6 +49,7 @@
 //   icp_final      T (fp32), fitness, rmse (fp64), iterations (int32).
 #include "ri_common.cuh"
 #include "rigid.cuh"
+#include "ri_b200.h"
 
 namespace {
 
@@ -324,13 +331,100 @@ __device__ __forceinline__ void gicp_moments(const float* Tf, double qx, double 
     acc[28] += i02 * dx + i12 * dy + i22 * dz;
 }
 
-// EST = kPointToPoint / kPointToPlane / kGeneralized.  src_nrm [P,n1,3] and eps are read by kGeneralized only.
-template <int EST>
+// Open3D's RobustKernel::Weight(r) in fp64 (RI_LOSS_*; k > 0 for Huber, Cauchy, GM and Tukey), with e = |r|:
+// L2 1; L1 1/e (0 at e = 0, where Open3D's +inf would make the step non-finite); Huber k / max(e, k);
+// Cauchy 1 / (1 + (r/k)^2); GM k / (k + r^2)^2 (k in squared-residual units); Tukey (1 - (e/k)^2)^2 for e <= k, else 0.
+__device__ __forceinline__ double robust_weight(int loss, double k, double r)
+{
+    const double e = fabs(r);
+    switch (loss) {
+    case RI_LOSS_L1: return e > 0.0 ? 1.0 / e : 0.0;
+    case RI_LOSS_HUBER: return k / fmax(e, k);
+    case RI_LOSS_CAUCHY: { const double u = r / k; return 1.0 / (1.0 + u * u); }
+    case RI_LOSS_GM: { const double s = k + r * r; return k / (s * s); }
+    case RI_LOSS_TUKEY: { if (!(e <= k)) return 0.0; const double u = e / k, v = 1.0 - u * u; return v * v; }
+    default: return 1.0;
+    }
+}
+
+// One robust generalized-ICP correspondence into acc[2..28] (arguments as gicp_moments, eps = 1 - c).  W = (M^-1)^(1/2) in
+// closed form: M = 2I - c (a a^T + b b^T) has the eigenvalue 2 off span{a, b}; for unit a and b, u+- = a +- b are
+// eigenvectors with lambda+- = 2 - c (1 +- a.b), so W = 2^-1/2 I + sum (lambda+-^-1/2 - 2^-1/2) u u^T / |u|^2 (a zero u has
+// lambda = 2 and is skipped); with one of a, b zero and u the other, W = 2^-1/2 I + ((2 - c)^-1/2 - 2^-1/2) u u^T.
+// r = W d, w_k = robust_weight(r_k), A = W diag(w) W; the moments are gicp_moments' with A in place of M^-1.
+__device__ __forceinline__ void robust_gicp_moments(const float* Tf, double qx, double qy, double qz, double tx, double ty,
+                                                    double tz, const float* ns, float4 nt, double c, int loss, double kp,
+                                                    double* acc)
+{
+    constexpr double kR2 = 0.70710678118654752440;     // 2^-1/2
+    double n[3], a[3], b[3];
+    unit_or_zero(ns[0], ns[1], ns[2], n);
+    unit_or_zero(nt.x, nt.y, nt.z, b);
+#pragma unroll
+    for (int k = 0; k < 3; ++k)
+        a[k] = (double)Tf[4 * k] * n[0] + (double)Tf[4 * k + 1] * n[1] + (double)Tf[4 * k + 2] * n[2];
+    const bool za = n[0] == 0.0 && n[1] == 0.0 && n[2] == 0.0, zb = b[0] == 0.0 && b[1] == 0.0 && b[2] == 0.0;
+    double w00 = kR2, w01 = 0.0, w02 = 0.0, w11 = kR2, w12 = 0.0, w22 = kR2;     // W, symmetric
+    auto add = [&](double u0, double u1, double u2, double f) {                   // W += f u u^T
+        w00 += f * u0 * u0; w01 += f * u0 * u1; w02 += f * u0 * u2;
+        w11 += f * u1 * u1; w12 += f * u1 * u2; w22 += f * u2 * u2;
+    };
+    if (!za && !zb) {
+        const double s = a[0] * b[0] + a[1] * b[1] + a[2] * b[2];
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+            const double sg = h == 0 ? 1.0 : -1.0;
+            const double u0 = a[0] + sg * b[0], u1 = a[1] + sg * b[1], u2 = a[2] + sg * b[2];
+            const double uu = u0 * u0 + u1 * u1 + u2 * u2;
+            if (uu > 0.0) add(u0, u1, u2, (1.0 / sqrt(2.0 - c * (1.0 + sg * s)) - kR2) / uu);
+        }
+    } else if (!(za && zb)) {
+        const double* u = za ? b : a;
+        add(u[0], u[1], u[2], 1.0 / sqrt(2.0 - c) - kR2);
+    }
+    const double dx = qx - tx, dy = qy - ty, dz = qz - tz;
+    const double v0 = robust_weight(loss, kp, w00 * dx + w01 * dy + w02 * dz);
+    const double v1 = robust_weight(loss, kp, w01 * dx + w11 * dy + w12 * dz);
+    const double v2 = robust_weight(loss, kp, w02 * dx + w12 * dy + w22 * dz);
+    // A = W diag(v) W
+    const double i00 = v0 * w00 * w00 + v1 * w01 * w01 + v2 * w02 * w02;
+    const double i01 = v0 * w00 * w01 + v1 * w01 * w11 + v2 * w02 * w12;
+    const double i02 = v0 * w00 * w02 + v1 * w01 * w12 + v2 * w02 * w22;
+    const double i11 = v0 * w01 * w01 + v1 * w11 * w11 + v2 * w12 * w12;
+    const double i12 = v0 * w01 * w02 + v1 * w11 * w12 + v2 * w12 * w22;
+    const double i22 = v0 * w02 * w02 + v1 * w12 * w12 + v2 * w22 * w22;
+    const double w0[3] = {i02 * qy - i01 * qz, i12 * qy - i11 * qz, i22 * qy - i12 * qz};
+    const double w1[3] = {i00 * qz - i02 * qx, i01 * qz - i12 * qx, i02 * qz - i22 * qx};
+    const double w2[3] = {i01 * qx - i00 * qy, i11 * qx - i01 * qy, i12 * qx - i02 * qy};
+    acc[2] += w0[2] * qy - w0[1] * qz;
+    acc[3] += w1[2] * qy - w1[1] * qz;
+    acc[4] += w2[2] * qy - w2[1] * qz;
+    acc[5] += w0[0]; acc[6] += w0[1]; acc[7] += w0[2];
+    acc[8] += w1[0] * qz - w1[2] * qx;
+    acc[9] += w2[0] * qz - w2[2] * qx;
+    acc[10] += w1[0]; acc[11] += w1[1]; acc[12] += w1[2];
+    acc[13] += w2[1] * qx - w2[0] * qy;
+    acc[14] += w2[0]; acc[15] += w2[1]; acc[16] += w2[2];
+    acc[17] += i00; acc[18] += i01; acc[19] += i02;
+    acc[20] += i11; acc[21] += i12;
+    acc[22] += i22;
+    acc[23] += w0[0] * dx + w0[1] * dy + w0[2] * dz;
+    acc[24] += w1[0] * dx + w1[1] * dy + w1[2] * dz;
+    acc[25] += w2[0] * dx + w2[1] * dy + w2[2] * dz;
+    acc[26] += i00 * dx + i01 * dy + i02 * dz;
+    acc[27] += i01 * dx + i11 * dy + i12 * dz;
+    acc[28] += i02 * dx + i12 * dy + i22 * dz;
+}
+
+// EST = kPointToPoint / kPointToPlane / kGeneralized.  src_nrm [P,n1,3] and eps are read by kGeneralized only; ROBUST
+// (point-to-plane and generalized only) weights each residual row with robust_weight(loss, kp, .).
+template <int EST, bool ROBUST>
 __global__ void __launch_bounds__(kThreads)
 icp_iter_kernel(const float* __restrict__ src, int P, int n1, int n2, float r, int it, int max_iter, float rel_fitness,
                 float rel_rmse, int* __restrict__ corr, unsigned char* __restrict__ ws, const float* __restrict__ src_nrm,
-                float eps)
+                float eps, int loss, float kp)
 {
+    static_assert(!ROBUST || EST != kPointToPoint, "point-to-point takes no robust kernel");
     constexpr bool PLANE = EST != kPointToPoint;       // the 27-moment layout and the linearised solve
     constexpr int K = PLANE ? kKMax : kKPoint;
     __shared__ double red[(kThreads / 32) * K];
@@ -405,12 +499,26 @@ icp_iter_kernel(const float* __restrict__ src, int P, int n1, int n2, float r, i
             const double res = (dqx - tx) * nx + (dqy - ty) * ny + (dqz - tz) * nz;
             const double J[6] = {dqy * nz - dqz * ny, dqz * nx - dqx * nz, dqx * ny - dqy * nx, nx, ny, nz};
             int k = 2;
+            if (ROBUST) {      // w J_a, then the same fma as below: w = 1 gives bit-identical sums
+                const double w = robust_weight(loss, (double)kp, res);
 #pragma unroll
-            for (int a = 0; a < 6; ++a)
+                for (int a = 0; a < 6; ++a) {
+                    const double wJ = w * J[a];
 #pragma unroll
-                for (int b = a; b < 6; ++b) acc[k++] += J[a] * J[b];
+                    for (int b = a; b < 6; ++b) acc[k++] += wJ * J[b];
+                    acc[23 + a] += wJ * res;
+                }
+            } else {
 #pragma unroll
-            for (int a = 0; a < 6; ++a) acc[23 + a] += J[a] * res;
+                for (int a = 0; a < 6; ++a)
+#pragma unroll
+                    for (int b = a; b < 6; ++b) acc[k++] += J[a] * J[b];
+#pragma unroll
+                for (int a = 0; a < 6; ++a) acc[23 + a] += J[a] * res;
+            }
+        } else if (ROBUST) {
+            robust_gicp_moments(Tf, dqx, dqy, dqz, tx, ty, tz, src_nrm + ((size_t)p * n1 + i) * 3, __ldg(Nt + bp),
+                                1.0 - (double)eps, loss, (double)kp, acc);
         } else {
             gicp_moments(Tf, dqx, dqy, dqz, tx, ty, tz, src_nrm + ((size_t)p * n1 + i) * 3, __ldg(Nt + bp),
                          1.0 - (double)eps, acc);
@@ -498,10 +606,11 @@ __global__ void icp_final_kernel(int P, int n1, int n2, const unsigned char* __r
 }
 
 // The launch sequence of one call, after the arguments have been checked (P > 0): setup, binning, max_iter + 1 iteration
-// launches, final.  nrm: target normals binned with the grid (NULL for point-to-point).
-int icp_launch(int est, const float* src, const float* tgt, const float* nrm, const float* src_nrm, const float* init,
-               int P, int n1, int n2, float max_corr_dist, float eps, int max_iter, float rel_fitness, float rel_rmse,
-               float* T, double* fitness, double* inlier_rmse, int* iters, int* corr, void* workspace,
+// launches, final.  nrm: target normals binned with the grid (NULL for point-to-point).  loss >= 0 selects the robust
+// instantiation of est (point-to-plane or generalized) with parameter kp; -1 the plain one.
+int icp_launch(int est, int loss, float kp, const float* src, const float* tgt, const float* nrm, const float* src_nrm,
+               const float* init, int P, int n1, int n2, float max_corr_dist, float eps, int max_iter, float rel_fitness,
+               float rel_rmse, float* T, double* fitness, double* inlier_rmse, int* iters, int* corr, void* workspace,
                size_t workspace_bytes, void* stream)
 {
     if (P > 65535) return RI_ERR_UNSUPPORTED;
@@ -521,16 +630,28 @@ int icp_launch(int est, const float* src, const float* tgt, const float* nrm, co
     icp_bin_kernel<1><<<gb, 256, 0, st>>>(tgt, nrm, P, n1, n2, ws);
     RI_LAUNCH_CHECK();
     const dim3 gi(L.tiles, P);
+    const bool robust = loss >= 0;
     for (int it = 0; it <= max_iter; ++it) {
-        if (est == kGeneralized)
-            icp_iter_kernel<kGeneralized><<<gi, kThreads, 0, st>>>(src, P, n1, n2, max_corr_dist, it, max_iter,
-                                                                   rel_fitness, rel_rmse, corr, ws, src_nrm, eps);
+        if (est == kGeneralized && robust)
+            icp_iter_kernel<kGeneralized, true><<<gi, kThreads, 0, st>>>(src, P, n1, n2, max_corr_dist, it, max_iter,
+                                                                         rel_fitness, rel_rmse, corr, ws, src_nrm, eps,
+                                                                         loss, kp);
+        else if (est == kGeneralized)
+            icp_iter_kernel<kGeneralized, false><<<gi, kThreads, 0, st>>>(src, P, n1, n2, max_corr_dist, it, max_iter,
+                                                                          rel_fitness, rel_rmse, corr, ws, src_nrm, eps,
+                                                                          0, 0.f);
+        else if (est == kPointToPlane && robust)
+            icp_iter_kernel<kPointToPlane, true><<<gi, kThreads, 0, st>>>(src, P, n1, n2, max_corr_dist, it, max_iter,
+                                                                          rel_fitness, rel_rmse, corr, ws, nullptr, 0.f,
+                                                                          loss, kp);
         else if (est == kPointToPlane)
-            icp_iter_kernel<kPointToPlane><<<gi, kThreads, 0, st>>>(src, P, n1, n2, max_corr_dist, it, max_iter,
-                                                                    rel_fitness, rel_rmse, corr, ws, nullptr, 0.f);
+            icp_iter_kernel<kPointToPlane, false><<<gi, kThreads, 0, st>>>(src, P, n1, n2, max_corr_dist, it, max_iter,
+                                                                           rel_fitness, rel_rmse, corr, ws, nullptr, 0.f,
+                                                                           0, 0.f);
         else
-            icp_iter_kernel<kPointToPoint><<<gi, kThreads, 0, st>>>(src, P, n1, n2, max_corr_dist, it, max_iter,
-                                                                    rel_fitness, rel_rmse, corr, ws, nullptr, 0.f);
+            icp_iter_kernel<kPointToPoint, false><<<gi, kThreads, 0, st>>>(src, P, n1, n2, max_corr_dist, it, max_iter,
+                                                                           rel_fitness, rel_rmse, corr, ws, nullptr, 0.f,
+                                                                           0, 0.f);
         RI_LAUNCH_CHECK();
     }
     icp_final_kernel<<<(P + 127) / 128, 128, 0, st>>>(P, n1, n2, ws, T, fitness, inlier_rmse, iters);
@@ -556,9 +677,9 @@ extern "C" int ri_icp_f32(const float* src, const float* tgt, const float* tgt_n
 {
     if (P < 0 || n1 <= 0 || n2 <= 0 || !(max_corr_dist > 0.f) || max_iter < 0) return RI_ERR_BAD_ARG;
     if (point_to_plane && tgt_normals == nullptr) return RI_ERR_BAD_ARG;
-    return icp_launch(point_to_plane ? kPointToPlane : kPointToPoint, src, tgt, point_to_plane ? tgt_normals : nullptr,
-                      nullptr, init, P, n1, n2, max_corr_dist, 0.f, max_iter, rel_fitness, rel_rmse, T, fitness,
-                      inlier_rmse, iters, corr, workspace, workspace_bytes, stream);
+    return icp_launch(point_to_plane ? kPointToPlane : kPointToPoint, -1, 0.f, src, tgt,
+                      point_to_plane ? tgt_normals : nullptr, nullptr, init, P, n1, n2, max_corr_dist, 0.f, max_iter,
+                      rel_fitness, rel_rmse, T, fitness, inlier_rmse, iters, corr, workspace, workspace_bytes, stream);
 }
 
 // ri_icp_f32 with the generalized (plane-to-plane) estimator: src_normals [P,n1,3] and tgt_normals [P,n2,3] fp32 point-major
@@ -571,6 +692,26 @@ extern "C" int ri_generalized_icp_f32(const float* src, const float* tgt, const 
 {
     if (P < 0 || n1 <= 0 || n2 <= 0 || !(max_corr_dist > 0.f) || max_iter < 0) return RI_ERR_BAD_ARG;
     if (!(epsilon > 0.f) || !isfinite(epsilon) || src_normals == nullptr || tgt_normals == nullptr) return RI_ERR_BAD_ARG;
-    return icp_launch(kGeneralized, src, tgt, tgt_normals, src_normals, init, P, n1, n2, max_corr_dist, epsilon, max_iter,
-                      rel_fitness, rel_rmse, T, fitness, inlier_rmse, iters, corr, workspace, workspace_bytes, stream);
+    return icp_launch(kGeneralized, -1, 0.f, src, tgt, tgt_normals, src_normals, init, P, n1, n2, max_corr_dist, epsilon,
+                      max_iter, rel_fitness, rel_rmse, T, fitness, inlier_rmse, iters, corr, workspace, workspace_bytes,
+                      stream);
+}
+
+// ri_icp_f32 (point-to-plane) or ri_generalized_icp_f32 (generalized != 0) with a robust kernel: loss RI_LOSS_*, k its
+// parameter (finite, > 0; read by Huber, Cauchy, GM and Tukey only).  src_normals is read when generalized only.
+extern "C" int ri_robust_icp_f32(const float* src, const float* tgt, const float* src_normals, const float* tgt_normals,
+                                 const float* init, int P, int n1, int n2, float max_corr_dist, int generalized,
+                                 float epsilon, int loss, float k, int max_iter, float rel_fitness, float rel_rmse,
+                                 float* T, double* fitness, double* inlier_rmse, int* iters, int* corr, void* workspace,
+                                 size_t workspace_bytes, void* stream)
+{
+    if (P < 0 || n1 <= 0 || n2 <= 0 || !(max_corr_dist > 0.f) || max_iter < 0) return RI_ERR_BAD_ARG;
+    if (loss < RI_LOSS_L2 || loss > RI_LOSS_TUKEY) return RI_ERR_BAD_ARG;
+    if (loss >= RI_LOSS_HUBER && !(k > 0.f && isfinite(k))) return RI_ERR_BAD_ARG;
+    if (tgt_normals == nullptr) return RI_ERR_BAD_ARG;
+    if (generalized && (!(epsilon > 0.f) || !isfinite(epsilon) || src_normals == nullptr)) return RI_ERR_BAD_ARG;
+    return icp_launch(generalized ? kGeneralized : kPointToPlane, loss, k, src, tgt, tgt_normals,
+                      generalized ? src_normals : nullptr, init, P, n1, n2, max_corr_dist, generalized ? epsilon : 0.f,
+                      max_iter, rel_fitness, rel_rmse, T, fitness, inlier_rmse, iters, corr, workspace, workspace_bytes,
+                      stream);
 }

@@ -895,6 +895,61 @@ def _(src, tgt, src_normals, tgt_normals, init, r, epsilon, max_iter, rel_fitnes
             src.new_empty((P,), dtype=torch.int32), src.new_empty((P, n1 if want_corr else 0), dtype=torch.int32))
 
 
+# ---------------------------------------------------------------------------------------------- robust kernels (f11)
+ROBUST_LOSSES = ('l2', 'l1', 'huber', 'cauchy', 'gm', 'tukey')      # position = RI_LOSS_* of include/ri_b200.h
+
+
+def check_robust_icp(src, tgt, src_normals, tgt_normals, init, r, generalized, epsilon, loss, k, max_iter):
+    """Raise RuntimeError unless the arguments of robust_icp are valid; a normals argument may be None here (the Python
+    wrapper estimates generalized ICP's after this check, so a bad call launches nothing).  Point-to-plane reads neither
+    src_normals nor epsilon."""
+    check_generalized_icp(src, tgt, src_normals if generalized else None, tgt_normals, init, r,
+                          epsilon if generalized else 1.0, max_iter)
+    if not 0 <= int(loss) < len(ROBUST_LOSSES):
+        raise RuntimeError("loss must be in [0, %d), got %r" % (len(ROBUST_LOSSES), loss))
+    if int(loss) >= 2 and not (math.isfinite(float(k)) and float(k) > 0.0):
+        raise RuntimeError("the %s kernel's parameter k must be finite and > 0, got %r" % (ROBUST_LOSSES[int(loss)], k))
+
+
+@torch.library.custom_op("ri::robust_icp", mutates_args=())
+def robust_icp(src: torch.Tensor, tgt: torch.Tensor, src_normals: Optional[torch.Tensor], tgt_normals: torch.Tensor,
+               init: torch.Tensor, r: float, generalized: bool, epsilon: float, loss: int, k: float, max_iter: int,
+               rel_fitness: float, rel_rmse: float, want_corr: bool) -> tuple[
+               torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    """Point-to-plane (generalized=False: tgt_normals [P,n2,3]) or generalized ICP (src_normals [P,n1,3] too) with a robust
+    kernel: loss = ROBUST_LOSSES.index(name), k its parameter.  Other arguments and the outputs as icp / generalized_icp.
+    Open3D's TransformationEstimationPointToPlane(loss) / ForGeneralizedICP(epsilon, loss) per pair (csrc/icp.cu)."""
+    check_robust_icp(src, tgt, src_normals, tgt_normals, init, r, generalized, epsilon, loss, k, max_iter)
+    if tgt_normals is None or (generalized and src_normals is None):
+        raise RuntimeError("robust_icp needs tgt_normals, and src_normals when generalized")
+    P, n1, _ = src.shape
+    n2 = tgt.shape[1]
+    dev = src.device
+    with torch.cuda.device(dev):
+        T = torch.empty((P, 4, 4), dtype=torch.float32, device=dev)
+        fit = torch.empty((P,), dtype=torch.float64, device=dev)
+        rmse = torch.empty((P,), dtype=torch.float64, device=dev)
+        iters = torch.empty((P,), dtype=torch.int32, device=dev)
+        corr = torch.empty((P, n1 if want_corr else 0), dtype=torch.int32, device=dev)
+        nws = _L.ri_icp_workspace_bytes(P, n1, n2)
+        ws = torch.empty(nws, dtype=torch.uint8, device=dev)
+        _check(_L.ri_robust_icp_f32(src.data_ptr(), tgt.data_ptr(), src_normals.data_ptr() if generalized else None,
+                                    tgt_normals.data_ptr(), init.data_ptr(), P, n1, n2, float(r), int(generalized),
+                                    float(epsilon), int(loss), float(k), int(max_iter), float(rel_fitness),
+                                    float(rel_rmse), T.data_ptr(), fit.data_ptr(), rmse.data_ptr(), iters.data_ptr(),
+                                    corr.data_ptr() if want_corr else None, ws.data_ptr(), nws, _stream()),
+               "ri_robust_icp")
+    return T, fit, rmse, iters, corr
+
+
+@robust_icp.register_fake
+def _(src, tgt, src_normals, tgt_normals, init, r, generalized, epsilon, loss, k, max_iter, rel_fitness, rel_rmse,
+      want_corr):
+    P, n1 = src.shape[0], src.shape[1]
+    return (src.new_empty((P, 4, 4)), src.new_empty((P,), dtype=torch.float64), src.new_empty((P,), dtype=torch.float64),
+            src.new_empty((P,), dtype=torch.int32), src.new_empty((P, n1 if want_corr else 0), dtype=torch.int32))
+
+
 # ---------------------------------------------------------------------------------------------- normal estimation (f6)
 @torch.library.custom_op("ri::estimate_normals", mutates_args=())
 def estimate_normals(xyz: torch.Tensor, radius: float, max_nn: int, camera: Optional[torch.Tensor],

@@ -12,8 +12,10 @@ scale (`teaser()`: maximum clique of the pairwise-consistency graph, GNC-TLS rot
 registration_icp (point-to-point and point-to-plane) and evaluate_registration, batched over pairs; `register_pairs` and
 the meter refine their pose with it when given `icp={...}`.  `generalized_icp()` is Open3D's registration_generalized_icp
 (plane-to-plane, covariances from normals), a separate refinement after any of them: `generalized_icp(pt1, pt2, r, init=T)`.
+Both point-to-plane `icp()` and `generalized_icp()` take Open3D's robust kernels (`kernel=('tukey', k)` and the like).
 func='icp' raises in `estimate_poses`: ICP refines a pose, it does not estimate one from matches.
 """
+import math
 import time
 
 import torch
@@ -120,27 +122,62 @@ def registration_metrics(gt_trans, est_trans, pts):
 
 
 _ESTIMATIONS = ('point_to_point', 'point_to_plane')
+_KERNELS_WITH_K = ('huber', 'cauchy', 'gm', 'tukey')
+
+
+def _robust_loss(kernel):
+    """A robust-kernel spec -> (loss index of ops.ROBUST_LOSSES, k), or None for None and 'l2' (the plain estimators).
+    ValueError for anything else than 'l1' or (name, k) with name in _KERNELS_WITH_K and k finite and > 0."""
+    if kernel is None or (isinstance(kernel, str) and kernel == 'l2'):
+        return None
+    if isinstance(kernel, str) and kernel == 'l1':
+        return ops.ROBUST_LOSSES.index('l1'), 0.0
+    if isinstance(kernel, (tuple, list)) and len(kernel) == 2 and isinstance(kernel[0], str) \
+            and kernel[0] in _KERNELS_WITH_K:
+        try:
+            k = float(kernel[1])
+        except (TypeError, ValueError):
+            k = float('nan')
+        if math.isfinite(k) and k > 0.0:
+            return ops.ROBUST_LOSSES.index(kernel[0]), k
+        raise ValueError("the %s kernel needs a finite k > 0, got %r" % (kernel[0], kernel[1]))
+    raise ValueError("kernel must be None, 'l2', 'l1' or (name, k) with name one of %s, got %r" % (_KERNELS_WITH_K, kernel))
 
 
 def icp(src, tgt, max_correspondence_distance, init=None, estimation='point_to_point', tgt_normals=None, max_iter=30,
-        relative_fitness=1e-6, relative_rmse=1e-6, return_correspondences=False):
+        relative_fitness=1e-6, relative_rmse=1e-6, return_correspondences=False, kernel=None):
     """Open3D's registration_icp for P pairs at once.  src [P,n1,3], tgt [P,n2,3] CUDA fp32; init [P,4,4] (default identity);
     tgt_normals [P,n2,3] for estimation='point_to_plane'.  Stops a pair when both its fitness and its inlier RMSE change by
     less than the relative criteria (Open3D's ICPConvergenceCriteria), or after max_iter updates.
+    kernel (point_to_plane only; Open3D's TransformationEstimationPointToPlane(loss)): None or 'l2' (the plain least
+    squares), 'l1', or (name, k) with name 'huber', 'cauchy', 'gm' or 'tukey'.  Each correspondence's row of the update is
+    weighted by w(r) of its point-to-plane residual r; k is in distance units (for 'gm' in squared distance units).
+    include/ri_b200.h (ri_robust_icp_f32) states the weights and the deltas from Open3D.
     -> dict(transformation [P,4,4] fp32 src -> tgt, fitness [P] f64, inlier_rmse [P] f64, iterations [P] int32
     [, correspondences [P,n1] int32: target index or -1, under the returned transformation])."""
     if estimation not in _ESTIMATIONS:
         raise ValueError("estimation must be one of %s, got %r" % (_ESTIMATIONS, estimation))
     plane = estimation == 'point_to_plane'
+    if kernel is not None and not plane:
+        raise ValueError("a robust kernel needs estimation='point_to_plane' (Open3D's point-to-point takes none)")
+    robust = _robust_loss(kernel)
     if plane and tgt_normals is None:
         raise ValueError("estimation='point_to_plane' needs tgt_normals")
     src = src.float().contiguous()
     if init is None:
         init = torch.eye(4, dtype=torch.float32, device=src.device).expand(src.shape[0], 4, 4)
     nrm = tgt_normals.float().contiguous() if plane else None
-    T, fit, rmse, iters, corr = torch.ops.ri.icp(src, tgt.float().contiguous(), nrm, init.float().contiguous(),
-                                                 float(max_correspondence_distance), plane, int(max_iter),
-                                                 float(relative_fitness), float(relative_rmse), bool(return_correspondences))
+    if robust is not None:
+        T, fit, rmse, iters, corr = torch.ops.ri.robust_icp(src, tgt.float().contiguous(), None, nrm,
+                                                            init.float().contiguous(),
+                                                            float(max_correspondence_distance), False, 1.0, robust[0],
+                                                            robust[1], int(max_iter), float(relative_fitness),
+                                                            float(relative_rmse), bool(return_correspondences))
+    else:
+        T, fit, rmse, iters, corr = torch.ops.ri.icp(src, tgt.float().contiguous(), nrm, init.float().contiguous(),
+                                                     float(max_correspondence_distance), plane, int(max_iter),
+                                                     float(relative_fitness), float(relative_rmse),
+                                                     bool(return_correspondences))
     out = {'transformation': T, 'fitness': fit, 'inlier_rmse': rmse, 'iterations': iters}
     if return_correspondences:
         out['correspondences'] = corr
@@ -151,7 +188,7 @@ _icp = icp       # register_pairs() and the meter take an `icp` argument of thei
 
 
 def generalized_icp(src, tgt, max_correspondence_distance, init=None, epsilon=1e-3, src_normals=None, tgt_normals=None,
-                    max_iter=30, relative_fitness=1e-6, relative_rmse=1e-6, return_correspondences=False):
+                    max_iter=30, relative_fitness=1e-6, relative_rmse=1e-6, return_correspondences=False, kernel=None):
     """Open3D's registration_generalized_icp (plane-to-plane) for P pairs at once.  src [P,n1,3], tgt [P,n2,3] CUDA fp32;
     init [P,4,4] (default identity).  The loop, the stopping rule, fitness, inlier_rmse and the correspondences are icp()'s;
     the update minimises sum d^T (C_t + R C_s R^T)^-1 d over correspondences, d = T s - t, with the covariances
@@ -161,8 +198,13 @@ def generalized_icp(src, tgt, max_correspondence_distance, init=None, epsilon=1e
     (0,0,1) with fewer than 3).  A normal's sign does not matter.
     Deltas from Open3D: M^-1 is used directly rather than its square root (equal up to rounding); every normal uses the
     exact covariance, where Open3D substitutes that of e1 for normals within about 8 degrees of -x (read from its source,
-    not verified against a build); no robust kernels and no caller-supplied covariance matrices.
-    include/ri_b200.h (ri_generalized_icp_f32) states the arithmetic.
+    not verified against a build); no caller-supplied covariance matrices.
+    kernel: as in icp() (Open3D's TransformationEstimationForGeneralizedICP(epsilon, loss)).  Open3D's way: the residual is
+    whitened, r = W d with W = (C_t + R C_s R^T)^-1/2, and each of its three rows weighted by w(r_k); so k is in whitened
+    units (distance / sqrt(eigenvalue of C_t + R C_s R^T), e.g. distance / sqrt(2 epsilon) along a shared normal and
+    distance / sqrt(2) across it; for 'gm' squared whitened units), and a robust result is not invariant to rotating both
+    clouds together (the rows are the world axes).  None and 'l2' run the plain estimator.
+    include/ri_b200.h (ri_generalized_icp_f32, ri_robust_icp_f32) states the arithmetic.
     -> dict(transformation [P,4,4] fp32 src -> tgt, fitness [P] f64, inlier_rmse [P] f64, iterations [P] int32
     [, correspondences [P,n1] int32: target index or -1, under the returned transformation])."""
     from .functional import estimate_normals
@@ -173,16 +215,24 @@ def generalized_icp(src, tgt, max_correspondence_distance, init=None, epsilon=1e
     init = init.float().contiguous()
     src_normals = None if src_normals is None else src_normals.float().contiguous()
     tgt_normals = None if tgt_normals is None else tgt_normals.float().contiguous()
+    robust = _robust_loss(kernel)
     ops.check_generalized_icp(src, tgt, src_normals, tgt_normals, init, max_correspondence_distance, epsilon, max_iter)
     estimate = lambda x: estimate_normals(x.transpose(1, 2), radius=float('inf'), max_nn=20).transpose(1, 2).contiguous()
     if src_normals is None:
         src_normals = estimate(src)
     if tgt_normals is None:
         tgt_normals = estimate(tgt)
-    T, fit, rmse, iters, corr = torch.ops.ri.generalized_icp(src, tgt, src_normals, tgt_normals, init,
-                                                             float(max_correspondence_distance), float(epsilon),
-                                                             int(max_iter), float(relative_fitness), float(relative_rmse),
-                                                             bool(return_correspondences))
+    if robust is not None:
+        T, fit, rmse, iters, corr = torch.ops.ri.robust_icp(src, tgt, src_normals, tgt_normals, init,
+                                                            float(max_correspondence_distance), True, float(epsilon),
+                                                            robust[0], robust[1], int(max_iter),
+                                                            float(relative_fitness), float(relative_rmse),
+                                                            bool(return_correspondences))
+    else:
+        T, fit, rmse, iters, corr = torch.ops.ri.generalized_icp(src, tgt, src_normals, tgt_normals, init,
+                                                                 float(max_correspondence_distance), float(epsilon),
+                                                                 int(max_iter), float(relative_fitness),
+                                                                 float(relative_rmse), bool(return_correspondences))
     out = {'transformation': T, 'fitness': fit, 'inlier_rmse': rmse, 'iterations': iters}
     if return_correspondences:
         out['correspondences'] = corr
