@@ -502,6 +502,30 @@ size_t ri_fpfh_workspace_bytes(int B, int N, int max_nn);
 int ri_compute_fpfh_f32(const float* xyz, const float* normals, int B, int N, float radius, int max_nn, float* fpfh,
                         float* spfh, int* counts, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- farthest point sampling over variable-length clouds (SURVEY.md 8f, row f12) -------------------------------------
+ * The reference's furthest_point_sampling (backend name; F.furthest_point_sample) and Open3D's farthest_point_down_sample,
+ * B clouds per call.  xyz [B,3,N] fp32; lengths [B] int32 (device) or NULL: cloud b uses its first n_b = lengths[b]
+ * points, 0 <= n_b <= N (values outside are clamped), NULL means n_b = N; m >= 1.  Per cloud, with dist[i] = +inf for
+ * i < n_b and s = 0:
+ *   for k in 0 .. m-1:  idx[b,k] = s;  q = s;  best = 0
+ *                       for i in 0 .. n_b-1 ascending:  d = (dx*dx + dy*dy) + dz*dz in fp64, dx = (double)x_i - (double)x_q,
+ *                                                       each operation rounded (no contraction)
+ *                                                       dist[i] = d < dist[i] ? d : dist[i]
+ *                                                       if dist[i] > best: best = dist[i], s = i
+ * So the lowest index wins ties, s is unchanged when every dist is 0 (once every distinct point is taken, or m > n_b, the
+ * last index repeats), a duplicate of a taken point is never taken, and n_b = 0 gives all -1.  Non-finite coordinates
+ * follow the rule literally (a NaN point keeps dist = +inf; once taken it repeats).  tests/fps_oracle.py replays it.
+ * Deltas.  Open3D (recalled, unverified): the same loop from index 0 with fp64 distances, std::min and a strict > from
+ * max_dist = 0, but it raises when num_samples > n, and Eigen's squaredNorm may sum in another order, so near-ties can
+ * split differently.  The reference kernel (not checked here, unverified): fp32 distances, ties broken in its reduction
+ * tree's order and, if it follows pointnet2, points with |p|^2 <= 1e-3 skipped; no parity with it is claimed.
+ * Output idx [B,m] int32.  Points past n_b are never read.  No float atomics, no workspace, no host synchronisation: a
+ * cloud's result is bit-reproducible and does not depend on the rest of the batch or on its padding.  RI_ERR_BAD_ARG for
+ * B < 0, N < 0, m < 1 or a NULL pointer; RI_ERR_UNSUPPORTED for N > RI_FPS_MAX_POINTS, or N > 65536 on a device that
+ * cannot schedule a 16-CTA cluster (clouds up to 65536 points run on portable clusters of at most 8 CTAs). */
+#define RI_FPS_MAX_POINTS 131072
+int ri_furthest_point_sample_f32(const float* xyz, const int* lengths, int B, int N, int m, int* idx, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

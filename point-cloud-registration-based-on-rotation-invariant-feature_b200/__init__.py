@@ -11,7 +11,8 @@ Layout:
     frontend.py     the fused, graph-captured front-end engine (what bench.py measures)
     matcher.py      mutual-nearest-neighbour descriptor matching
     registration.py matches -> RANSAC / Kabsch pose -> RRE / RTE / RMSE meter (the reference's registration meter)
-    subsampling.py  barycentre grid subsampling (the reference's utils/grid_subsampleing.py API)
+    subsampling.py  barycentre grid subsampling (the reference's utils/grid_subsampleing.py API) and the farthest-point
+                    bridge from its variable-length output to a fixed-size batch
     shard.py        one-process-per-GPU sharding helpers
     synth.py        seeded synthetic inputs
 """
@@ -21,6 +22,6 @@ from .backend import _backend  # noqa: F401
 from . import functional, modules  # noqa: F401
 from .frontend import FrontEnd, FrontEndLanes, FrontEndPipeline  # noqa: F401
 from . import shard, synth, matcher, subsampling, registration  # noqa: F401
-from .subsampling import grid_sub_sampling, grid_sub_sampling_many  # noqa: F401
+from .subsampling import grid_sub_sampling, grid_sub_sampling_many, farthest_point_batch  # noqa: F401
 
 __version__ = '0.1.0'

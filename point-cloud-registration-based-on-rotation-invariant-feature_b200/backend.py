@@ -6,8 +6,8 @@ src/bindings.cpp:13-56).  This object exposes the SAME function names, positiona
 dtypes and shapes for every hot-path function, so the reference's functional/*.py files run unchanged when
 their `from PVCNN.modules.functional.backend import _backend` resolves to it (INTEGRATION.md).
 
-ball_query / grouping (SURVEY.md §8f row f1) are served too.  The remaining functions of the reference backend (sampling,
-3-NN interpolation; SURVEY.md §2 rows 13-14) are outside the path, are not provided here and raise AttributeError.
+ball_query / grouping (SURVEY.md §8f row f1) and sampling (furthest_point_sampling, gather_features_*; row f12) are served
+too.  Only 3-NN interpolation (SURVEY.md §2 row 14) is not provided here and raises AttributeError.
 """
 import torch
 
@@ -85,6 +85,22 @@ class _Backend:
     @staticmethod
     def grouping_backward(grad_y, indices, n):
         return _ri.grouping_backward(grad_y, indices, int(n))
+
+    # sampling/sampling.cpp: furthest_point_sampling(coords [B,3,N], num_samples) -> indices [B,M] int32
+    @staticmethod
+    def furthest_point_sampling(coords, num_samples):
+        return _ri.furthest_point_sample(coords, None, int(num_samples))
+
+    # gather_features_forward(features [B,C,N], indices [B,M]) -> [B,C,M]: grouping with one neighbour per centre
+    @staticmethod
+    def gather_features_forward(features, indices):
+        B, C, _ = features.shape
+        return _ri.grouping(features, indices.unsqueeze(-1)).view(B, C, indices.shape[1])
+
+    # gather_features_backward(grad_y [B,C,M], indices [B,M], n) -> [B,C,n], contributions of repeated indices summed
+    @staticmethod
+    def gather_features_backward(grad_y, indices, n):
+        return _ri.grouping_backward(grad_y.unsqueeze(-1), indices.unsqueeze(-1), int(n))
 
 
 _backend = _Backend()

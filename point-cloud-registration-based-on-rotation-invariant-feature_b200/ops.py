@@ -1142,3 +1142,43 @@ def _(src, tgt, idx1, idx2, count, noise_bound, cbar2, gnc_factor, max_iteration
     P, ld = idx1.shape
     return (src.new_empty((P, 4, 4)), count.new_empty((P,)), count.new_empty((P, ld)), count.new_empty((P,)),
             count.new_empty((P,)))
+
+
+# ---------------------------------------------------------------------------------------------- farthest point sampling (f12)
+def check_furthest_point_sample(xyz, lengths, m):
+    """Every check of ri::furthest_point_sample, on the host and before anything is enqueued."""
+    _req(xyz, "xyz", torch.float32)
+    _shape(xyz, "xyz", None, 3, None)
+    B, _, N = xyz.shape
+    if int(m) < 1:
+        raise RuntimeError("the number of samples must be >= 1")
+    if N > _lib.FPS_MAX_POINTS:
+        raise RuntimeError("farthest point sampling takes at most %d points per cloud, got N = %d" % (_lib.FPS_MAX_POINTS, N))
+    if lengths is not None:
+        if lengths.device.type != "cpu":
+            raise RuntimeError("lengths must be a host (CPU) tensor: its values are checked before the launch")
+        if lengths.dtype != torch.int32:
+            raise RuntimeError("lengths must be an int32 tensor")
+        _shape(lengths, "lengths", B)
+        if B and (int(lengths.min()) < 0 or int(lengths.max()) > N):
+            raise RuntimeError("lengths must lie in [0, N] = [0, %d]" % N)
+
+
+@torch.library.custom_op("ri::furthest_point_sample", mutates_args=())
+def furthest_point_sample(xyz: torch.Tensor, lengths: Optional[torch.Tensor], m: int) -> torch.Tensor:
+    """xyz [B,3,N] f32 (CUDA), lengths [B] i32 on the host or None (every cloud has N points), m >= 1 -> idx [B,m] i32.
+    Farthest point sampling from index 0 with fp64 distances, the lowest index on ties (csrc/fps.cu, include/ri_b200.h)."""
+    check_furthest_point_sample(xyz, lengths, m)
+    B, _, N = xyz.shape
+    dev = xyz.device
+    with torch.cuda.device(dev):
+        lens = lengths.contiguous().to(dev, non_blocking=True) if lengths is not None else None
+        idx = torch.empty((B, int(m)), dtype=torch.int32, device=dev)
+        _check(_L.ri_furthest_point_sample_f32(xyz.data_ptr(), lens.data_ptr() if lens is not None else None, B, N, int(m),
+                                               idx.data_ptr(), _stream()), "ri_furthest_point_sample")
+    return idx
+
+
+@furthest_point_sample.register_fake
+def _(xyz, lengths, m):
+    return xyz.new_empty((xyz.shape[0], m), dtype=torch.int32)

@@ -5,9 +5,14 @@
 return convention (points; points, features; points, labels; or all three — `wrapper.cpp:265-284`).  numpy inputs come back
 as numpy arrays (the reference's types), CUDA tensors come back as CUDA tensors.  Cells are returned in ascending cell
 index (the reference: unordered_map order), barycentres and mean features are bit-identical to the reference's.
+
+`farthest_point_batch(clouds, num_samples)` turns the variable-length output of `grid_sub_sampling_many` into one fixed-size
+batch by farthest point sampling (csrc/fps.cu).
 """
 import numpy as np
 import torch
+
+from .backend import _backend
 
 
 def _prepare(points, features, labels, dev):
@@ -70,3 +75,49 @@ def grid_sub_sampling(points, features=None, labels=None, grid_size=0.1, verbose
     if as_numpy:
         out = [o.cpu().numpy() for o in out]
     return out[0] if len(out) == 1 else tuple(out)
+
+
+def farthest_point_batch(clouds, num_samples):
+    """Variable-length clouds -> one fixed-size batch by farthest point sampling (csrc/fps.cu), the bridge from
+    grid_sub_sampling_many to the batched ops that take dense [B, N, 3] clouds (normals, FPFH, registration).
+
+    `clouds` is a list of CUDA point tensors [n_b, 3] or of tuples (points, features, ...) as grid_sub_sampling_many
+    returns them (features [n_b, C] or None; further entries are ignored).  The clouds are padded into one [B, 3, N_max]
+    batch; their lengths are known on the host, so nothing waits for the GPU.  Each cloud is sampled from its own first
+    point, covering the whole cloud rather than a prefix of it.  A cloud with fewer than num_samples distinct points
+    repeats its last pick; an empty cloud gives idx -1 and undefined rows.
+
+    Returns (points [B, m, 3], features [B, m, C] or None, idx [B, m] int32), m = num_samples, rows in sampling order.
+    Features are gathered only when every cloud has them (with one channel count)."""
+    items = [c if isinstance(c, (tuple, list)) else (c,) for c in clouds]
+    if not items:
+        raise ValueError("farthest_point_batch needs at least one cloud")
+    pts = [torch.as_tensor(c[0]) for c in items]
+    feats = [c[1] if len(c) > 1 else None for c in items]
+    dev = pts[0].device
+    if dev.type != "cuda":
+        raise RuntimeError("farthest_point_batch runs on a CUDA device only (no CPU path exists in this package)")
+    for p in pts:
+        if p.dim() != 2 or p.shape[1] != 3 or p.device != dev:
+            raise RuntimeError("every cloud must be a [n, 3] tensor on %s" % dev)
+    has_f = all(f is not None for f in feats)
+    if not has_f and any(f is not None for f in feats):
+        raise ValueError("either every cloud has features or none has")
+    lengths = [int(p.shape[0]) for p in pts]
+    B, N = len(pts), max(lengths)
+    xyz = torch.zeros((B, 3, N), dtype=torch.float32, device=dev)
+    for b, p in enumerate(pts):
+        xyz[b, :, :lengths[b]] = p.t()
+    idx = torch.ops.ri.furthest_point_sample(xyz, torch.tensor(lengths, dtype=torch.int32), int(num_samples))
+    safe = idx.clamp(min=0)
+    points = _backend.gather_features_forward(xyz, safe).transpose(1, 2).contiguous()
+    features = None
+    if has_f:
+        C = feats[0].shape[1]
+        if any(f.dim() != 2 or f.shape != (n, C) for f, n in zip(feats, lengths)):
+            raise RuntimeError("features must be [n_b, C] with one C for every cloud")
+        fb = torch.zeros((B, C, N), dtype=torch.float32, device=dev)
+        for b, f in enumerate(feats):
+            fb[b, :, :lengths[b]] = torch.as_tensor(f, dtype=torch.float32, device=dev).t()
+        features = _backend.gather_features_forward(fb, safe).transpose(1, 2).contiguous()
+    return points, features, idx
