@@ -526,6 +526,42 @@ int ri_compute_fpfh_f32(const float* xyz, const float* normals, int B, int N, fl
 #define RI_FPS_MAX_POINTS 131072
 int ri_furthest_point_sample_f32(const float* xyz, const int* lengths, int B, int N, int m, int* idx, void* stream);
 
+/* ---- ISS keypoints (SURVEY.md 8f, row f13) ---------------------------------------------------------------------------
+ * Intrinsic Shape Signatures (Zhong, ICCV Workshops 2009) as Open3D's geometry::keypoint::ComputeISSKeypoints computes
+ * them, B clouds per call.  xyz [B,3,N] fp32; gamma a HOST pointer to {gamma_21, gamma_32} in fp64 (read during the call:
+ * Open3D's thresholds are doubles).  tests/iss_oracle.py replays every step.
+ *   distance    d(q,p) = fma(dz,dz, fma(dy,dy, dx*dx)), d* = q - p in fp32 (the expression of ri_estimate_normals_f32);
+ *               N_r(q) = {p : d(q,p) < r*r}, r*r rounded to fp32, q itself included.  A point with a non-finite coordinate
+ *               is nobody's neighbour, has s = 0 and is never a keypoint.
+ *   radii       salient_radius == 0 or non_max_radius == 0: both come from the resolution res_b = the mean, over the
+ *               cloud's finite points, of sqrt((double)d) to the nearest other point (the second key of the k = 2 list:
+ *               0 for a duplicate), summed in fp64 in a fixed order; r_s = (float)(6 res_b), r_nm = (float)(4 res_b).
+ *               Computed on the device per cloud.  A cloud with fewer than 2 finite points gets radii 0 and no keypoints.
+ *               Otherwise both radii must be finite and > 0.
+ *   saliency    s(q) = 0 unless |N_rs(q)| >= min_neighbors; C = the population covariance of N_rs(q) from p - q in fp64,
+ *               summed in an order that depends on the cloud alone; C is not skipped (skipped: every |C_ij| <= 1e-12
+ *               (Eigen's isZero()), an entry not finite, or trace(C) not positive); its eigenvalues e1 >= e2 >= e3 (fp64
+ *               Jacobi on C / trace(C), scaled back) pass e2 / e1 < gamma_21 && e3 / e2 < gamma_32 (fp64 divisions, a NaN
+ *               ratio fails).  Then s(q) = e3.
+ *   keypoint    s(q) > 0, |N_rnm(q)| >= min_neighbors, and no p in N_rnm(q) has s(p) > s(q) (ties keep both points, as
+ *               Open3D's IsLocalMaxima).
+ * Outputs idx [B,N] int32: row b holds the keypoints in ascending index in idx[b, 0:count[b]], -1 after them (the convention
+ * of the matcher's idx1 / count); count [B] int32; unless NULL, saliency [B,N] fp64 = s and radii [B,2] fp32 = (r_s, r_nm)
+ * as used.  No float atomics, no host synchronisation: a cloud's result is bit-reproducible and does not depend on the
+ * rest of the batch.
+ * Deltas from Open3D (read from its source, not verified against a build): the keypoints come back as indices in ascending
+ * order (Open3D pushes them in an unspecified OpenMP order and returns a point cloud); the radius cut is strict; the moments
+ * are centred on q instead of raw cumulants (differs by rounding only); a cloud with fewer than 2 (finite) points and
+ * automatic radii has no keypoints (Open3D reads out of bounds there) and non-finite points are skipped in the resolution.
+ * workspace >= ri_iss_workspace_bytes(B, N) bytes (0 when B <= 0), 256-byte aligned.  RI_ERR_BAD_ARG for B < 0, N < 0, a
+ * radius that is negative or not finite, a NULL gamma, gamma_21 or gamma_32 not > 0, min_neighbors < 1, or a NULL
+ * idx / count / xyz that the call would use; RI_ERR_UNSUPPORTED for B > 65535 or B * N > INT_MAX; RI_ERR_WORKSPACE for a missing, misaligned
+ * or short workspace.  Every check happens before any launch. */
+size_t ri_iss_workspace_bytes(int B, int N);
+int ri_iss_keypoints_f32(const float* xyz, int B, int N, float salient_radius, float non_max_radius, const double* gamma,
+                         int min_neighbors, int* idx, int* count, double* saliency, float* radii, void* workspace,
+                         size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -69,6 +69,8 @@ SIGNATURES = {
     "ri_fpfh_workspace_bytes": (_Z, [_I, _I, _I]),
     "ri_compute_fpfh_f32": (_I, [_P, _P, _I, _I, ctypes.c_float, _I, _P, _P, _P, _P, _Z, _P]),
     "ri_furthest_point_sample_f32": (_I, [_P, _P, _I, _I, _I, _P, _P]),
+    "ri_iss_workspace_bytes": (_Z, [_I, _I]),
+    "ri_iss_keypoints_f32": (_I, [_P, _I, _I, ctypes.c_float, ctypes.c_float, _P, _I, _P, _P, _P, _P, _P, _Z, _P]),
     "ri_mutual_nn_workspace_bytes":(_Z, [_I, _I, _I, _I]),
     "ri_mutual_nn_tf32x3": (_I, [_P, _P, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P, _Z, _P]),
 }

@@ -16,7 +16,7 @@ OBJ = os.path.join(CSRC, "build")
 LIB = os.path.join(HERE, "libri_b200.so")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 
-SOURCES = ["abi.cu", "knn.cu", "knn_warp.cu", "ppf.cu", "prologue.cu", "voxelize.cu", "devox.cu", "grad.cu", "knn_grid.cu", "matcher.cu", "ballquery.cu", "localmlp.cu", "gridsub.cu", "pose.cu", "lrf.cu", "icp.cu", "normals.cu", "fgr.cu", "fpfh.cu", "teaser.cu", "fps.cu"]
+SOURCES = ["abi.cu", "knn.cu", "knn_warp.cu", "ppf.cu", "prologue.cu", "voxelize.cu", "devox.cu", "grad.cu", "knn_grid.cu", "matcher.cu", "ballquery.cu", "localmlp.cu", "gridsub.cu", "pose.cu", "lrf.cu", "icp.cu", "normals.cu", "fgr.cu", "fpfh.cu", "teaser.cu", "fps.cu", "iss.cu"]
 
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
          "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr", "-Xptxas", "-v"]

@@ -3,7 +3,7 @@
 
 #include <string.h>
 
-extern "C" int ri_abi_version(void) { return 10; }
+extern "C" int ri_abi_version(void) { return 11; }
 
 // ---- environment knobs (DESIGN.md §11): read once per process, here
 namespace {

@@ -16,51 +16,20 @@
 // normals_query_kernel: one thread per point in cell order, the ring search of grid_query_kernel with a second exit (every
 // unvisited cell is at least radius away), then the fp64 epilogue in registers.  No atomics after the scatter, so a point's
 // result depends only on its cloud and is bit-reproducible.
+#include "eig3.cuh"
 #include "grid.cuh"
 
 namespace {
 
 // Smallest-eigenvalue eigenvector of the symmetric 3x3 c (c00 c01 c02 c11 c12 c22), scaled to unit trace by the caller.
-// Cyclic Jacobi as horn_rotation (csrc/rigid.cuh), fp64.
+// Cyclic Jacobi of csrc/eig3.cuh, fp64.
 __device__ __forceinline__ void smallest_eigvec3(const double c[6], double& nx, double& ny, double& nz)
 {
     double a[3][3], v[3][3];
     a[0][0] = c[0]; a[0][1] = c[1]; a[0][2] = c[2];
     a[1][1] = c[3]; a[1][2] = c[4]; a[2][2] = c[5];
     a[1][0] = c[1]; a[2][0] = c[2]; a[2][1] = c[4];
-#pragma unroll
-    for (int i = 0; i < 3; ++i)
-#pragma unroll
-        for (int j = 0; j < 3; ++j) v[i][j] = i == j ? 1.0 : 0.0;
-    for (int sweep = 0; sweep < 12; ++sweep) {
-        const double off = a[0][1] * a[0][1] + a[0][2] * a[0][2] + a[1][2] * a[1][2];
-        if (off < 1e-30) break;
-#pragma unroll
-        for (int p = 0; p < 2; ++p)
-#pragma unroll
-            for (int q = p + 1; q < 3; ++q) {
-                const double apq = a[p][q];
-                if (fabs(apq) < 1e-300) continue;
-                const double theta = (a[q][q] - a[p][p]) / (2.0 * apq);
-                const double t = (theta >= 0.0 ? 1.0 : -1.0) / (fabs(theta) + sqrt(theta * theta + 1.0));
-                const double cs = 1.0 / sqrt(t * t + 1.0), sn = t * cs;
-#pragma unroll
-                for (int k = 0; k < 3; ++k) {               // A <- A J (columns p, q)
-                    const double akp = a[k][p], akq = a[k][q];
-                    a[k][p] = cs * akp - sn * akq; a[k][q] = sn * akp + cs * akq;
-                }
-#pragma unroll
-                for (int k = 0; k < 3; ++k) {               // A <- J^T A (rows p, q)
-                    const double apk = a[p][k], aqk = a[q][k];
-                    a[p][k] = cs * apk - sn * aqk; a[q][k] = sn * apk + cs * aqk;
-                }
-#pragma unroll
-                for (int k = 0; k < 3; ++k) {
-                    const double vkp = v[k][p], vkq = v[k][q];
-                    v[k][p] = cs * vkp - sn * vkq; v[k][q] = sn * vkp + cs * vkq;
-                }
-            }
-    }
+    jacobi3(a, v);
     double lo = a[0][0];                                // strict '<': the lowest index wins a tie
     nx = v[0][0]; ny = v[1][0]; nz = v[2][0];
 #pragma unroll

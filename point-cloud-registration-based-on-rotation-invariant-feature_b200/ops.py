@@ -6,6 +6,7 @@ torch (so they live in the caching allocator, as the reference's torch::zeros ou
 hand-written sm_100a kernels on torch's CURRENT stream through ctypes.  There is no other implementation behind
 these names: no Triton, no eager fallback, no CPU path.
 """
+import ctypes
 import math
 from typing import Optional
 
@@ -1182,3 +1183,55 @@ def furthest_point_sample(xyz: torch.Tensor, lengths: Optional[torch.Tensor], m:
 @furthest_point_sample.register_fake
 def _(xyz, lengths, m):
     return xyz.new_empty((xyz.shape[0], m), dtype=torch.int32)
+
+
+# ---------------------------------------------------------------------------------------------- ISS keypoints (f13)
+def check_iss_keypoints(xyz, salient_radius, non_max_radius, gamma_21, gamma_32, min_neighbors):
+    """Every check of ri::iss_keypoints, on the host and before anything is enqueued."""
+    _req(xyz, "xyz", torch.float32)
+    _shape(xyz, "xyz", None, 3, None)
+    B, _, N = xyz.shape
+    for name, v in (("salient_radius", salient_radius), ("non_max_radius", non_max_radius)):
+        if not (math.isfinite(float(v)) and float(v) >= 0.0):
+            raise RuntimeError("%s must be finite and >= 0 (0 = from the cloud's resolution)" % name)
+    for name, v in (("gamma_21", gamma_21), ("gamma_32", gamma_32)):
+        if not float(v) > 0.0:
+            raise RuntimeError("%s must be > 0" % name)
+    if int(min_neighbors) < 1:
+        raise RuntimeError("min_neighbors must be >= 1")
+    if B > 65535 or B * N > 0x7FFFFFFF:
+        raise RuntimeError("ri_iss_keypoints: unsupported size (B <= 65535 and B * N <= 2^31 - 1)")
+
+
+@torch.library.custom_op("ri::iss_keypoints", mutates_args=())
+def iss_keypoints(xyz: torch.Tensor, salient_radius: float, non_max_radius: float, gamma_21: float, gamma_32: float,
+                  min_neighbors: int, want_saliency: bool) -> tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    """xyz [B,3,N] f32 (CUDA) -> (idx [B,N] i32 (keypoints ascending, -1 after count[b]), count [B] i32,
+    saliency [B,N] f64 ([0] unless want_saliency), radii [B,2] f32 (salient, non-max) as used).  Open3D's
+    compute_iss_keypoints, every cloud of the batch in one call (csrc/iss.cu); a radius of 0 takes both radii from the
+    cloud's resolution."""
+    check_iss_keypoints(xyz, salient_radius, non_max_radius, gamma_21, gamma_32, min_neighbors)
+    B, _, N = xyz.shape
+    dev = xyz.device
+    with torch.cuda.device(dev):
+        idx = torch.empty((B, N), dtype=torch.int32, device=dev)
+        count = torch.empty((B,), dtype=torch.int32, device=dev)
+        sal = torch.empty((B, N) if want_saliency else (0,), dtype=torch.float64, device=dev)
+        radii = torch.empty((B, 2), dtype=torch.float32, device=dev)
+        if B == 0:
+            return idx, count, sal, radii
+        nws = _L.ri_iss_workspace_bytes(B, N)
+        ws = torch.empty(nws, dtype=torch.uint8, device=dev)
+        gamma = (ctypes.c_double * 2)(float(gamma_21), float(gamma_32))
+        _check(_L.ri_iss_keypoints_f32(xyz.data_ptr(), B, N, float(salient_radius), float(non_max_radius), gamma,
+                                       int(min_neighbors), idx.data_ptr(), count.data_ptr(),
+                                       sal.data_ptr() if want_saliency else None, radii.data_ptr(), ws.data_ptr(), nws,
+                                       _stream()), "ri_iss_keypoints")
+    return idx, count, sal, radii
+
+
+@iss_keypoints.register_fake
+def _(xyz, salient_radius, non_max_radius, gamma_21, gamma_32, min_neighbors, want_saliency):
+    B, _, N = xyz.shape
+    return (xyz.new_empty((B, N), dtype=torch.int32), xyz.new_empty((B,), dtype=torch.int32),
+            xyz.new_empty((B, N) if want_saliency else (0,), dtype=torch.float64), xyz.new_empty((B, 2)))
